@@ -12,6 +12,7 @@ A step = one pass of the hot path (seed lookup -> candidate windows -> scoring/t
   python bench.py --gpus 1 --steps 3 --warmup 3
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
   python bench.py --impl reference ...        # the reference algorithm's CPU restatement on the host cores
+  python bench.py ... --dump-outputs DIR      # also write the last timed step's results (seeded sample, float64 .npy) to compare builds
 
 Prints ONE JSON line on rank 0.
 """
@@ -27,9 +28,12 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "aligned reads/sec"
 UNIT = "reads/s"
+DUMP_LIMIT = 64 << 20   # bytes of .npy data --dump-outputs writes at most
+DUMP_SEED = 12345
 
 
 def parse():
@@ -46,7 +50,11 @@ def parse():
     ap.add_argument("--counts", action="store_true", help="accumulate the count planes / variant table (always on for c3)")
     ap.add_argument("--cpu-sample", type=int, default=1000000, help="reads in the cpu_baseline sample (about 30 core-seconds of the oracle)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (float64, a fixed seeded sample, at most 64 MB in all)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if a.workload == "auto":
         a.workload = "c1" if world == 1 else "c3"
@@ -177,6 +185,8 @@ def main():
         for _ in range(a.steps):
             dt, r = run()
             times.append(dt)
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, r)
         total = sum(times)
         value = n_sample * a.steps / total
         line = dict(metric=METRIC, value=value, unit=UNIT, n_gpus=a.gpus, steps=a.steps, warmup=a.warmup, ms_per_step=1000.0 * total / a.steps,
@@ -328,6 +338,20 @@ def main():
         stats = r["stats"]
     barrier()
     wall_dev = time.time() - t0
+    if a.dump_outputs and rank == 0:
+        # before any other step runs: the count planes and the variant table are still those of the last timed step
+        extra = {}
+        if a.counts:
+            rng = np.random.default_rng(DUMP_SEED)
+            pidx = np.unique(rng.integers(0, plane_ints, size=min(plane_ints, 1 << 20)))
+            extra["count_planes_index"] = pidx
+            extra["count_planes"] = planes_tensor()[torch.from_numpy(pidx).cuda()].cpu().numpy()
+            var = g.variants_fetch()
+            vidx = np.sort(rng.choice(len(var["count"]), size=min(len(var["count"]), 1 << 16), replace=False))
+            extra["variants_index"] = vidx
+            for k in ("gpos", "region", "dir", "ins", "allele", "count", "ex_gid", "ex_rev", "ex_index"):
+                extra["variants_" + k] = var[k][vidx]
+        dump_outputs(a.dump_outputs, r, extra)
     # reduced planes against the one-GPU planes, size-independent: the all-reduced checksum equals the sum of the ranks' local checksums
     # of the same step, and every rank holds the same reduced variant table
     reduce_check = None
@@ -499,6 +523,49 @@ def same_prefix(want, got, n):
         if len(x) != m or x.tobytes() != y.tobytes():
             return False
     return True
+
+
+def _children(off, rows):
+    """Rows `rows` (ascending) of the CSR offsets `off`: (indices of their children, the children's offsets rebased to the selection)."""
+    lens = off[rows + 1] - off[rows]
+    new_off = np.zeros(len(rows) + 1, dtype=np.int64)
+    np.cumsum(lens, out=new_off[1:])
+    return np.repeat(off[rows] - new_off[:-1], lens) + np.arange(new_off[-1]), new_off
+
+
+def select_queries(r, qs):
+    """The result arrays of the queries qs (ascending indices), laid out as the library returns them for a batch of those queries alone."""
+    comps, q_off = _children(r["q_comp_off"], qs)
+    choices, c_off = _children(r["comp_choice_off"], comps)
+    sas, ch_off = _children(r["choice_sa_off"], choices)
+    blocks, sa_off = _children(r["sa_block_off"], sas)
+    return dict(q_comp_off=q_off, comp_choice_off=c_off, choice_sa_off=ch_off, sa_block_off=sa_off,
+                choice_f64=np.asarray(r["choice_f64"]).reshape(-1, 4)[choices].ravel(), sa_f64=np.asarray(r["sa_f64"]).reshape(-1, 2)[sas].ravel(),
+                choice_inner=r["choice_inner"][choices], sa_contig=r["sa_contig"][sas], blocks=np.asarray(r["blocks"]).reshape(-1, 4)[blocks].ravel(),
+                q_status=r["q_status"][qs], sa_reversed=r["sa_reversed"][sas])
+
+
+def dump_outputs(path, r, extra=None):
+    """Writes what a caller of the timed path received in the last step as path/<name>.npy, every array as float64 (the integers
+    involved are below 2^53, so exact): the result arrays of a fixed, seeded sample of the queries (query_index.npy lists them) and
+    `extra`, arrays already sampled by the caller.  The sample is drawn with a fixed seed: 2^17 queries (all of a smaller batch),
+    halved while the files would exceed DUMP_LIMIT."""
+    out = {k: np.asarray(v, dtype=np.float64) for k, v in (extra or {}).items()}
+    size = lambda arrays: sum(128 + v.nbytes for v in arrays.values())   # a .npy file of a 1-D array = 128-byte header + data
+    room = DUMP_LIMIT - size(out)
+    nq = len(r["q_status"])
+    k = min(nq, 1 << 17)
+    while True:
+        qs = np.sort(np.random.default_rng(DUMP_SEED).choice(nq, size=k, replace=False))
+        sel = {n: np.asarray(v, dtype=np.float64) for n, v in select_queries(r, qs).items()}
+        sel["query_index"] = qs.astype(np.float64)
+        if size(sel) <= room:
+            break
+        k //= 2
+    out.update(sel)
+    os.makedirs(path, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(path, name + ".npy"), v)
 
 
 def _emit(line):
