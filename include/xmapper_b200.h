@@ -109,6 +109,23 @@ int xm_build_duplications(xm_handle* h, int32_t min_len, int32_t max_len, int32_
 int xm_build_duplications_host(xm_handle* h, int32_t min_len, int32_t max_len, int32_t min_copies, int32_t window);
 int xm_get_duplications(xm_handle* h, int32_t contig, int32_t* n, int32_t* starts);
 
+/* --infer-ancestors: AncestryDetector.unionRecentAncestors (M/AncestryDetector.java:89-147) over the handle's reference, set up as
+ * M/Mapper.java:666-692 does it.  The handle's reference is replaced by the "-anc" reference: same contigs, same order, same lengths,
+ * with IUPAC unions written where a recent common ancestor was inferred.  The index and the duplication table are discarded, as after
+ * xm_set_reference (in every case: the call builds a temporary index of its own in their place).
+ * min_interesting_size <= 0 / max_short_matches < 0: the HashBlock_Database defaults; Mapper passes (minDuplicationLength, 8) and
+ * dissimilarity_threshold = MaxErrorRate / MutationPenalty.  *n_changed = forward positions whose code changed.
+ * Runs on the device: index build, duplication-group scan (3 copies, window 1), the containment merge on the host, then one warp per
+ * (group, direction) analysis and a kernel that writes the unions into the packed reference.  A position written twice
+ * (OverriddenSequence.putEncoded) returns XM_ERR_STATE with "Cannot override contig <i>[-rev][<index>]: already overridden" (the
+ * reference names the sequence instead of "contig <i>") and leaves the reference unchanged; so does every other error.
+ * References with minDuplicationLength > 32 (over 2^32 bases) are not supported (XM_ERR_ARG). */
+int xm_infer_ancestors(xm_handle* h, double dissimilarity_threshold, int32_t min_interesting_size, int32_t max_short_matches,
+                       int32_t verify_no_duplicate_analyses, int64_t* n_changed);
+/* Packed 4-bit codes of forward contig `contig` as the handle holds it now (ceil(length / 4) words; e.g. the "-anc" reference after
+ * xm_infer_ancestors, for the host's own SequenceDatabase and writers). */
+int xm_get_reference(xm_handle* h, int32_t contig, uint16_t* packed4);
+
 /* AlignerWorker.process(): aligns n_queries queries. Query q owns n_seqs_per_query[q] (1 or 2) consecutive
  * sequences; sequence s is seq_len[s] bases at packed4 + seq_word_off[s] (16-bit words). seq_word_off holds
  * n_sequences + 1 entries: the last one is the total number of 16-bit words of packed4 (what gets copied to the device).

@@ -14,7 +14,7 @@ LIB_PATH = os.environ.get("XM_LIB_PATH") or os.path.join(HERE, "libxmapper_b200.
 
 EXPORTS = ["xm_create", "xm_destroy", "xm_last_error", "xm_set_reference", "xm_set_index_length", "xm_finish_index",
            "xm_set_index_length_wide", "xm_build_index", "xm_get_index_length", "xm_get_index_length_wide", "xm_index_info", "xm_set_duplications", "xm_build_duplications", "xm_build_duplications_host",
-           "xm_get_duplications", "xm_align_batch", "xm_align_batch_device", "xm_results_array", "xm_release_results",
+           "xm_get_duplications", "xm_infer_ancestors", "xm_get_reference", "xm_align_batch", "xm_align_batch_device", "xm_results_array", "xm_release_results",
            "xm_counts_enable", "xm_counts_device_ptr", "xm_counts_fetch", "xm_format_sam",
            "xm_comm_unique_id", "xm_comm_init", "xm_counts_reduce", "xm_counts_batch_info", "xm_variants_fetch", "xm_measure_peaks", "xm_counts_reduce_times"]
 
@@ -123,6 +123,26 @@ class XMapper:
         self._keep = [packed_contigs, lens]
         self._ok(self.L.xm_set_reference(self.h, n, arr, _ptr(lens)))
         self.contig_lengths = [int(x) for x in lens]
+
+    def set_reference_from_codes(self, contigs):
+        """contigs: list of uint8 code arrays (or of (name, codes) pairs), in database order."""
+        codes = [c[1] if isinstance(c, tuple) else c for c in contigs]
+        from mapper_b200 import synth
+        self.set_reference([synth.pack_contig(c) for c in codes], [len(c) for c in codes])
+
+    def infer_ancestors(self, threshold, min_interesting=-1, max_short=-1, verify=False):
+        """xm_infer_ancestors: replaces the reference by its "-anc" reference (the index and duplication table are discarded);
+        returns the number of forward positions whose code changed."""
+        n = C.c_int64()
+        self._ok(self.L.xm_infer_ancestors(self.h, C.c_double(threshold), int(min_interesting), int(max_short), int(bool(verify)), C.byref(n)))
+        return n.value
+
+    def get_reference(self, contig):
+        """Codes (uint8, one per base) of forward contig `contig` as the handle holds it now."""
+        n = self.contig_lengths[contig]
+        out = np.zeros(max((n + 3) // 4, 1), dtype=np.uint16)
+        self._ok(self.L.xm_get_reference(self.h, int(contig), _ptr(out)))
+        return np.stack([out & 15, (out >> 4) & 15, (out >> 8) & 15, (out >> 12) & 15], axis=1).reshape(-1)[:n].astype(np.uint8)
 
     def set_index_length(self, t, wide=False):
         """wide: positions are uint64 (xm_set_index_length_wide; required when 2 x the reference size exceeds 2^32)."""

@@ -609,12 +609,12 @@ __global__ void xm_index_dedupe_kernel(const unsigned long long* keys, const Pos
 }
 struct IxUnmulti { __host__ __device__ unsigned long long operator()(unsigned long long k) const { return k & ~XM_IX_MULTI; } };
 // per run r of equal (used, bucket): kept[r] = count unless the bucket is overfull
-__global__ void xm_index_runs_kernel(const unsigned long long* run_key, const int* run_cnt, int n_runs, long long* kept) {
+__global__ void xm_index_runs_kernel(const unsigned long long* run_key, const int* run_cnt, int n_runs, long long* kept, int max_short) {
   int r = blockIdx.x * blockDim.x + threadIdx.x;
   if (r > n_runs) return;
   if (r == n_runs) { kept[r] = 0; return; }
   const int n = (int)(run_key[r] >> 32);
-  int mx = n * n; if (mx < 5) mx = 5; if (mx > 32766) mx = 32766;
+  int mx = n * n; if (mx < max_short) mx = max_short; if (mx > 32766) mx = 32766; if (mx < 1) mx = 1;   // HostModel::max_count_for
   kept[r] = run_cnt[r] > mx ? 0 : run_cnt[r];
 }
 // first_run[n] = first run whose used >= n (n = 0 .. hi + 1)
@@ -1007,15 +1007,24 @@ static int mirror_model(xm_handle* h) {
 struct DupItem { unsigned long long klo, khi; int32_t sid, st; };   // sid < 0: not a member (ambiguous text, or an image that repeats a stored position)
 struct DupScanD {
   RefD ref; TableD t; int bl, min_copies, prefix;
-  char* scratch; long long scratch_stride;   // per warp: 2 * max_count items
+  char* scratch; long long scratch_stride;   // per warp: 2 * max_count items (GROUPS: followed by 3 int32 per item)
   HostModel::DupRecH* recs; unsigned long long cap; unsigned long long* n_recs;
+  HostModel::DupGrpRec* grecs; int* n_groups; int max_items;   // GROUPS only
 };
+// GROUPS = false: the duplication table's scan (forward-strand blocks, one record each).  GROUPS = true: the ancestry detector's scan
+// (M/AncestryDetector.java:89-147 reads M/Duplication.java objects): every text group of a bucket with >= min_copies distinct members
+// gets an id, and every member - on both strands, reverse-strand images included - becomes one record (sequence, start, length,
+// count, hashcode, group id) in `grecs`.
+template <bool GROUPS>
 __global__ void __launch_bounds__(128) xm_dup_scan_kernel(DupScanD D) {
   const int lane = threadIdx.x & 31;
   const unsigned lt_mask = (1u << lane) - 1u;
   const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
   DupItem* items = (DupItem*)(D.scratch + warp * D.scratch_stride);
+  int* g_count = GROUPS ? (int*)(items + D.max_items) : nullptr;   // per item: members of its text group, first item of the group, group id
+  int* g_first = GROUPS ? g_count + D.max_items : nullptr;
+  int* g_id = GROUPS ? g_first + D.max_items : nullptr;
   for (long long base = warp * 32; base < D.t.capacity; base += n_warps * 32) {
     const long long my = base + lane;
     unsigned long long word = 0;
@@ -1047,19 +1056,45 @@ __global__ void __launch_bounds__(128) xm_dup_scan_kernel(DupScanD D) {
         items[k] = it;
       }
       __syncwarp();
-      for (int ib = 0; ib < n; ib += 32) {
-        const int i = ib + lane;
-        DupItem me; me.sid = -1; me.klo = 0; me.khi = 0; me.st = 0;
-        if (i < n) me = items[i];
-        int count = 0;
-        for (int j = 0; j < n; j++) { const DupItem o = items[j]; count += (o.sid >= 0 && o.klo == me.klo && o.khi == me.khi) ? 1 : 0; }
-        const bool emit = me.sid >= 0 && !(me.sid & 1) && count >= D.min_copies;
-        const unsigned em = __ballot_sync(0xffffffffu, emit);
-        if (em) {
-          unsigned long long at = 0;
-          if (lane == 0) at = atomicAdd(D.n_recs, (unsigned long long)__popc(em));
-          at = __shfl_sync(0xffffffffu, at, 0) + __popc(em & lt_mask);
-          if (emit && at < D.cap) { HostModel::DupRecH r; r.contig = me.sid >> 1; r.st = me.st; r.count_len = count | (D.bl << 24); r.hc = (int32_t)(base + src); D.recs[at] = r; }
+      if constexpr (!GROUPS) {
+        for (int ib = 0; ib < n; ib += 32) {
+          const int i = ib + lane;
+          DupItem me; me.sid = -1; me.klo = 0; me.khi = 0; me.st = 0;
+          if (i < n) me = items[i];
+          int count = 0;
+          for (int j = 0; j < n; j++) { const DupItem o = items[j]; count += (o.sid >= 0 && o.klo == me.klo && o.khi == me.khi) ? 1 : 0; }
+          const bool emit = me.sid >= 0 && !(me.sid & 1) && count >= D.min_copies;
+          const unsigned em = __ballot_sync(0xffffffffu, emit);
+          if (em) {
+            unsigned long long at = 0;
+            if (lane == 0) at = atomicAdd(D.n_recs, (unsigned long long)__popc(em));
+            at = __shfl_sync(0xffffffffu, at, 0) + __popc(em & lt_mask);
+            if (emit && at < D.cap) { HostModel::DupRecH r; r.contig = me.sid >> 1; r.st = me.st; r.count_len = count | (D.bl << 24); r.hc = (int32_t)(base + src); D.recs[at] = r; }
+          }
+        }
+      } else {
+        // pass 1: group sizes, and an id for every group of >= min_copies members (allocated by its first item)
+        for (int i = lane; i < n; i += 32) {
+          const DupItem me = items[i];
+          int count = 0, first = -1;
+          if (me.sid >= 0)
+            for (int j = 0; j < n; j++) { const DupItem o = items[j]; if (o.sid >= 0 && o.klo == me.klo && o.khi == me.khi) { count++; if (first < 0) first = j; } }
+          g_count[i] = count; g_first[i] = first;
+          if (me.sid >= 0 && first == i && count >= D.min_copies) g_id[i] = atomicAdd(D.n_groups, 1);
+        }
+        __syncwarp();
+        // pass 2: one record per member
+        for (int ib = 0; ib < n; ib += 32) {
+          const int i = ib + lane;
+          bool emit = false; int sid = -1, stv = 0, count = 0, gid = -1;
+          if (i < n) { sid = items[i].sid; stv = items[i].st; count = g_count[i]; emit = sid >= 0 && count >= D.min_copies; if (emit) gid = g_id[g_first[i]]; }
+          const unsigned em = __ballot_sync(0xffffffffu, emit);
+          if (em) {
+            unsigned long long at = 0;
+            if (lane == 0) at = atomicAdd(D.n_recs, (unsigned long long)__popc(em));
+            at = __shfl_sync(0xffffffffu, at, 0) + __popc(em & lt_mask);
+            if (emit && at < D.cap) { HostModel::DupGrpRec r; r.sid = sid; r.st = stv; r.count_len = count | (D.bl << 24); r.hc = (int32_t)(base + src); r.gid = gid; D.grecs[at] = r; }
+          }
         }
       }
       __syncwarp();
@@ -1099,7 +1134,7 @@ static int build_duplications_device(xm_handle* h, int min_len, int max_len, int
       const TableD& T = h->tables_host[(size_t)bl];
       if (T.buckets == nullptr) continue;
       D.t = T; D.bl = bl; D.prefix = (bl + 3) / 4;
-      xm_dup_scan_kernel<<<blocks, 128, 0, st>>>(D);
+      xm_dup_scan_kernel<false><<<blocks, 128, 0, st>>>(D);
     }
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(&found, d_n.p, 8, cudaMemcpyDeviceToHost, st));
@@ -1115,6 +1150,204 @@ static int build_duplications_device(xm_handle* h, int min_len, int max_len, int
   return XM_OK;
 }
 
+// ---- ancestor inference on the device (--infer-ancestors: M/AncestryDetector.java:89-439, as M/Mapper.java:666-692 sets it up) ----
+// infer_ancestors_device: a temporary index of the original reference (build_index_device with the caller's minInterestingSize and
+// maxNumShortMatches), the group scan (xm_dup_scan_kernel<true>), saveDuplications on the host over all 2 * n_contigs sequences with the
+// groups kept (HostModel::merge_duplication_groups), then xm_ancestry_kernel - one warp per (group, polarity) analysis,
+// AncestryDetector.analyze :157-337 - and xm_anc_apply_kernel, which writes the inferred unions into the packed reference.
+// Every analysis reads the original codes only, and a position can be written once (M/OverriddenSequence.java:19-27), so the order in
+// which the analyses run does not change the result.  Writes are kept per global position: one bit per position of both strands detects
+// a second write; only forward-strand writes reach the code plane (the reverse sequences are regenerated from the forward ones).
+struct AncMember { int32_t sid, start, bound, cur, best_idx; uint32_t flags; double cum, best; };   // one SimilarityAnalysis
+enum : uint32_t { ANC_AV = 1, ANC_IN = 2, ANC_NLI = 4, ANC_NLA = 8 };   // available, interested; this step: no longer interested / available
+struct AncD {
+  RefD ref;
+  const HostModel::DupGrpRec* recs; const uint32_t* member; const int* goff;   // members of group g: recs[member[goff[g] .. goff[g + 1])]
+  const int64_t* moff; const int32_t* mst; const int32_t* mlen; const int32_t* mgid;   // merged map of sequence s: [moff[s], moff[s + 1]), starts ascending
+  const int32_t* groups; int n_work;   // the analysed groups; work item w: group groups[w >> 1], polarity (w & 1) ? +1 : -1
+  const int32_t* retry_item; const int32_t* retry_resume; const long long* retry_off;   // second attempt: items, the step their writes resume at, scratch offsets
+  AncMember* state; long long n_members;   // per polarity, one AncMember per group member
+  uint8_t* popular; long long pop_cap;     // first attempt: pop_cap steps of `popular` per warp
+  int* ticket;
+  unsigned int* written; uint8_t* plane; const int64_t* fwd_off;   // written: bit per position of both strands; plane: forward codes (0xFF: untouched)
+  int* ovf_n; int32_t* ovf_item; int32_t* ovf_resume; long long* ovf_need;
+  int* err;   // [0] != 0: a position was written twice, [1] its sequence id, [2] its index
+  double threshold, match1, mismatch1, leave_bonus; int verify;   // matchScore(1), mismatchScore(1), mismatchScore(3) * -1 (:423-431)
+};
+__device__ __forceinline__ uint8_t anc_code(const RefD& ref, int sid, int i) { return ref.contig(sid >> 1, sid & 1).at(i); }
+__device__ __forceinline__ void anc_add(AncMember& s, double v) {   // SimilarityAnalysis.addScore
+  s.cum += v;
+  if (s.cum > s.best) { s.best = s.cum; s.best_idx = s.cur; }
+}
+__device__ __forceinline__ void anc_write(const AncD& A, int sid, int index, uint8_t code) {   // :339-351 + OverriddenSequence.putEncoded
+  const long long bit = A.ref.gstart[sid] - A.ref.gstart[0] + index;
+  const unsigned m = 1u << (unsigned)(bit & 31);
+  if (atomicOr(&A.written[bit >> 5], m) & m) {
+    if (atomicCAS(&A.err[0], 0, 1) == 0) { A.err[1] = sid; A.err[2] = index; }
+    return;
+  }
+  if (!(sid & 1)) A.plane[A.fwd_off[sid >> 1] + index] = code;
+}
+__global__ void __launch_bounds__(128) xm_ancestry_kernel(AncD A) {
+  __shared__ int hist_s[4][16];
+  const unsigned full = 0xffffffffu;
+  const int lane = threadIdx.x & 31;
+  int* hist = hist_s[threadIdx.x >> 5];
+  const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  while (true) {
+    int t = 0;
+    if (lane == 0) t = atomicAdd(A.ticket, 1);
+    t = __shfl_sync(full, t, 0);
+    if (t >= A.n_work) break;
+    int item = t, resume = 0;
+    uint8_t* popular = A.popular + warp * A.pop_cap; long long cap = A.pop_cap;
+    if (A.retry_item) { item = A.retry_item[t]; resume = A.retry_resume[t]; popular = A.popular + A.retry_off[t]; cap = A.retry_off[t + 1] - A.retry_off[t]; }
+    const int gid = A.groups[item >> 1], pol = (item & 1) ? 1 : -1;
+    const int m0 = A.goff[gid], nm = A.goff[gid + 1] - m0;
+    const int L = A.recs[A.member[m0]].count_len >> 24;
+    const bool small = nm <= 32;   // one member per lane: its analysis stays in registers
+    AncMember* S = A.state + (item & 1) * A.n_members + m0;
+    AncMember reg; reg.sid = 0; reg.start = reg.bound = reg.cur = reg.best_idx = 0; reg.flags = 0; reg.cum = reg.best = 0;
+    // set-up: analysisBounds :384-421 (every merged entry has >= 3 instances, so interestingBefore / After are the neighbouring
+    // entries) and interest :88-90 (the entry saved at this (sequence, start) still belongs to this group)
+    int n_av = 0, n_in = 0; long long need = 0;
+    for (int j = lane; j < nm; j += 32) {
+      const HostModel::DupGrpRec r = A.recs[A.member[m0 + j]];
+      const int slen = A.ref.len[r.sid >> 1];
+      const long long lo = A.moff[r.sid], hi = A.moff[r.sid + 1];
+      long long a = lo, b = hi;   // first entry with start >= r.st
+      while (a < b) { const long long mid = (a + b) >> 1; if (A.mst[mid] < r.st) a = mid + 1; else b = mid; }
+      const bool exact = a < hi && A.mst[a] == r.st;
+      const int middle = r.st + L / 2;
+      int initial, bound;
+      if (pol > 0) {
+        initial = middle + 1; bound = slen;
+        const long long nx = exact ? a + 1 : a;
+        if (nx < hi) bound = (middle + (A.mst[nx] + A.mlen[nx] / 2)) / 2 + 1;
+      } else {
+        initial = middle; bound = -1;
+        if (a > lo) bound = ((A.mst[a - 1] + A.mlen[a - 1] / 2) + middle) / 2;
+      }
+      const bool valid = (bound - initial) * pol >= 0;
+      const bool in = valid && exact && A.mgid[a] == gid;
+      AncMember s;
+      s.sid = r.sid; s.start = initial; s.bound = bound; s.cur = initial; s.best_idx = initial;
+      s.flags = (valid ? ANC_AV : 0u) | (in ? ANC_IN : 0u);
+      s.cum = s.best = A.threshold * (double)L;   // matchScore(length)
+      n_av += valid ? 1 : 0; n_in += in ? 1 : 0;
+      if (in) need = max(need, (long long)(bound - initial) * pol + 1);   // an interested analysis leaves at its bound at the latest
+      if (small) reg = s; else S[j] = s;
+    }
+    n_av = __reduce_add_sync(full, n_av); n_in = __reduce_add_sync(full, n_in);
+    for (int o = 16; o > 0; o >>= 1) need = max(need, __shfl_xor_sync(full, need, o));
+    __syncwarp();
+    long long step = 0;
+    while (n_in >= 1 && n_av >= 3) {   // :94-137
+      if (step >= cap) {   // out of scratch: the second attempt re-runs the analysis and writes from this step on
+        if (lane == 0) { const int o = atomicAdd(A.ovf_n, 1); A.ovf_item[o] = item; A.ovf_resume[o] = (int32_t)step; A.ovf_need[o] = need; }
+        break;
+      }
+      if (lane < 16) hist[lane] = 0;
+      __syncwarp();
+      for (int j = lane; j < nm; j += 32) {   // :96-102
+        AncMember s;
+        if (small) s = reg; else s = S[j];
+        uint32_t f = s.flags & (ANC_AV | ANC_IN);
+        if ((f & ANC_IN) && s.cur == s.bound) f |= ANC_NLI;
+        if (f & ANC_AV) {
+          if (s.cur < 0 || s.cur >= A.ref.len[s.sid >> 1]) { f |= ANC_NLA; if (f & ANC_IN) f |= ANC_NLI; }
+          else atomicAdd(&hist[anc_code(A.ref, s.sid, s.cur)], 1);
+        }
+        if (small) reg.flags = f; else S[j].flags = f;
+      }
+      __syncwarp();
+      // :103-111 the most frequent code, scanned in ascending code order; a tie gives 0 ('-')
+      const int cnt = lane < 16 ? hist[lane] : 0;
+      const int mx = __reduce_max_sync(full, cnt);
+      const unsigned at_max = __ballot_sync(full, cnt == mx && cnt > 0);
+      const uint8_t best = (mx == 0 || __popc(at_max) > 1) ? (uint8_t)0 : (uint8_t)(__ffs(at_max) - 1);
+      if (lane == 0) popular[step] = best;
+      __syncwarp();
+      int av = 0, in = 0;
+      for (int base = 0; base < nm; base += 32) {
+        const int j = base + lane;
+        bool leaves = false;
+        AncMember s = reg;
+        if (j < nm) {
+          if (!small) s = S[j];
+          const uint32_t f = s.flags;
+          bool nli = (f & ANC_NLI) != 0, inn = (f & ANC_IN) != 0, ava = (f & ANC_AV) != 0;
+          if (nli) {   // :112-117 a leaver with a neighbour and a non-negative score earns mismatchScore(3) * -1
+            if (s.cur >= 0 && s.cur < A.ref.len[s.sid >> 1] && s.cum >= 0) anc_add(s, A.leave_bonus);
+            inn = false;
+          }
+          if (f & ANC_NLA) ava = false;
+          if (ava) {   // :119-123
+            anc_add(s, anc_code(A.ref, s.sid, s.cur) == best ? A.match1 : A.mismatch1);
+            if (s.cum < 0) { ava = false; if (inn) { nli = true; inn = false; } }
+          }
+          if (ava) s.cur += pol;   // :126
+          s.flags = (ava ? ANC_AV : 0u) | (inn ? ANC_IN : 0u);
+          if (small) reg = s; else S[j] = s;
+          av += ava ? 1 : 0; in += inn ? 1 : 0;
+          leaves = nli && step >= resume;
+        }
+        // :127-136 an analysis that stops being interested writes the popular codes over its own sequence, from its start up to its
+        // best index (never reaching its bound); the whole warp writes one leaver's stretch at a time
+        unsigned lm = __ballot_sync(full, leaves);
+        while (lm) {
+          const int src = __ffs(lm) - 1; lm &= lm - 1;
+          const int sid = __shfl_sync(full, s.sid, src), start = __shfl_sync(full, s.start, src);
+          const int bound = __shfl_sync(full, s.bound, src), best_idx = __shfl_sync(full, s.best_idx, src);
+          const long long end = min(min((long long)(bound - start) * pol, (long long)(best_idx - start) * pol + 1), step + 1);
+          for (long long off = lane; off < end; off += 32) {
+            const int index = start + (int)off * pol;
+            const uint8_t anc = popular[off], here = anc_code(A.ref, sid, index);
+            if ((anc != here && anc != 0) || A.verify) anc_write(A, sid, index, (uint8_t)(anc | here));
+          }
+        }
+      }
+      n_av = __reduce_add_sync(full, av); n_in = __reduce_add_sync(full, in);
+      step++;
+    }
+    __syncwarp();
+  }
+}
+// The forward code plane into the packed reference (one thread per 16-bit word); counts the positions whose code changed.
+__global__ void __launch_bounds__(256) xm_anc_apply_kernel(uint16_t* words, long long n_words, const int64_t* word_off, const int32_t* len, int n_contigs,
+                                                           const int64_t* fwd_off, const uint8_t* plane, unsigned long long* n_changed) {
+  const long long w = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  unsigned changed = 0;
+  if (w < n_words) {
+    int lo = 0, hi = n_contigs;   // the last contig whose first word is <= w
+    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (word_off[mid] <= w) lo = mid; else hi = mid; }
+    const long long i0 = (w - word_off[lo]) * 4;
+    if (w >= word_off[lo] && i0 < len[lo]) {
+      unsigned v = words[w];
+      const unsigned v0 = v;
+      for (int k = 0; k < 4 && i0 + k < len[lo]; k++) {
+        const unsigned c = plane[fwd_off[lo] + i0 + k];
+        if (c == 0xFF) continue;
+        if (((v >> (4 * k)) & 15u) != c) { changed++; v = (v & ~(15u << (4 * k))) | (c << (4 * k)); }
+      }
+      if (v != v0) words[w] = (uint16_t)v;
+    }
+  }
+  const unsigned total = __reduce_add_sync(0xffffffffu, changed);
+  if ((threadIdx.x & 31) == 0 && total) atomicAdd(n_changed, (unsigned long long)total);
+}
+__global__ void xm_anc_keys_kernel(const HostModel::DupGrpRec* recs, int n, uint32_t* keys, uint32_t* vals) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) { keys[i] = (uint32_t)recs[i].gid; vals[i] = (uint32_t)i; }
+}
+// goff[g] = first member of group g in the sorted order, goff[n_groups] = n
+__global__ void xm_anc_goff_kernel(const uint32_t* keys, int n, int n_groups, int* goff) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int k = (int)keys[i];
+  for (int g = (i == 0 ? 0 : (int)keys[i - 1] + 1); g <= k; g++) goff[g] = i;
+  if (i == n - 1) for (int g = k + 1; g <= n_groups; g++) goff[g] = n;
+}
 extern "C" {
 
 int xm_create(const xm_params* p, int device, xm_handle** out) {
@@ -1249,11 +1482,12 @@ int xm_finish_index(xm_handle* h, int32_t min_interesting, int32_t max_built) {
   h->m.finish_index(min_interesting, max_built);
   return XM_OK;
 }
-// xm_build_index(h, max_used, 0): the tables of M/HashBlock_Database.java built by the kernels above
-static int build_index_device(xm_handle* h, int max_used) {
+// xm_build_index(h, max_used, 0): the tables of M/HashBlock_Database.java built by the kernels above.  min_interesting > 0 / max_short:
+// the database's minInterestingSize and maxNumShortMatches when a caller chooses them (:68-89; xm_infer_ancestors), else the defaults.
+static int build_index_device(xm_handle* h, int max_used, int min_interesting = -1, int max_short = 5) {
   HostModel& M = h->m;
   int hi = 0; std::vector<int> cap;
-  if (!M.index_plan(max_used, hi, cap, h->err)) return XM_ERR_ARG;
+  if (!M.index_plan(max_used, hi, cap, h->err, min_interesting)) return XM_ERR_ARG;
   if (hi > 16000) { h->err = "xm_build_index: lengths above 16000 are not supported by the device builder (16-bit block coordinates within a slice)"; return XM_ERR_ARG; }
   int key_bits = 33; while ((1 << (key_bits - 32)) <= hi) key_bits++;   // sort key = used << 32 | bucket
   cudaStream_t st = h->stream;
@@ -1404,7 +1638,7 @@ static int build_index_device(xm_handle* h, int max_used) {
     if (!d_cnt64.ensure(((size_t)n_runs + 1) * 16) || !d_kept.ensure(((size_t)n_runs + 1) * 16) || !d_first.ensure(((size_t)hi + 2) * 4)) { h->err = "out of device memory (index offsets)"; return XM_ERR_CUDA; }
     long long* kept = (long long*)d_kept.p; long long* kept_off = kept + (n_runs + 1);
     long long* cnt64 = (long long*)d_cnt64.p; long long* run_start = cnt64 + (n_runs + 1);
-    xm_index_runs_kernel<<<(n_runs + 256) / 256, 256, 0, st>>>((const unsigned long long*)d_run_key.p, (const int*)d_run_cnt.p, n_runs, kept);
+    xm_index_runs_kernel<<<(n_runs + 256) / 256, 256, 0, st>>>((const unsigned long long*)d_run_key.p, (const int*)d_run_cnt.p, n_runs, kept, max_short);
     CK(cudaMemsetAsync(cnt64, 0, ((size_t)n_runs + 1) * 8, st));  // widen the int32 counts to int64 for the scan
     CK(cudaMemcpy2DAsync(cnt64, 8, d_run_cnt.p, 4, 4, (size_t)n_runs, cudaMemcpyDeviceToDevice, st));
     q = tb; CK(cub::DeviceScan::ExclusiveSum(d_tmp.p, q, (const long long*)kept, kept_off, n_runs + 1, st));
@@ -1431,7 +1665,7 @@ static int build_index_device(xm_handle* h, int max_used) {
     for (int k = 1; k <= hi; k++) {
       if (first[(size_t)k + 1] <= first[(size_t)k]) continue;   // no block of this length: PackedMap(1, 1)
       HostTable& T = M.tables[(size_t)k];
-      T.capacity = cap[(size_t)k]; T.max_count = HostModel::max_count_for(k, 5);
+      T.capacity = cap[(size_t)k]; T.max_count = HostModel::max_count_for(k, max_short);
       T.buckets.resize((size_t)T.capacity);
       CK(cudaMemcpy(T.buckets.data(), (const unsigned long long*)d_buckets.p + bbase[(size_t)k], (size_t)T.capacity * 8, cudaMemcpyDeviceToHost));
       const long long np = koff[(size_t)k + 1] - koff[(size_t)k];
@@ -1463,6 +1697,178 @@ static int build_index_device(xm_handle* h, int max_used) {
   if (!up(h->d_tables, tabs.data(), tabs.size() * sizeof(TableD))) { h->err = "device upload failed (index tables)"; return XM_ERR_CUDA; }
   h->tables_host = tabs;
   h->mirrored_generation = M.generation; h->mirrored_dup_generation = ~0ull;   // mirror_model still uploads the duplication table and sets the views
+  return XM_OK;
+}
+
+static int infer_ancestors_device(xm_handle* h, double threshold, int min_interesting, int max_short, bool verify, int64_t* n_changed) {
+  HostModel& M = h->m;
+  const bool trace = getenv("XM_TRACE_SETUP") != nullptr;
+  auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+  const double t_begin = now();
+  *n_changed = 0;
+  // a) the temporary index: lengths up to 2 * minDuplicationLength (M/DuplicationDetector.java:17-31)
+  const int min_len = M.choose_min_dup_len(), max_len = 2 * min_len;
+  if (max_len > 64) { h->err = "xm_infer_ancestors: duplication lengths above 64 (a reference over 2^32 bases) are not supported by the device scan"; return XM_ERR_ARG; }
+  if (int rc = build_index_device(h, max_len, min_interesting, max_short)) return rc;
+  if (int rc = mirror_model(h)) return rc;
+  const double t_index = now();
+  // b) the group scan: DuplicationDetector(3 copies, window 1) :129-214, every member of every group
+  cudaStream_t st = h->stream;
+  const int blocks = h->sm_count * 8, warps = blocks * 4;
+  int max_items = 2;
+  for (int bl = min_len; bl <= max_len; bl++) max_items = std::max(max_items, 2 * h->tables_host[(size_t)bl].max_count);
+  DevBuf d_scratch, d_recs, d_n, d_keys, d_vals, d_keys2, d_vals2, d_tmp, d_goff, d_moff, d_mst, d_mlen, d_mgid, d_groups, d_state, d_pop, d_bits, d_plane, d_fwd_off,
+         d_ovf, d_retry, d_retry_off;
+  struct Free { std::vector<DevBuf*> v; ~Free() { for (DevBuf* b : v) b->release(); } } fr;
+  fr.v = {&d_scratch, &d_recs, &d_n, &d_keys, &d_vals, &d_keys2, &d_vals2, &d_tmp, &d_goff, &d_moff, &d_mst, &d_mlen, &d_mgid, &d_groups, &d_state, &d_pop, &d_bits, &d_plane,
+          &d_fwd_off, &d_ovf, &d_retry, &d_retry_off};
+  DupScanD D; D.ref = h->ref; D.min_copies = 3; D.max_items = max_items; D.recs = nullptr;
+  D.scratch_stride = (((long long)max_items * (long long)(sizeof(DupItem) + 12)) + 255) & ~255LL;
+  if (!d_scratch.ensure((size_t)warps * (size_t)D.scratch_stride) || !d_n.ensure(64)) { h->err = "out of device memory (ancestry group scan)"; return XM_ERR_CUDA; }
+  D.scratch = (char*)d_scratch.p; D.n_recs = (unsigned long long*)d_n.p; D.n_groups = (int*)((char*)d_n.p + 8);
+  unsigned long long cap = 1ull << 20, found = 0;
+  int n_groups = 0;
+  for (int attempt = 0; attempt < 2; attempt++) {   // second attempt: the buffer sized by the first one's count
+    if (!d_recs.ensure((size_t)cap * sizeof(HostModel::DupGrpRec))) { h->err = "out of device memory (ancestry group records)"; return XM_ERR_CUDA; }
+    D.grecs = (HostModel::DupGrpRec*)d_recs.p; D.cap = cap;
+    CK(cudaMemsetAsync(d_n.p, 0, 64, st));
+    for (int bl = min_len; bl <= max_len; bl++) {
+      const TableD& T = h->tables_host[(size_t)bl];
+      if (T.buckets == nullptr) continue;
+      D.t = T; D.bl = bl; D.prefix = (bl + 3) / 4;
+      xm_dup_scan_kernel<true><<<blocks, 128, 0, st>>>(D);
+    }
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(&found, d_n.p, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&n_groups, (char*)d_n.p + 8, 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (found <= cap) break;
+    cap = found;
+  }
+  if (found >= (1ull << 31)) { h->err = "xm_infer_ancestors: more than 2^31 duplication group members"; return XM_ERR_ARG; }
+  const int n_rec = (int)found;
+  std::vector<HostModel::DupGrpRec> recs((size_t)n_rec);
+  if (n_rec) CK(cudaMemcpy(recs.data(), d_recs.p, (size_t)n_rec * sizeof(HostModel::DupGrpRec), cudaMemcpyDeviceToHost));
+  const double t_scan = now();
+  // c) saveDuplications with the groups kept, every sequence; the groups some merged entry still references (DuplicationDetector.getAll)
+  std::vector<std::vector<std::pair<int32_t, HostModel::Dup>>> by_seq;
+  M.merge_duplication_groups(recs, 1, by_seq);
+  const size_t n_seqs = 2 * (size_t)M.n_contigs;
+  std::vector<int64_t> moff(n_seqs + 1, 0);
+  std::vector<int32_t> mst, mlen, mgid;
+  std::vector<char> referenced((size_t)n_groups, 0);
+  for (size_t s = 0; s < n_seqs; s++) {
+    for (const auto& e : by_seq[s]) { mst.push_back(e.first); mlen.push_back(e.second.length); mgid.push_back(e.second.group); referenced[(size_t)e.second.group] = 1; }
+    moff[s + 1] = (int64_t)mst.size();
+  }
+  std::vector<int32_t> groups;
+  for (int g = 0; g < n_groups; g++) if (referenced[(size_t)g]) groups.push_back(g);
+  const double t_merge = now();
+  double t_analysis = t_merge;
+  int n_retried = 0;
+  if (!groups.empty()) {
+    auto up = [&](DevBuf& b, const void* src, size_t bytes) -> bool { return b.ensure(bytes ? bytes : 16) && (!bytes || cudaMemcpy(b.p, src, bytes, cudaMemcpyHostToDevice) == cudaSuccess); };
+    if (!up(d_moff, moff.data(), moff.size() * 8) || !up(d_mst, mst.data(), mst.size() * 4) || !up(d_mlen, mlen.data(), mlen.size() * 4) ||
+        !up(d_mgid, mgid.data(), mgid.size() * 4) || !up(d_groups, groups.data(), groups.size() * 4)) { h->err = "device upload failed (merged duplications)"; return XM_ERR_CUDA; }
+    // the member CSR: records sorted by group id
+    int key_bits = 1; while (key_bits < 32 && (1ll << key_bits) < (long long)n_groups) key_bits++;
+    if (!d_keys.ensure((size_t)n_rec * 4) || !d_vals.ensure((size_t)n_rec * 4) || !d_keys2.ensure((size_t)n_rec * 4) || !d_vals2.ensure((size_t)n_rec * 4) ||
+        !d_goff.ensure(((size_t)n_groups + 1) * 4)) { h->err = "out of device memory (ancestry groups)"; return XM_ERR_CUDA; }
+    xm_anc_keys_kernel<<<(n_rec + 255) / 256, 256, 0, st>>>((const HostModel::DupGrpRec*)d_recs.p, n_rec, (uint32_t*)d_keys.p, (uint32_t*)d_vals.p);
+    size_t tb = 0;
+    cub::DeviceRadixSort::SortPairs(nullptr, tb, (const uint32_t*)d_keys.p, (uint32_t*)d_keys2.p, (const uint32_t*)d_vals.p, (uint32_t*)d_vals2.p, n_rec, 0, key_bits, st);
+    if (!d_tmp.ensure(tb + 16)) { h->err = "out of device memory (ancestry group sort)"; return XM_ERR_CUDA; }
+    CK(cub::DeviceRadixSort::SortPairs(d_tmp.p, tb, (const uint32_t*)d_keys.p, (uint32_t*)d_keys2.p, (const uint32_t*)d_vals.p, (uint32_t*)d_vals2.p, n_rec, 0, key_bits, st));
+    xm_anc_goff_kernel<<<(n_rec + 255) / 256, 256, 0, st>>>((const uint32_t*)d_keys2.p, n_rec, n_groups, (int*)d_goff.p);
+    // d) the analyses
+    long long pop_cap = 32768;   // steps of one analysis the first attempt holds (XM_ANC_SCRATCH: forces the second attempt in tests)
+    if (const char* e = getenv("XM_ANC_SCRATCH")) pop_cap = std::max(1LL, atoll(e));
+    std::vector<int64_t> fwd_off((size_t)M.n_contigs + 1, 0);
+    for (int c = 0; c < M.n_contigs; c++) fwd_off[(size_t)c + 1] = fwd_off[(size_t)c] + M.len[(size_t)c];
+    const int n_work = 2 * (int)groups.size();
+    const size_t bit_words = (size_t)((M.total_fr + 31) / 32);
+    if (!d_state.ensure(2 * (size_t)n_rec * sizeof(AncMember)) || !d_pop.ensure((size_t)warps * (size_t)pop_cap) || !d_bits.ensure(bit_words * 4) ||
+        !d_plane.ensure((size_t)M.total_forward) || !up(d_fwd_off, fwd_off.data(), fwd_off.size() * 8) || !d_ovf.ensure((size_t)n_work * 16 + 64)) {
+      h->err = "out of device memory (ancestry analyses)"; return XM_ERR_CUDA;
+    }
+    CK(cudaMemsetAsync(d_bits.p, 0, bit_words * 4, st));
+    CK(cudaMemsetAsync(d_plane.p, 0xFF, (size_t)M.total_forward, st));
+    AncD A;
+    A.ref = h->ref; A.recs = (const HostModel::DupGrpRec*)d_recs.p; A.member = (const uint32_t*)d_vals2.p; A.goff = (const int*)d_goff.p;
+    A.moff = (const int64_t*)d_moff.p; A.mst = (const int32_t*)d_mst.p; A.mlen = (const int32_t*)d_mlen.p; A.mgid = (const int32_t*)d_mgid.p;
+    A.groups = (const int32_t*)d_groups.p; A.n_work = n_work;
+    A.retry_item = nullptr; A.retry_resume = nullptr; A.retry_off = nullptr;
+    A.state = (AncMember*)d_state.p; A.n_members = n_rec;
+    A.popular = (uint8_t*)d_pop.p; A.pop_cap = pop_cap;
+    int* counters = (int*)d_n.p;   // [0] ticket, [1] overflow count, [2..4] error record
+    A.ticket = counters; A.ovf_n = counters + 1; A.err = counters + 2;
+    A.written = (unsigned int*)d_bits.p; A.plane = (uint8_t*)d_plane.p; A.fwd_off = (const int64_t*)d_fwd_off.p;
+    A.ovf_need = (long long*)d_ovf.p; A.ovf_item = (int32_t*)((char*)d_ovf.p + (size_t)n_work * 8); A.ovf_resume = A.ovf_item + n_work;
+    A.threshold = threshold;
+    A.match1 = threshold * 1;                   // matchScore(1)
+    A.mismatch1 = -1 + threshold * 1;           // mismatchScore(1)
+    A.leave_bonus = (-3 + threshold * 3) * -1;  // mismatchScore(3) * -1
+    A.verify = verify ? 1 : 0;
+    CK(cudaMemsetAsync(d_n.p, 0, 64, st));
+    xm_ancestry_kernel<<<blocks, 128, 0, st>>>(A);
+    CK(cudaGetLastError());
+    int ctr[8] = {0};
+    CK(cudaMemcpyAsync(ctr, d_n.p, 32, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (ctr[1] > 0) {   // second attempt: the analyses that ran out of scratch, each with the scratch its bounds can need
+      const int n_ovf = ctr[1];
+      n_retried = n_ovf;
+      std::vector<long long> need((size_t)n_ovf);
+      std::vector<int32_t> ovf_item((size_t)n_ovf), ovf_resume((size_t)n_ovf);
+      CK(cudaMemcpy(need.data(), A.ovf_need, (size_t)n_ovf * 8, cudaMemcpyDeviceToHost));
+      CK(cudaMemcpy(ovf_item.data(), A.ovf_item, (size_t)n_ovf * 4, cudaMemcpyDeviceToHost));
+      CK(cudaMemcpy(ovf_resume.data(), A.ovf_resume, (size_t)n_ovf * 4, cudaMemcpyDeviceToHost));
+      size_t free_b = 0, total_b = 0;
+      long long budget = 1LL << 30;
+      if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) budget = std::max(budget, (long long)(free_b / 2));
+      for (int i0 = 0; i0 < n_ovf;) {   // batches of analyses whose scratch fits the budget
+        std::vector<int32_t> retry;   // items, then resume steps
+        std::vector<long long> off(1, 0);
+        int i1 = i0;
+        while (i1 < n_ovf && (i1 == i0 || off.back() + need[(size_t)i1] <= budget)) { off.push_back(off.back() + ((need[(size_t)i1] + 15) & ~15LL)); i1++; }
+        const int nb = i1 - i0;
+        retry.insert(retry.end(), ovf_item.begin() + i0, ovf_item.begin() + i1);
+        retry.insert(retry.end(), ovf_resume.begin() + i0, ovf_resume.begin() + i1);
+        if (!up(d_retry, retry.data(), retry.size() * 4) || !up(d_retry_off, off.data(), off.size() * 8) || !d_pop.ensure((size_t)off.back() + 16)) {
+          h->err = "out of device memory (ancestry analyses, second attempt)"; return XM_ERR_CUDA;
+        }
+        A.retry_item = (const int32_t*)d_retry.p; A.retry_resume = A.retry_item + nb; A.retry_off = (const long long*)d_retry_off.p;
+        A.popular = (uint8_t*)d_pop.p; A.n_work = nb;
+        CK(cudaMemsetAsync(d_n.p, 0, 8, st));   // ticket and overflow count; the error record stays
+        xm_ancestry_kernel<<<blocks, 128, 0, st>>>(A);
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(ctr, d_n.p, 32, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        if (ctr[1] != 0) { h->err = "xm_infer_ancestors: an analysis outran the scratch its bounds allow (internal error)"; return XM_ERR_STATE; }
+        i0 = i1;
+      }
+    }
+    t_analysis = now();
+    if (ctr[2]) {   // OverriddenSequence.putEncoded :19-27
+      const int sid = ctr[3];
+      h->err = "Cannot override contig " + std::to_string(sid >> 1) + ((sid & 1) ? "-rev" : "") + "[" + std::to_string(ctr[4]) + "]: already overridden";
+      return XM_ERR_STATE;
+    }
+    // e) the forward plane into the packed reference, and back into the handle's reference
+    const long long n_words = (long long)M.words.size();
+    xm_anc_apply_kernel<<<(unsigned)((n_words + 255) / 256), 256, 0, st>>>((uint16_t*)h->d_words.p, n_words, (const int64_t*)h->d_word_off.p, (const int32_t*)h->d_len.p, M.n_contigs,
+                                                                          (const int64_t*)d_fwd_off.p, (const uint8_t*)d_plane.p, (unsigned long long*)((char*)d_n.p + 32));
+    CK(cudaGetLastError());
+    unsigned long long changed = 0;
+    CK(cudaMemcpyAsync(&changed, (char*)d_n.p + 32, 8, cudaMemcpyDeviceToHost, st));
+    std::vector<uint16_t> words((size_t)n_words);
+    CK(cudaMemcpyAsync(words.data(), h->d_words.p, (size_t)n_words * 2, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    M.words.swap(words);
+    *n_changed = (int64_t)changed;
+  }
+  if (trace) fprintf(stderr, "[xm] infer ancestors: index %.3f s, scan %.3f s (%d members of %d groups), merge %.3f s (%zu groups analysed), analysis %.3f s (%d analyses re-run), apply %.3f s (%lld positions changed)\n",
+                     t_index - t_begin, t_scan - t_index, n_rec, n_groups, t_merge - t_scan, groups.size(), t_analysis - t_merge, n_retried, now() - t_analysis, (long long)*n_changed);
   return XM_OK;
 }
 
@@ -1511,6 +1917,33 @@ int xm_build_duplications_host(xm_handle* h, int32_t min_len, int32_t max_len, i
   std::lock_guard<std::mutex> compute(h->compute_mu);
   if (!h->m.index_finished) { h->err = "index not set"; return XM_ERR_STATE; }
   h->m.build_duplications(min_len, max_len, min_copies, window);
+  return XM_OK;
+}
+int xm_infer_ancestors(xm_handle* h, double dissimilarity_threshold, int32_t min_interesting_size, int32_t max_short_matches, int32_t verify_no_duplicate_analyses,
+                       int64_t* n_changed) {
+  if (!h || !n_changed) return XM_ERR_ARG;
+  std::lock_guard<std::mutex> compute(h->compute_mu);
+  if (h->m.n_contigs < 1) { h->err = "reference not set"; return XM_ERR_STATE; }
+  CK(cudaSetDevice(h->device));
+  const int rc = infer_ancestors_device(h, dissimilarity_threshold, min_interesting_size > 0 ? min_interesting_size : -1, max_short_matches < 0 ? 5 : max_short_matches,
+                                        verify_no_duplicate_analyses != 0, n_changed);
+  // The temporary index replaced the handle's tables: in every case the index and the duplication table are gone, as after
+  // xm_set_reference; the codes changed only on success (infer_ancestors_device touches HostModel::words last).
+  if (rc != XM_OK) *n_changed = 0;
+  h->m.reference_codes_changed();
+  for (auto& b : h->d_ix_chunks) b.release();
+  h->d_ix_chunks.clear();
+  for (auto& b : h->d_buckets) b.release();
+  for (auto& b : h->d_positions) b.release();
+  for (auto& b : h->d_positions_hi) b.release();
+  return rc;
+}
+int xm_get_reference(xm_handle* h, int32_t contig, uint16_t* packed4) {
+  if (!h || !packed4) return XM_ERR_ARG;
+  if (h->m.n_contigs < 1) { h->err = "reference not set"; return XM_ERR_STATE; }
+  if (contig < 0 || contig >= h->m.n_contigs) return XM_ERR_ARG;
+  const size_t nw = ((size_t)h->m.len[(size_t)contig] + 3) / 4;
+  memcpy(packed4, h->m.words.data() + h->m.word_off[(size_t)contig], nw * 2);
   return XM_OK;
 }
 int xm_get_duplications(xm_handle* h, int32_t contig, int32_t* n, int32_t* starts) {

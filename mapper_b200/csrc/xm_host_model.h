@@ -70,8 +70,13 @@ struct HostModel {
     int64_t g = position_bias;
     for (int c = 0; c < n; c++) { gstart[2 * c] = g; g += lengths[c]; gstart[2 * c + 1] = g; g += lengths[c]; }
     gstart[2 * (size_t)n] = g; position_end = g; total_fr = g - position_bias;
-    for (int c = 0; c < n && !ref_ambiguous; c++) { SeqView v = contig_view(c, 0); for (int i = 0; i < v.len; i++) if (bp_is_ambiguous(v.at(i))) { ref_ambiguous = true; break; } }
-    tables.clear(); max_built = 0; index_finished = false; dup_starts.assign(n, {}); dup_set = false; dup_generation++;
+    reference_codes_changed();
+  }
+  // after the codes of the reference changed (set_reference, or the "-anc" reference written over it): everything derived from them is gone
+  void reference_codes_changed() {
+    ref_ambiguous = false;
+    for (int c = 0; c < n_contigs && !ref_ambiguous; c++) { SeqView v = contig_view(c, 0); for (int i = 0; i < v.len; i++) if (bp_is_ambiguous(v.at(i))) { ref_ambiguous = true; break; } }
+    tables.clear(); max_built = 0; index_finished = false; dup_starts.assign((size_t)n_contigs, {}); dup_set = false; dup_generation++;
     generation++;
   }
 
@@ -124,9 +129,10 @@ struct HostModel {
 
   struct Entry { uint32_t bucket; uint64_t pos; };
 
-  // what both index builders start from: minInterestingSize :51-55, the longest length built and the capacity per length
-  bool index_plan(int max_used, int& hi, std::vector<int>& cap, std::string& err) {
-    min_interesting = j2i(std::max((std::log((double)(total_forward + 1)) / std::log(4.0)) - 2, 1.0));
+  // what both index builders start from: minInterestingSize :51-55 (or the one a caller passes, :68-89), the longest length built and
+  // the capacity per length
+  bool index_plan(int max_used, int& hi, std::vector<int>& cap, std::string& err, int min_interesting_size = -1) {
+    min_interesting = min_interesting_size > 0 ? min_interesting_size : j2i(std::max((std::log((double)(total_forward + 1)) / std::log(4.0)) - 2, 1.0));
     hi = std::max(max_used, 2 * choose_min_dup_len());
     cap.assign((size_t)hi + 1, 1);
     for (int n = 1; n <= hi; n++) { int c = estimate_capacity(n); cap[(size_t)n] = c < 1 ? 1 : c; }
@@ -313,7 +319,7 @@ struct HostModel {
   }
 
   // ---- duplication detector (DuplicationDetector.process :129-214, saveDuplications :332-400) ----
-  struct Dup { int length, count; };
+  struct Dup { int length, count; int group = -1; };   // group: the duplication group (M/Duplication.java object) when the merge keeps them
   static int compare_dups(int window, int s1, const Dup& d1, int s2, const Dup& d2) {  // :406-436
     if (window > 1) { if (s1 / window != s2 / window) return 0; }
     int e1 = s1 + d1.length, e2 = s2 + d2.length;
@@ -342,9 +348,32 @@ struct HostModel {
   // saveDuplications once per 10000 hashcodes, sequences and starts ascending within such a chunk, the last hashcode winning when a
   // chunk names a start twice.  Only forward-strand maps are kept: the table that is handed out (dup_starts) never reads the others.
   struct DupRecH { int32_t contig, st, count_len, hc; };   // count_len = count | length << 24
+  // A member of a duplication group as the group scan (xm_dup_scan_kernel<true>) finds it: every (sequence, start) of the group on both
+  // strands, sid = 2 * contig + (reverse strand), gid = the group's identity
+  struct DupGrpRec { int32_t sid, st, count_len, hc, gid; };
+  static int rec_group(const DupRecH&) { return -1; }
+  static int rec_group(const DupGrpRec& r) { return r.gid; }
+  // saveDuplications over the records of one unit (a stretch that no other unit's blocks interact with): sorts them into the reference's
+  // order - lengths ascending, one saveDuplications per 10000 hashcodes, starts ascending within such a chunk, the last hashcode winning
+  // when a chunk names a start twice - and returns the surviving map
+  template <class R>
+  static void merge_unit(R* lo, R* hi, int window, std::map<int, Dup>& m) {
+    const int chunk_len = 10000;
+    std::sort(lo, hi, [&](const R& a, const R& b) {
+      const int la = a.count_len >> 24, lb = b.count_len >> 24;
+      if (la != lb) return la < lb;
+      const int ca = a.hc / chunk_len, cb = b.hc / chunk_len;
+      if (ca != cb) return ca < cb;
+      if (a.st != b.st) return a.st < b.st;
+      return a.hc < b.hc;
+    });
+    for (R* r = lo; r < hi; r++) {
+      if (r + 1 < hi) { const R& x = r[1]; if ((x.count_len >> 24) == (r->count_len >> 24) && x.hc / chunk_len == r->hc / chunk_len && x.st == r->st) continue; }
+      dup_insert(m, window, r->st, Dup{r->count_len >> 24, r->count_len & 0xFFFFFF, rec_group(*r)});
+    }
+  }
   void merge_duplications(std::vector<DupRecH>& recs, int min_len, int window) {
     dup_window = window; dup_granularity = gapmers ? (double)(min_len * 5 / 8) : (double)min_len;  // :67-77
-    const int chunk_len = 10000;
     // Units that cannot interact are merged by different threads: contigs, and - when window > 1, where compareDuplications :406-436
     // only relates blocks of one window - stretches of whole windows within a contig.
     const long long seg = window > 1 ? (long long)window * ((1000000 + window - 1) / window) : (1LL << 40);
@@ -365,19 +394,8 @@ struct HostModel {
         if (u >= n_units) break;
         DupRecH* lo = by_unit.data() + first[u]; DupRecH* hi = by_unit.data() + first[u + 1];
         if (lo == hi) continue;
-        std::sort(lo, hi, [&](const DupRecH& a, const DupRecH& b) {
-          const int la = a.count_len >> 24, lb = b.count_len >> 24;
-          if (la != lb) return la < lb;
-          const int ca = a.hc / chunk_len, cb = b.hc / chunk_len;
-          if (ca != cb) return ca < cb;
-          if (a.st != b.st) return a.st < b.st;
-          return a.hc < b.hc;
-        });
         std::map<int, Dup> m;
-        for (DupRecH* r = lo; r < hi; r++) {
-          if (r + 1 < hi) { const DupRecH& x = r[1]; if ((x.count_len >> 24) == (r->count_len >> 24) && x.hc / chunk_len == r->hc / chunk_len && x.st == r->st) continue; }
-          dup_insert(m, window, r->st, Dup{r->count_len >> 24, r->count_len & 0xFFFFFF});
-        }
+        merge_unit(lo, hi, window, m);
         for (auto& e : m) unit_starts[u].push_back(e.first);
       }
     };
@@ -389,6 +407,33 @@ struct HostModel {
     for (int c = 0; c < n_contigs; c++)
       for (long long u = unit_base[(size_t)c]; u < unit_base[(size_t)c + 1]; u++) dup_starts[(size_t)c].insert(dup_starts[(size_t)c].end(), unit_starts[(size_t)u].begin(), unit_starts[(size_t)u].end());
     dup_set = true; dup_generation++;
+  }
+  // The same merge for the ancestry detector (window 1, M/Mapper.java:675-681): the maps of all 2 * n_contigs sequences - bounds and
+  // interest are looked up in the map of a member's own sequence, which may be a reverse one - with the group of every surviving entry.
+  // With window 1 a unit is a sequence.  by_seq[sid]: (start, Dup) in start order.  Leaves the handle's own duplication table alone.
+  void merge_duplication_groups(const std::vector<DupGrpRec>& recs, int window, std::vector<std::vector<std::pair<int32_t, Dup>>>& by_seq) const {
+    const size_t n_seqs = 2 * (size_t)n_contigs;
+    std::vector<size_t> first(n_seqs + 1, 0);
+    for (const DupGrpRec& r : recs) first[(size_t)r.sid + 1]++;
+    for (size_t s = 0; s < n_seqs; s++) first[s + 1] += first[s];
+    std::vector<DupGrpRec> by_unit(recs.size());
+    { std::vector<size_t> at(first.begin(), first.end() - 1); for (const DupGrpRec& r : recs) by_unit[at[(size_t)r.sid]++] = r; }
+    by_seq.assign(n_seqs, {});
+    std::atomic<size_t> next(0);
+    auto work = [&]() {
+      while (true) {
+        const size_t s = next.fetch_add(1);
+        if (s >= n_seqs) break;
+        if (first[s] == first[s + 1]) continue;
+        std::map<int, Dup> m;
+        merge_unit(by_unit.data() + first[s], by_unit.data() + first[s + 1], window, m);
+        by_seq[s].assign(m.begin(), m.end());
+      }
+    };
+    unsigned hw = std::thread::hardware_concurrency();
+    const int n_thr = (int)std::max<size_t>(1, std::min<size_t>(std::min<size_t>(hw ? hw : 1u, 32u), std::min(n_seqs, recs.size() / 4096 + 1)));
+    if (n_thr == 1) work();
+    else { std::vector<std::thread> th; for (int t = 0; t < n_thr; t++) th.emplace_back(work); for (auto& x : th) x.join(); }
   }
   // via_merge: the blocks this scan finds go through merge_duplications (the path the device scan feeds) instead of the maps below -
   // how the CPU tests check that routine against this one
