@@ -222,6 +222,46 @@ int xm_counts_device_ptr(xm_handle* h, void** d_ptr, int64_t* n_int32);
 int xm_counts_fetch(xm_handle* h, int32_t contig, int32_t* out /* 4 * contig length */);
 int xm_variants_fetch(xm_handle* h, int64_t* n, uint64_t* keys, int32_t* counts, int64_t* ex_gid, int32_t* ex_index /* NULL arrays: size query */);
 
+/* VCF and mutations BODIES formatted on the device from the count planes and the variant table (QV/VcfFormatterWorker.java:27-159,
+ * QV/MutationsFormatterWorker.java:25-147 over QV/FilteredAlignments; the headers embed the command line and stay with the host, as
+ * do the file writer and the order of the contigs: VcfWriter / MutationsWriter visit them in the TreeMap order of their names,
+ * :111-114, and the library does not sort names).  The host asks for one forward contig and a range of positions [start, end) at a
+ * time, of any size it likes:
+ *   - the VCF text of any split of [0, contig length) concatenates to the text of the whole contig;
+ *   - so does the mutations text of any split at multiples of 8192 (start % 8192 == 0, end % 8192 == 0 or end == contig length):
+ *     a run of deletions is reported per writer job of 8192 positions, so a run that crosses a job boundary is two records.
+ * The text is placed in a pinned host buffer owned by the handle; *text stays valid until the next xm_format_vcf /
+ * xm_format_mutations on the handle, or xm_destroy.  Format calls are ordered with xm_align_batch on the same handle.  Every
+ * entry point of this library may be called by concurrent threads on one handle.
+ * After xm_counts_reduce every rank holds the planes and the table of the whole run, so any rank can format any contig and the
+ * ranks may split the contigs between them.
+ * Errors: counts not enabled -> XM_ERR_STATE; a bad contig or range, a mutations range not on the 8192 grid -> XM_ERR_ARG. */
+/* MutationDetectionParameters (QV/MutationDetectionParameters.java): the six thresholds of FilteredAlignments.  All zero (or a NULL
+ * filter) = MutationDetectionParameters.emptyFilter(). */
+typedef struct xm_variant_filter {
+  float min_snp_total_depth, min_snp_depth_fraction;
+  float min_indel_start_total_depth, min_indel_start_depth_fraction;
+  float min_indel_continuation_total_depth, min_indel_continuation_depth_fraction;
+} xm_variant_filter;
+/* The reads the VCF support column can show: the distinct global sequence ids (ascending) of the examples of the current variant
+ * table.  gids == NULL: size query.  Reduces pending records first, like xm_variants_fetch. */
+int xm_variants_examples(xm_handle* h, int64_t* n, int64_t* gids);
+/* The forward texts of exactly those sequences, in that order: gids as xm_variants_examples listed them, then the reads packed as
+ * xm_align_batch takes them (seq_word_off has n + 1 entries).  The "-rev" view of an example (ex_gid & 1) is made on the device.
+ * A count, id or order that differs from xm_variants_examples, or a read whose length is not the length of the read that was
+ * counted, returns XM_ERR_ARG.  The upload belongs to the table as it is now: a later batch, xm_counts_reduce or xm_counts_enable
+ * makes it stale. */
+int xm_variants_set_examples(xm_handle* h, int64_t n, const int64_t* gids, const uint16_t* packed4, const int64_t* seq_word_off, const int32_t* seq_len);
+/* VcfFormatterWorker.format over positions [start, end) of forward contig `contig`, named contig_name: body lines only.
+ * show_support != 0 needs the examples of the current table (xm_variants_set_examples), else XM_ERR_STATE; show_support == 0 needs
+ * none.  Reference characters are the handle's reference codes (IUPAC letters on ambiguous references). */
+int xm_format_vcf(xm_handle* h, int32_t contig, const char* contig_name, int64_t start, int64_t end, const xm_variant_filter* f,
+                  int32_t include_non_mutations, int32_t show_support, const char** text, int64_t* n_bytes);
+/* MutationsFormatterWorker.format over [start, end) of forward contig `contig` (start % 8192 == 0; end % 8192 == 0 or end == contig
+ * length); needs no examples. */
+int xm_format_mutations(xm_handle* h, int32_t contig, const char* contig_name, int64_t start, int64_t end, const xm_variant_filter* f,
+                        const char** text, int64_t* n_bytes);
+
 /* Measurement aid (bench.py's roofline): sustained issue rates of this GPU, in warp-instructions per second over the whole chip,
  * from three micro-benchmark kernels timed with CUDA events - out[0] INT32 (IMAD chains), out[1] FP64 (DADD chains), out[2] FP32
  * FFMA chains (full-rate pipe: the issue-slot ceiling); out[3] = number of SMs, out[4] = maximum SM clock in Hz.  SURVEY.md §8(d) takes the relevant

@@ -16,7 +16,8 @@ EXPORTS = ["xm_create", "xm_destroy", "xm_last_error", "xm_set_reference", "xm_s
            "xm_set_index_length_wide", "xm_build_index", "xm_get_index_length", "xm_get_index_length_wide", "xm_index_info", "xm_set_duplications", "xm_build_duplications", "xm_build_duplications_host",
            "xm_get_duplications", "xm_infer_ancestors", "xm_get_reference", "xm_align_batch", "xm_align_batch_device", "xm_results_array", "xm_release_results",
            "xm_counts_enable", "xm_counts_device_ptr", "xm_counts_fetch", "xm_format_sam",
-           "xm_comm_unique_id", "xm_comm_init", "xm_counts_reduce", "xm_counts_batch_info", "xm_variants_fetch", "xm_measure_peaks", "xm_counts_reduce_times"]
+           "xm_comm_unique_id", "xm_comm_init", "xm_counts_reduce", "xm_counts_batch_info", "xm_variants_fetch", "xm_measure_peaks", "xm_counts_reduce_times",
+           "xm_variants_examples", "xm_variants_set_examples", "xm_format_vcf", "xm_format_mutations"]
 
 RESULT_ARRAYS = [("q_comp_off", np.int64), ("comp_choice_off", np.int64), ("choice_sa_off", np.int64), ("sa_block_off", np.int64),
                  ("choice_f64", np.float64), ("sa_f64", np.float64), ("choice_inner", np.int32), ("sa_contig", np.int32),
@@ -31,6 +32,29 @@ class XmParams(C.Structure):
                 ("deletion_start_penalty", C.c_double), ("deletion_extension_penalty", C.c_double), ("max_error_rate", C.c_double),
                 ("unaligned_penalty", C.c_double), ("ambiguity_penalty", C.c_double), ("max_penalty_span", C.c_double),
                 ("max_num_matches", C.c_int32), ("enable_gapmers", C.c_int32)]
+
+
+class XmVariantFilter(C.Structure):
+    _fields_ = [("min_snp_total_depth", C.c_float), ("min_snp_depth_fraction", C.c_float),
+                ("min_indel_start_total_depth", C.c_float), ("min_indel_start_depth_fraction", C.c_float),
+                ("min_indel_continuation_total_depth", C.c_float), ("min_indel_continuation_depth_fraction", C.c_float)]
+
+
+# MutationDetectionParameters field names -> xm_variant_filter fields
+FILTER_FIELDS = dict(minSNPTotalDepth="min_snp_total_depth", minSNPDepthFraction="min_snp_depth_fraction",
+                     minIndelTotalStartDepth="min_indel_start_total_depth", minIndelStartDepthFraction="min_indel_start_depth_fraction",
+                     minIndelContinuationTotalDepth="min_indel_continuation_total_depth",
+                     minIndelContinuationDepthFraction="min_indel_continuation_depth_fraction")
+
+
+def to_xm_filter(flt):
+    """flt: None (the empty filter) or a dict keyed by FILTER_FIELDS' names (missing thresholds are 0)."""
+    f = XmVariantFilter()
+    for k, v in (flt or {}).items():
+        if k not in FILTER_FIELDS:
+            raise ValueError("unknown filter threshold %r (expected one of %s)" % (k, ", ".join(FILTER_FIELDS)))
+        setattr(f, FILTER_FIELDS[k], float(v))
+    return f
 
 
 _LIB = None
@@ -328,3 +352,39 @@ class XMapper:
         out = np.zeros(4 * self.contig_lengths[contig], dtype=np.int32)
         self._ok(self.L.xm_counts_fetch(self.h, contig, _ptr(out)))
         return out.reshape(2, 2, -1)
+
+    # ---- VCF / mutations bodies ----
+    def variants_examples(self):
+        """The global sequence ids (ascending) whose reads the VCF support column of the current variant table can show."""
+        n = C.c_int64()
+        self._ok(self.L.xm_variants_examples(self.h, C.byref(n), None))
+        out = np.zeros(max(n.value, 1), dtype=np.int64)
+        self._ok(self.L.xm_variants_examples(self.h, C.byref(n), _ptr(out)))
+        return out[:n.value]
+
+    def set_variant_examples(self, codes_by_gid):
+        """Uploads the forward reads of variants_examples(): codes_by_gid maps a global sequence id to its uint8 codes."""
+        from mapper_b200 import synth
+        gids = self.variants_examples()
+        packed = [synth.pack_contig(np.asarray(codes_by_gid[int(g)], dtype=np.uint8)) for g in gids]
+        lens = np.array([len(codes_by_gid[int(g)]) for g in gids], dtype=np.int32)
+        off = np.zeros(len(gids) + 1, dtype=np.int64)
+        if len(gids):
+            off[1:] = np.cumsum([len(p) for p in packed])
+        words = np.concatenate(packed + [np.zeros(1, dtype=np.uint16)])
+        self._ok(self.L.xm_variants_set_examples(self.h, C.c_int64(len(gids)), _ptr(np.ascontiguousarray(gids)), _ptr(words), _ptr(off), _ptr(lens)))
+
+    def format_vcf(self, contig, name, start, end, flt=None, include_non_mutations=True, show_support=True):
+        """VCF body lines of positions [start, end) of contig `contig`; flt: dict of MutationDetectionParameters thresholds or None."""
+        f = to_xm_filter(flt)
+        text, n = C.c_char_p(), C.c_int64()
+        self._ok(self.L.xm_format_vcf(self.h, int(contig), name.encode(), C.c_int64(start), C.c_int64(end), C.byref(f), int(bool(include_non_mutations)),
+                                      int(bool(show_support)), C.byref(text), C.byref(n)))
+        return C.string_at(text, n.value).decode()
+
+    def format_mutations(self, contig, name, start, end, flt=None):
+        """Mutations body lines of [start, end) of contig `contig` (start and end on the 8192 grid, or end = the contig length)."""
+        f = to_xm_filter(flt)
+        text, n = C.c_char_p(), C.c_int64()
+        self._ok(self.L.xm_format_mutations(self.h, int(contig), name.encode(), C.c_int64(start), C.c_int64(end), C.byref(f), C.byref(text), C.byref(n)))
+        return C.string_at(text, n.value).decode()

@@ -663,63 +663,7 @@ struct SamD {
   long long* q_len;                         // per query: bytes of text (count pass), then exclusive offsets
   char* text;
 };
-struct SamOut {
-  char* p; long long n;
-  __device__ __forceinline__ void ch(char c) { if (p) p[n] = c; n++; }
-  __device__ void str(const char* s, long long len) { for (long long i = 0; i < len; i++) ch(s[i]); }
-  __device__ void lit(const char* s) { while (*s) ch(*s++); }
-  __device__ void num(long long v) {  // "" + int
-    if (v < 0) { ch('-'); v = -v; }
-    char d[20]; int k = 0;
-    do { d[k++] = (char)('0' + (int)(v % 10)); v /= 10; } while (v);
-    while (k) ch(d[--k]);
-  }
-  // Java Float.toString of a finite float: shortest digits that identify it; decimal form for 1e-3 <= |v| < 1e7, else d.dddE<n>
-  __device__ void jfloat(float v) {
-    if (v == 0.0f) { if (signbit(v)) ch('-'); lit("0.0"); return; }
-    if (v < 0) { ch('-'); v = -v; }
-    const double s = (double)v;
-    // powers of ten are exact doubles up to 1e22; negative exponents divide by the exact power instead of multiplying by an inexact one
-    auto p10 = [](int k) { double r = 1.0; for (int i = 0; i < k; i++) r *= 10.0; return r; };
-    auto scale = [&](double x, int ex) { return ex >= 0 ? x * p10(ex) : x / p10(-ex); };  // x * 10^ex
-    int e10 = (int)floor(log10(s));
-    if (scale(1.0, e10) > s) e10--;
-    if (scale(1.0, e10 + 1) <= s) e10++;
-    unsigned long long D = 0; int p = 1;
-    for (p = 1; p <= 9; p++) {
-      const int ex = e10 - p + 1;               // candidate = D * 10^ex with p digits
-      D = (unsigned long long)rint(scale(s, -ex));
-      if ((float)scale((double)D, ex) == v) break;
-    }
-    if (p > 9) p = 9;
-    { unsigned long long lim = 1; for (int i = 0; i < p; i++) lim *= 10; if (D >= lim) { D /= 10; e10++; } }  // rounding carried into a new digit
-    while (p > 1 && D % 10 == 0) { D /= 10; p--; }
-    char dg[12];
-    { unsigned long long t = D; for (int i = p - 1; i >= 0; i--) { dg[i] = (char)('0' + (int)(t % 10)); t /= 10; } }
-    if (s >= 1e-3 && s < 1e7) {
-      if (e10 >= 0) {
-        for (int i = 0; i <= e10; i++) ch(i < p ? dg[i] : '0');
-        ch('.');
-        if (p > e10 + 1) { for (int i = e10 + 1; i < p; i++) ch(dg[i]); } else ch('0');
-      } else {
-        lit("0.");
-        for (int i = 0; i < -e10 - 1; i++) ch('0');
-        for (int i = 0; i < p; i++) ch(dg[i]);
-      }
-    } else {
-      ch(dg[0]); ch('.');
-      if (p > 1) { for (int i = 1; i < p; i++) ch(dg[i]); } else ch('0');
-      ch('E'); num(e10);
-    }
-  }
-  __device__ void score(const char* tag, double penalty) {  // formatSequencePenalty / formatQueryPenalty / formatNumber :263-277
-    const float sc = (float)(-1 * penalty);
-    const double scaled = (double)sc * (double)10000.0f;
-    const long long r = (long long)floor(scaled + 0.5);        // Math.round(double)
-    const float rounded = (float)r / 10000.0f;                 // long / float -> float
-    lit(tag); lit("f:"); jfloat(rounded);
-  }
-};
+#include "xm_text.cuh"
 template <bool WRITE>
 __global__ void xm_sam_kernel(SamD S, BatchD batch, int nq) {
   const int q = blockIdx.x * blockDim.x + threadIdx.x;
@@ -810,6 +754,7 @@ struct DevBuf {
 };
 
 #include "xm_counts.cuh"
+#include "xm_variants_fmt.cuh"
 
 // pinned host slabs for results, recycled between batches (cudaHostAlloc of 100 MB costs tens of ms)
 struct PinnedPool {
@@ -927,6 +872,13 @@ struct xm_handle {
   unsigned long long var_n = 0, var_cap = 0, var_reduced_n = 0;
   long long next_gid = 0;                       // global id of the first sequence of the next batch (xm_counts_batch_info overrides it)
   bool have_batch_info = false; long long info_first_gid = 0; std::vector<int64_t> info_order;
+  // VCF / mutations bodies (xm_variants_fmt.cuh).  var_gen changes whenever the planes or the table do (a batch accumulates, a reduce
+  // runs, counts are enabled); the example list and the uploaded example texts belong to the generation they were made for.
+  unsigned long long var_gen = 0, ex_list_gen = ~0ull, ex_gen = ~0ull;
+  std::vector<int64_t> ex_list;
+  DevBuf d_ex_words, d_ex_word_off, d_ex_len, d_ex_gids, d_ex_slot, d_ex_bad;
+  DevBuf d_fmt_dec, d_fmt_state, d_fmt_len, d_fmt_range, d_fmt_name, d_fmt_text, d_fmt_tmp, d_fmt_ids;
+  void* fmt_text = nullptr; size_t fmt_cap = 0;   // pinned text of the latest xm_format_vcf / xm_format_mutations
   ncclComm_t comm = nullptr; int comm_ranks = 0, comm_rank = 0;
   double last_planes_ms = 0, last_variants_ms = 0;   // xm_counts_reduce: device time of the plane all-reduce, wall time of the variant-table exchange   // xm_comm_init: the communicator xm_counts_reduce uses
 };
@@ -1421,8 +1373,11 @@ void xm_destroy(xm_handle* h) {
   }
   DevBuf* bufs[] = {&h->d_words, &h->d_word_off, &h->d_len, &h->d_gstart, &h->d_tables, &h->d_dup_off, &h->d_dup_starts, &h->d_chunk, &h->d_q, &h->d_choices, &h->d_sas, &h->d_blocks,
                     &h->d_misc, &h->d_ids_a, &h->d_ids_b, &h->d_ids_full, &h->d_ws, &h->d_qcycles, &h->d_csr_cnt, &h->d_csr_base, &h->d_csr_tmp, &h->d_keys_a, &h->d_keys_b, &h->d_sort_tmp, &h->d_big, &h->d_big_busy, &h->d_sam_len, &h->d_sam_text, &h->d_sam_names, &h->d_sam_name_off, &h->d_sam_cnames, &h->d_sam_cname_off, &h->d_svc, &h->d_planes, &h->d_contig_off, &h->d_var, &h->d_var_n, &h->d_order, &h->d_var_sizes,
-                    &h->var_scratch.keys_a, &h->var_scratch.keys_b, &h->var_scratch.idx_a, &h->var_scratch.idx_b, &h->var_scratch.gathered, &h->var_scratch.out_keys, &h->var_scratch.n_out, &h->var_scratch.tmp};
+                    &h->var_scratch.keys_a, &h->var_scratch.keys_b, &h->var_scratch.idx_a, &h->var_scratch.idx_b, &h->var_scratch.gathered, &h->var_scratch.out_keys, &h->var_scratch.n_out, &h->var_scratch.tmp,
+                    &h->d_ex_words, &h->d_ex_word_off, &h->d_ex_len, &h->d_ex_gids, &h->d_ex_slot, &h->d_ex_bad,
+                    &h->d_fmt_dec, &h->d_fmt_state, &h->d_fmt_len, &h->d_fmt_range, &h->d_fmt_name, &h->d_fmt_text, &h->d_fmt_tmp, &h->d_fmt_ids};
   for (DevBuf* b : bufs) b->release();
+  if (h->fmt_text) h->pinned->give(h->fmt_text, h->fmt_cap);
   for (auto& b : h->d_buckets) b.release();
   for (auto& b : h->d_positions) b.release();
   for (auto& b : h->d_positions_hi) b.release();
@@ -1980,6 +1935,7 @@ struct CountsPending { CountsD C; VarOut V; };
 static int counts_enqueue(xm_handle* h, const LaunchD& L, int nq, long long n_seqs_total, int& launches, CountsPending& P, unsigned long long* n_after) {
   cudaStream_t st = h->stream;
   CountsD& C = P.C; VarOut& V = P.V;
+  h->var_gen++;
   C.planes = (int32_t*)h->d_planes.p; C.contig_off = (const int64_t*)h->d_contig_off.p; C.end_fraction = h->end_fraction;
   V.order = nullptr;
   V.first_gid = h->have_batch_info ? h->info_first_gid : h->next_gid;
@@ -2455,6 +2411,7 @@ int xm_counts_enable(xm_handle* h, double query_end_fraction) {
   CK(cudaStreamSynchronize(h->stream));
   h->end_fraction = query_end_fraction; h->counts_enabled = true;
   h->var_n = 0; h->var_reduced_n = 0; h->next_gid = 0; h->have_batch_info = false;
+  h->var_gen++;
   return XM_OK;
 }
 int xm_comm_unique_id(uint8_t* id128) {
@@ -2487,6 +2444,7 @@ int xm_counts_reduce(xm_handle* h) {
   CK(cudaSetDevice(h->device));
   cudaStream_t st = h->stream;
   // int32 sums are exact and order-free: every rank ends with the planes of the whole run (QV/DirectionalAlignments.java:20-28)
+  h->var_gen++;
   CK(cudaEventRecord(h->ev2, st));
   ncclResult_t r = N.AllReduce(h->d_planes.p, h->d_planes.p, (size_t)h->n_plane_ints, ncclInt32, ncclSum, h->comm, st);
   if (r != ncclSuccess) { h->err = std::string("ncclAllReduce: ") + N.GetErrorString(r); return XM_ERR_CUDA; }
@@ -2564,6 +2522,162 @@ int xm_variants_fetch(xm_handle* h, int64_t* n, uint64_t* keys, int32_t* counts,
     if (ex_index) ex_index[i] = host[i].ex_index;
   }
   return XM_OK;
+}
+
+// ---- VCF / mutations bodies (xm_variants_fmt.cuh) ----
+// the sorted distinct example ids of the current table, cached for its generation
+static int ex_list_refresh(xm_handle* h) {
+  int rc = var_reduce_now(h);
+  if (rc != XM_OK) return rc;
+  if (h->ex_list_gen == h->var_gen) return XM_OK;
+  cudaStream_t st = h->stream;
+  const unsigned long long n = h->var_n;
+  h->ex_list.clear();
+  if (n) {
+    const int ni = (int)n;
+    size_t t1 = 0, t2 = 0;
+    cub::DeviceRadixSort::SortKeys(nullptr, t1, (const unsigned long long*)nullptr, (unsigned long long*)nullptr, ni, 0, 64, st);
+    cub::DeviceSelect::Unique(nullptr, t2, (const unsigned long long*)nullptr, (unsigned long long*)nullptr, (int*)nullptr, ni, st);
+    const size_t tb = (t1 > t2 ? t1 : t2) + 256;
+    if (!h->d_fmt_ids.ensure((size_t)n * 16 + 16) || !h->d_fmt_tmp.ensure(tb)) { h->err = "out of device memory (variant examples)"; return XM_ERR_CUDA; }
+    unsigned long long* a = (unsigned long long*)h->d_fmt_ids.p;
+    unsigned long long* b = a + n;
+    int* d_count = (int*)(b + n);
+    xm_ex_ids_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const VarRec*)h->d_var.p, n, a);
+    size_t q = tb;
+    CK(cub::DeviceRadixSort::SortKeys(h->d_fmt_tmp.p, q, a, b, ni, 0, 64, st));
+    q = tb;
+    CK(cub::DeviceSelect::Unique(h->d_fmt_tmp.p, q, b, a, d_count, ni, st));
+    int count = 0;
+    CK(cudaMemcpyAsync(&count, d_count, 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    h->ex_list.resize((size_t)count);
+    CK(cudaMemcpyAsync(h->ex_list.data(), a, (size_t)count * 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+  }
+  h->ex_list_gen = h->var_gen;
+  return XM_OK;
+}
+int xm_variants_examples(xm_handle* h, int64_t* n, int64_t* gids) {
+  if (!h || !n) return XM_ERR_ARG;
+  if (!h->counts_enabled) { h->err = "xm_variants_examples: counts are not enabled"; return XM_ERR_STATE; }
+  std::lock_guard<std::mutex> compute(h->compute_mu);
+  CK(cudaSetDevice(h->device));
+  int rc = ex_list_refresh(h);
+  if (rc != XM_OK) return rc;
+  *n = (int64_t)h->ex_list.size();
+  if (gids) for (size_t i = 0; i < h->ex_list.size(); i++) gids[i] = h->ex_list[i];
+  return XM_OK;
+}
+int xm_variants_set_examples(xm_handle* h, int64_t n, const int64_t* gids, const uint16_t* packed4, const int64_t* seq_word_off, const int32_t* seq_len) {
+  if (!h || n < 0 || (n > 0 && (!gids || !packed4 || !seq_word_off || !seq_len))) return XM_ERR_ARG;
+  if (!h->counts_enabled) { h->err = "xm_variants_set_examples: counts are not enabled"; return XM_ERR_STATE; }
+  std::lock_guard<std::mutex> compute(h->compute_mu);
+  CK(cudaSetDevice(h->device));
+  int rc = ex_list_refresh(h);
+  if (rc != XM_OK) return rc;
+  h->ex_gen = ~0ull;
+  if ((size_t)n != h->ex_list.size()) { h->err = "xm_variants_set_examples: " + std::to_string(n) + " sequences given, the variant table names " + std::to_string(h->ex_list.size()); return XM_ERR_ARG; }
+  for (int64_t i = 0; i < n; i++) {
+    if (gids[i] != h->ex_list[(size_t)i]) { h->err = "xm_variants_set_examples: sequence " + std::to_string(i) + " is not the one xm_variants_examples lists there"; return XM_ERR_ARG; }
+    if (seq_len[i] < 0 || seq_word_off[i] < 0 || seq_word_off[i] + (seq_len[i] + 3) / 4 > seq_word_off[n]) { h->err = "xm_variants_set_examples: sequence " + std::to_string(i) + " lies outside packed4"; return XM_ERR_ARG; }
+  }
+  cudaStream_t st = h->stream;
+  const size_t n_words = n ? (size_t)seq_word_off[n] : 0;
+  if (!h->d_ex_words.ensure(n_words * 2 + 16) || !h->d_ex_word_off.ensure((size_t)n * 8 + 16) || !h->d_ex_len.ensure((size_t)n * 4 + 16) ||
+      !h->d_ex_gids.ensure((size_t)n * 8 + 16) || !h->d_ex_slot.ensure((size_t)h->var_n * 4 + 16) || !h->d_ex_bad.ensure(16)) { h->err = "out of device memory (variant examples)"; return XM_ERR_CUDA; }
+  if (n) {
+    CK(cudaMemcpyAsync(h->d_ex_words.p, packed4, n_words * 2, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(h->d_ex_word_off.p, seq_word_off, (size_t)n * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(h->d_ex_len.p, seq_len, (size_t)n * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(h->d_ex_gids.p, gids, (size_t)n * 8, cudaMemcpyHostToDevice, st));
+  }
+  CK(cudaMemsetAsync(h->d_ex_bad.p, 0, 4, st));
+  if (h->var_n)
+    xm_ex_slot_kernel<<<(unsigned)((h->var_n + 255) / 256), 256, 0, st>>>((const VarRec*)h->d_var.p, h->var_n, (const int64_t*)h->d_ex_gids.p, (int)n,
+                                                                          (const int32_t*)h->d_ex_len.p, (int32_t*)h->d_ex_slot.p, (unsigned int*)h->d_ex_bad.p);
+  unsigned int bad = 0;
+  CK(cudaMemcpyAsync(&bad, h->d_ex_bad.p, 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  CK(cudaGetLastError());
+  if (bad) { h->err = "xm_variants_set_examples: " + std::to_string(bad) + " table entries name a read whose given length differs from the read they counted"; return XM_ERR_ARG; }
+  h->ex_gen = h->var_gen;
+  return XM_OK;
+}
+static int format_variants(xm_handle* h, int mode, int32_t contig, const char* contig_name, int64_t start, int64_t end, const xm_variant_filter* f,
+                           int32_t include_non_mutations, int32_t show_support, const char** text, int64_t* n_bytes) {
+  const char* fn = mode == XM_FMT_VCF ? "xm_format_vcf" : "xm_format_mutations";
+  if (!h || !contig_name || !text || !n_bytes) return XM_ERR_ARG;
+  *text = ""; *n_bytes = 0;
+  if (!h->counts_enabled) { h->err = std::string(fn) + ": counts are not enabled"; return XM_ERR_STATE; }
+  if (contig < 0 || contig >= h->m.n_contigs) { h->err = std::string(fn) + ": no contig " + std::to_string(contig); return XM_ERR_ARG; }
+  const long long len = h->m.len[(size_t)contig];
+  if (start < 0 || start > end || end > len) { h->err = std::string(fn) + ": range [" + std::to_string(start) + ", " + std::to_string(end) + ") is not inside [0, " + std::to_string(len) + ")"; return XM_ERR_ARG; }
+  if (mode == XM_FMT_MUT && (start % XM_FMT_JOB != 0 || (end % XM_FMT_JOB != 0 && end != len))) { h->err = "xm_format_mutations: start and end must be multiples of 8192 (end may be the contig length)"; return XM_ERR_ARG; }
+  std::lock_guard<std::mutex> compute(h->compute_mu);
+  CK(cudaSetDevice(h->device));
+  int rc = mirror_model(h);
+  if (rc != XM_OK) return rc;
+  rc = var_reduce_now(h);
+  if (rc != XM_OK) return rc;
+  if (show_support && h->ex_gen != h->var_gen) { h->err = "xm_format_vcf: the support column needs the example reads of the current variant table (xm_variants_examples, xm_variants_set_examples)"; return XM_ERR_STATE; }
+  const long long n = end - start;
+  if (n == 0) return XM_OK;
+  if (n + 1 >= (1ll << 31)) { h->err = std::string(fn) + ": ranges hold fewer than 2^31 - 1 positions"; return XM_ERR_ARG; }
+  cudaStream_t st = h->stream;
+  const size_t name_len = strlen(contig_name);
+  if (!h->d_fmt_dec.ensure((size_t)n + 16) || !h->d_fmt_state.ensure((size_t)n + 16) || !h->d_fmt_len.ensure(((size_t)n + 1) * 8) || !h->d_fmt_range.ensure(16) ||
+      !h->d_fmt_name.ensure(name_len + 16) || !h->d_ex_slot.ensure(16)) { h->err = std::string("out of device memory (") + fn + ")"; return XM_ERR_CUDA; }
+  CK(cudaMemcpyAsync(h->d_fmt_name.p, contig_name, name_len, cudaMemcpyHostToDevice, st));
+  FmtD D;
+  D.ref = h->ref; D.planes = (const int32_t*)h->d_planes.p; D.contig_off = (const int64_t*)h->d_contig_off.p;
+  D.recs = (const VarRec*)h->d_var.p; D.n_recs = h->var_n; D.range = (unsigned long long*)h->d_fmt_range.p;
+  D.contig = contig; D.start = start; D.end = end;
+  D.f = VarFilter{0, 0, 0, 0, 0, 0};
+  if (f) D.f = VarFilter{f->min_snp_total_depth, f->min_snp_depth_fraction, f->min_indel_start_total_depth, f->min_indel_start_depth_fraction,
+                         f->min_indel_continuation_total_depth, f->min_indel_continuation_depth_fraction};
+  D.name = (const char*)h->d_fmt_name.p; D.name_len = (int)name_len;
+  D.include_non_mutations = include_non_mutations ? 1 : 0; D.show_support = (mode == XM_FMT_VCF && show_support) ? 1 : 0;
+  D.dec = (uint8_t*)h->d_fmt_dec.p; D.could_delete = (const uint8_t*)h->d_fmt_state.p; D.len = (long long*)h->d_fmt_len.p; D.text = nullptr;
+  D.ex_slot = (const int32_t*)h->d_ex_slot.p; D.ex_words = (const uint16_t*)h->d_ex_words.p; D.ex_word_off = (const int64_t*)h->d_ex_word_off.p; D.ex_len = (const int32_t*)h->d_ex_len.p;
+  const unsigned blocks = (unsigned)((n + 127) / 128);
+  xm_fmt_carry_kernel<<<1, 256, 0, st>>>(D);
+  xm_fmt_decide_kernel<<<blocks, 128, 0, st>>>(D);
+  size_t t1 = 0, t2 = 0;
+  cub::DeviceScan::InclusiveScan(nullptr, t1, (const uint8_t*)nullptr, (uint8_t*)nullptr, FmtLastDecisive(), (int)(n + 1), st);
+  cub::DeviceScan::ExclusiveSum(nullptr, t2, (const long long*)nullptr, (long long*)nullptr, (int)(n + 1), st);
+  const size_t tb = (t1 > t2 ? t1 : t2) + 256;
+  if (!h->d_fmt_tmp.ensure(tb)) { h->err = std::string("out of device memory (") + fn + ")"; return XM_ERR_CUDA; }
+  size_t q = tb;
+  CK(cub::DeviceScan::InclusiveScan(h->d_fmt_tmp.p, q, D.dec, (uint8_t*)h->d_fmt_state.p, FmtLastDecisive(), (int)(n + 1), st));
+  CK(cudaMemsetAsync(D.len + n, 0, 8, st));
+  if (mode == XM_FMT_VCF) xm_fmt_kernel<XM_FMT_VCF, false><<<blocks, 128, 0, st>>>(D); else xm_fmt_kernel<XM_FMT_MUT, false><<<blocks, 128, 0, st>>>(D);
+  q = tb;
+  CK(cub::DeviceScan::ExclusiveSum(h->d_fmt_tmp.p, q, (const long long*)D.len, D.len, (int)(n + 1), st));
+  long long total = 0;
+  CK(cudaMemcpyAsync(&total, D.len + n, 8, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  CK(cudaGetLastError());
+  if (!h->d_fmt_text.ensure((size_t)total + 16)) { h->err = std::string("out of device memory (") + fn + " text)"; return XM_ERR_CUDA; }
+  D.text = (char*)h->d_fmt_text.p;
+  if (mode == XM_FMT_VCF) xm_fmt_kernel<XM_FMT_VCF, true><<<blocks, 128, 0, st>>>(D); else xm_fmt_kernel<XM_FMT_MUT, true><<<blocks, 128, 0, st>>>(D);
+  CK(cudaGetLastError());
+  if (h->fmt_text && h->fmt_cap < (size_t)total + 1) { h->pinned->give(h->fmt_text, h->fmt_cap); h->fmt_text = nullptr; }
+  if (!h->fmt_text) h->fmt_text = h->pinned->take((size_t)total + 1, h->fmt_cap);
+  if (!h->fmt_text) { h->err = std::string("out of pinned host memory (") + fn + " text)"; return XM_ERR_CUDA; }
+  CK(cudaMemcpyAsync(h->fmt_text, D.text, (size_t)total, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  ((char*)h->fmt_text)[(size_t)total] = 0;
+  *text = (const char*)h->fmt_text; *n_bytes = total;
+  return XM_OK;
+}
+int xm_format_vcf(xm_handle* h, int32_t contig, const char* contig_name, int64_t start, int64_t end, const xm_variant_filter* f,
+                  int32_t include_non_mutations, int32_t show_support, const char** text, int64_t* n_bytes) {
+  return format_variants(h, XM_FMT_VCF, contig, contig_name, start, end, f, include_non_mutations, show_support, text, n_bytes);
+}
+int xm_format_mutations(xm_handle* h, int32_t contig, const char* contig_name, int64_t start, int64_t end, const xm_variant_filter* f,
+                        const char** text, int64_t* n_bytes) {
+  return format_variants(h, XM_FMT_MUT, contig, contig_name, start, end, f, 0, 0, text, n_bytes);
 }
 
 // out[0] INT32 IMAD, out[1] FP64 DADD, out[2] FP32 FFMA (full-rate pipe = the dispatch ceiling): sustained warp-instructions per second over the whole chip (the loop
