@@ -281,7 +281,7 @@ struct alignas(8) PMeta { uint32_t stamp, meta; };   // the last 8 bytes of a no
 struct PEnt { uint32_t xy; int32_t next; };
 struct PathState {
   Params prm; ACtx ctx;
-  int an_confident; double an_max_ins, an_max_del;   // the AlignmentAnalysis in force, by value (the search may run on another SM)
+  int an_confident; double an_max_ins, an_max_del;   // the AlignmentAnalysis in force, by value
   int start_a, end_a, start_b, end_b, A, B, W, H;
   int diagonal, step, reverse, may_extend;
   int start_x, start_y, goal_x, goal_y;
@@ -458,7 +458,7 @@ struct PaQueue {
 };
 
 XM_INLINE int pa_signed_dist(const PathState& s, int x, int y) { return x - y - s.diagonal; }
-XM_INLINE PNode pa_node(const PathState& s, int idx) {   // a node as the traceback reads it: past L1, the search may have run on another SM
+XM_INLINE PNode pa_node(const PathState& s, int idx) {   // a node as the traceback reads it: past L1, it visits each node about once
 #if defined(__CUDA_ARCH__)
   const double2 a = __ldcg((const double2*)&s.nodes[idx]);
   const double2 b = __ldcg((const double2*)&s.nodes[idx] + 1);
@@ -629,49 +629,6 @@ XM_FN int pa_search(WS& w, PathState& S, PaOverflow* ovf, int cap_ovf, int& last
   return rc;
 }
 
-// ---- PathAligner search service ----
-// The per-query code is ~480 KB of SASS and the kernel is bound by instruction delivery (ncu: SM instruction-cache hit rate 55 %, the GPC
-// instruction cache at 50-80 % of its request rate, stall_no_instruction 52 of 77 cycles per issued instruction, same run time at 24, 32
-// or 64 warps per SM).  Half of all instructions are the lattice search (pa_search + PaQueue, ~30 KB of code).  So some SMs run NOTHING
-// but that loop: a warp that reaches a search hands it to them through a ring in global memory and sleeps until the answer is back.
-// The search runs on the client's own arena (PathState, lattice nodes, queue entries); only the two sections are copied into the
-// server's shared memory.  Data that crosses SMs is read past L1 (__ldcg / volatile); the lattice nodes may stay L1-cached on the
-// server because a stale line can only hold an older generation, i.e. an absent node, which is what it is until this search writes it.
-struct PaReq { int state; int rc; int last_x, last_y; int status; int pad; unsigned long long steps; PathState* S; PaOverflow* ovf; int cap_ovf; int pad2; };
-typedef PaServiceRef PaService;
-static const int XM_SVC_SEQ_CAP = 1024;   // bytes of shared memory per server warp for the two padded sections
-XM_INLINE int ld_volatile_i(const int* p) { return *(const volatile int*)p; }
-#if defined(__CUDA_ARCH__)
-// client side: post the request, sleep, take the answer.  Returns pa_search's code.
-__device__ __noinline__ int pa_search_remote(WS& w, PathState& S, PaOverflow* ovf, int cap_ovf, int& last_x, int& last_y) {
-  const int lane = (int)(threadIdx.x & 31);
-  PaReq* rq = w.svc.reqs + w.svc_slot;
-  __threadfence();   // every lane's writes to the arena (PathState, sections) are ordered before lane 0 publishes the request
-  __syncwarp();
-  if (lane == 0) {
-    rq->S = &S; rq->ovf = ovf; rq->cap_ovf = cap_ovf; rq->state = 1;
-    __threadfence();   // PathState, sections and the request are in L2 before the ring entry is
-    const unsigned int pos = atomicAdd(w.svc.tail, 1u);
-    *(volatile int*)&w.svc.ring[pos & w.svc.ring_mask] = w.svc_slot + 1;
-  }
-  __syncwarp();
-  while (true) {   // every lane takes part in the wait (uniform control flow), lane 0 looks
-    int done = 0;
-    if (lane == 0) done = ld_volatile_i(&rq->state) == 2 ? 1 : 0;
-    done = __shfl_sync(0xffffffffu, done, 0);
-    if (done) break;
-    __nanosleep(400);
-  }
-  __threadfence();
-  __syncwarp();
-  const int rc = __ldcg(&rq->rc);
-  last_x = __ldcg(&rq->last_x); last_y = __ldcg(&rq->last_y);
-  const int st = __ldcg(&rq->status);
-  w.st_path_steps += __ldcg(&rq->steps);
-  if (st != 0) w.fail(st);
-  return rc;
-}
-#endif
 XM_FN DAln path_align(WS& w, const ACtx& c, const Sec& q, const Sec& r, const Params& p, Analysis& an) {  // PathAligner.align :55-293
   XM_CHECK_MASK(w);
   PhaseClock pc_(&w.st_cyc[3]);
@@ -769,18 +726,10 @@ XM_FN DAln path_align(WS& w, const ACtx& c, const Sec& q, const Sec& r, const Pa
   s.ent = (PEnt*)w.salloc(ent_cap * (long long)sizeof(PEnt));
   if (w.status != 0 || s.ent_cap < 8) { w.fail(Q_NEED_MORE); w.scratch_top = mark; return aln_null(); }
   int last_x = -1, last_y = -1;
-  bool remote = false;
   {
-    int rc;
-#if defined(__CUDA_ARCH__)
-    remote = w.svc.reqs != nullptr && s.A + s.B + 16 <= XM_SVC_SEQ_CAP;
-    if (remote) rc = pa_search_remote(w, s, ovf, cap_ovf, last_x, last_y);
-    else
-#endif
-      rc = pa_search(w, s, ovf, cap_ovf, last_x, last_y);
+    const int rc = pa_search(w, s, ovf, cap_ovf, last_x, last_y);
     if (rc == 1 && w.status == 0) { w.scratch_top = mark; return aln_null(); }
   }
-  (void)remote;
   if (w.status != 0) { w.scratch_top = mark; return aln_null(); }
   // traceback :193-269. Blocks are collected in a temporary array placed after the heap.
   int max_blocks = s.A + s.B + 4;
@@ -1278,7 +1227,6 @@ XM_HD inline DAln cascade_t(WS& w, const ACtx& c, const Sec& q, const Sec& r, co
 // Layout of a warp's staging area (XM_STAGE_BYTES): [0,8) mbarrier; [16, 16 + XM_STAGE_PACKED) the packed window as the bulk copy
 // delivers it (16-byte aligned source, whole 16-byte units); then XM_STAGE_WINDOW bytes: the window, one code per byte.
 static const int XM_STAGE_PACKED = 176, XM_STAGE_WINDOW = 320, XM_STAGE_BYTES = 16 + XM_STAGE_PACKED + XM_STAGE_WINDOW;
-static_assert(XM_STAGE_BYTES <= XM_SVC_SEQ_CAP, "the staging area lives in the per-warp dynamic shared memory slice");
 #if defined(__CUDA_ARCH__)
 __device__ __forceinline__ void stage_init(unsigned char* stage) {   // lane 0, once per warp
   const unsigned int mbar = (unsigned int)__cvta_generic_to_shared(stage);

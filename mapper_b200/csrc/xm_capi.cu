@@ -29,10 +29,9 @@
 using namespace xm;
 
 // ---------------------------------------------------------------- kernels
-// first pass: blocks of 4 warps, 16 per SM (64 warps per SM at 32 registers).  full kernel: ONE block of 32 warps per SM at 64
-// registers - the kernel is bound by instruction delivery (SM instruction-cache hit rate 55 %, the GPC instruction cache at 50-80 % of
-// its request rate), so its run time is the same at 24, 32 or 64 warps per SM (profiles/r2_*), and one block per SM lets a whole SM
-// take one role: a configurable number of SMs run nothing but the PathAligner lattice search for the others (xm_align.h: PaReq).
+// first pass: blocks of 4 warps, 16 per SM (64 warps per SM at 32 registers).  full kernel: blocks of 32 warps, XM_FULL_MIN_BLOCKS
+// per SM - the kernel is bound by instruction delivery (SM instruction-cache hit rate 55 %, the GPC instruction cache at 50-80 % of
+// its request rate), so its run time is the same at 24, 32 or 64 warps per SM (profiles/r2_*).
 #ifndef XM_BLOCK
 #define XM_BLOCK 128
 #endif
@@ -45,7 +44,6 @@ using namespace xm;
 #ifndef XM_FULL_MIN_BLOCKS
 #define XM_FULL_MIN_BLOCKS 2
 #endif
-#define XM_SVC_BYTES_PER_WARP (((sizeof(PathState) + 15) & ~(size_t)15) + XM_SVC_SEQ_CAP)   // dynamic shared memory per warp of the full kernel: a server's PathState + sections, or a client's TMA staging area (XM_STAGE_BYTES, smaller)
 struct BatchD {
   int n_queries;
   const uint16_t* packed; const int64_t* seq_word_off; const int32_t* seq_len; const int64_t* first_seq;  // first_seq: n_queries+1
@@ -64,11 +62,8 @@ struct LaunchD {
   char* arenas; long long arena_bytes;
   char* big_arenas; long long big_arena_bytes; int n_big; int* big_busy;  // pool of next-tier-sized arenas: a query that outgrows its warp's arena is re-run at once in a free one
   int last_tier;
-  int exp_groups;                         // experiment: distinct query streams per block (XM_EXP_GROUPS, default 1)
-  int exp_dup;                            // experiment (XM_EXP_DUP=n): every warp of a block aligns the same n queries, results discarded by overwrite
-  int dyn_stride;                         // bytes of dynamic shared memory per warp (XM_SVC_BYTES_PER_WARP with the search service on, else XM_STAGE_BYTES)
+  int dyn_stride;                         // bytes of dynamic shared memory per warp: the TMA staging area (XM_STAGE_BYTES) with use_tma, else 0
   int use_tma;                            // full kernel: reference windows are fetched with cp.async.bulk into the warp's staging area in shared memory
-  PaServiceRef svc; int n_server_sms;     // PathAligner search service: the blocks that land on the first n_server_sms SMs to ask run nothing but pa_search for the others (xm_align.h)
   long long* q_cycles;                    // optional per-query cost probe (XM_QCYCLES=1): clock64 ticks of the tier that finished it
 };
 
@@ -78,34 +73,7 @@ template <bool EASY>
 __global__ void __launch_bounds__(EASY ? XM_BLOCK : XM_FULL_BLOCK, EASY ? XM_MIN_BLOCKS : XM_FULL_MIN_BLOCKS) xm_align_kernel(LaunchD L) {
   const int lane = threadIdx.x & 31;
   const int warp_in_block = (int)(threadIdx.x >> 5), warps_per_block = (int)(blockDim.x >> 5);
-  const int n_srv = EASY ? 0 : L.n_server_sms;
-  // role of this block: a search server if its SM is one of the first n_srv to be claimed, else a client.  Both blocks of an SM get the
-  // same role, so a server SM fetches nothing but the search loop.
-  __shared__ int s_role;
-  if (!EASY && n_srv > 0) {
-    if (threadIdx.x == 0) {
-      unsigned int smid; asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-      int* cell = &L.svc.sm_role[smid & 1023];
-      int r = ld_volatile_i(cell);
-      if (r == 0) {
-        const int want = (atomicAdd(L.svc.n_claimed, 1) < n_srv) ? 2 : 1;
-        const int prev = atomicCAS(cell, 0, want);
-        if (prev == 0) r = want; else { r = prev; if (want == 2) atomicSub(L.svc.n_claimed, 1); }
-      }
-      s_role = r;
-      if (r == 1) atomicAdd(L.svc.active_clients, (int)(blockDim.x >> 5));
-      __threadfence();
-      atomicAdd(L.svc.started_blocks, 1);
-    }
-    __syncthreads();
-  }
-  const bool is_server = !EASY && n_srv > 0 && s_role == 2;
-  long long warp = (long long)blockIdx.x * warps_per_block + warp_in_block;   // arena slot (with the service on: handed out to client warps as they start)
-  if (!EASY && n_srv > 0 && !is_server) {
-    int slot = 0;
-    if (lane == 0) slot = atomicAdd(L.svc.client_slots, 1);
-    warp = (long long)__shfl_sync(0xffffffffu, slot, 0);
-  }
+  const long long warp = (long long)blockIdx.x * warps_per_block + warp_in_block;   // arena slot
   char* arena = L.arenas + warp * L.arena_bytes;
   __shared__ double s_pen[256];
   __shared__ uint8_t s_cls[1024];
@@ -117,81 +85,20 @@ __global__ void __launch_bounds__(EASY ? XM_BLOCK : XM_FULL_BLOCK, EASY ? XM_MIN
   __syncthreads();
   L.prm.pen_tab = s_pen; L.prm.cls_tab = s_cls;
   if (!EASY) {
-    if (is_server) {
-      // ---- search server: this SM runs only the lattice search, for whichever client asks next ----
-      extern __shared__ __align__(16) unsigned char xm_dyn_smem[];   // per warp: a PathState + the two padded sections (XM_SVC_BYTES_PER_WARP)
-      PathState& S = *(PathState*)(xm_dyn_smem + (size_t)warp_in_block * L.dyn_stride);
-      uint8_t* seq = xm_dyn_smem + (size_t)warp_in_block * L.dyn_stride + ((sizeof(PathState) + 15) & ~(size_t)15);
-      while (true) {
-        unsigned int pos = 0; int slot1 = 0;
-        if (lane == 0) pos = atomicAdd(L.svc.head, 1u);
-        pos = __shfl_sync(0xffffffffu, pos, 0);
-        int* cell = &L.svc.ring[pos & L.svc.ring_mask];
-        while (true) {   // uniform control flow: every lane takes part in the polling loop, lane 0 looks (a lane-0-only loop would leave the warp split)
-          int s = 0;
-          if (lane == 0) {
-            if (ld_volatile_i(cell) != 0) s = atomicExch(cell, 0);
-            if (s == 0 && ld_volatile_i(L.svc.started_blocks) >= (int)gridDim.x && ld_volatile_i(L.svc.active_clients) <= 0) s = -1;
-          }
-          s = __shfl_sync(0xffffffffu, s, 0);
-          if (s != 0) { slot1 = s; break; }
-          __nanosleep(200);
-        }
-        __threadfence();
-        __syncwarp();
-        if (slot1 < 0) break;
-        PaReq* rq = L.svc.reqs + (slot1 - 1);
-        PathState* gS = (PathState*)__ldcg((const unsigned long long*)&rq->S);
-        PaOverflow* ovf = (PaOverflow*)__ldcg((const unsigned long long*)&rq->ovf);
-        const int cap_ovf = __ldcg(&rq->cap_ovf);
-        for (int k = lane; k < (int)(sizeof(PathState) / 4); k += 32) ((uint32_t*)&S)[k] = __ldcg((const uint32_t*)gS + k);
-        __syncwarp();
-        const uint8_t* gqa = S.qa - 2; const uint8_t* grb = S.rb - 2;   // the client's padded sections
-        const int na = S.A + 4, nb = S.B + 4;
-        for (int k = lane; k < na; k += 32) seq[k] = __ldcg(gqa + k);
-        for (int k = lane; k < nb; k += 32) seq[na + k] = __ldcg(grb + k);
-        __syncwarp();
-        if (lane == 0) { S.qa = seq + 2; S.rb = seq + na + 2; S.prm.pen_tab = s_pen; S.prm.cls_tab = s_cls; w.status = 0; w.st_path_steps = 0; }
-        __syncwarp();
-        int lx = -1, ly = -1;
-        const int rc = pa_search(w, S, ovf, cap_ovf, lx, ly);
-        __threadfence();   // the lattice nodes this search wrote are in L2 before the answer is
-        __syncwarp();
-        if (lane == 0) {
-          rq->rc = rc; rq->last_x = lx; rq->last_y = ly; rq->status = w.status; rq->steps = w.st_path_steps;
-          __threadfence();
-          *(volatile int*)&rq->state = 2;
-        }
-        __syncwarp();
-      }
-      return;
-    }
-    w.svc = L.svc; w.svc_slot = (int)warp;
-    if (n_srv == 0) w.svc.reqs = nullptr;
-    {
-      extern __shared__ __align__(16) unsigned char xm_dyn_smem[];
-      unsigned char* stage = L.use_tma ? xm_dyn_smem + (size_t)warp_in_block * L.dyn_stride : nullptr;
+    extern __shared__ __align__(16) unsigned char xm_dyn_smem[];
+    unsigned char* stage = L.use_tma ? xm_dyn_smem + (size_t)warp_in_block * L.dyn_stride : nullptr;
 #if defined(__CUDA_ARCH__)
-      if (lane == 0) { w.stage = stage; w.stage_phase = 0; if (stage) stage_init(stage); }
+    if (lane == 0) { w.stage = stage; w.stage_phase = 0; if (stage) stage_init(stage); }
 #endif
-      __syncwarp();
-    }
+    __syncwarp();
   }
   unsigned long long st[14] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
   if (L.n_ids_ptr) L.n_ids = *L.n_ids_ptr;
-  int dup_i = 0;
   while (true) {
     int t = 0;
-    if (L.exp_dup > 0) {
-      if (dup_i >= L.exp_dup) break;
-      // exp_groups distinct query streams per block: warps with the same (warp % groups) align the same queries
-      t = (int)((((long long)blockIdx.x * L.exp_groups + (warp_in_block % L.exp_groups)) * L.exp_dup + dup_i) % L.n_ids);
-      dup_i++;
-    } else {
-      if (lane == 0) t = atomicAdd(L.ticket, 1);
-      t = __shfl_sync(0xffffffffu, t, 0);
-      if (t >= L.n_ids) break;
-    }
+    if (lane == 0) t = atomicAdd(L.ticket, 1);
+    t = __shfl_sync(0xffffffffu, t, 0);
+    if (t >= L.n_ids) break;
     __syncwarp();   // every query starts with the warp converged: the per-query code runs on warp-shared state with all 32 lanes
 #if defined(XM_DBG_UNIFORM)
     const bool split_at_start = __activemask() != 0xffffffffu;
@@ -208,7 +115,7 @@ __global__ void __launch_bounds__(EASY ? XM_BLOCK : XM_FULL_BLOCK, EASY ? XM_MIN
     q.per_penalty = q.n_seqs > 1 ? L.batch.per_penalty[qi] : 1.0;
     OutQuery rec; rec.status = 0; rec.n_comp = 1; rec.n_choice[0] = 0; rec.n_choice[1] = 0; rec.choice_first[0] = 0; rec.choice_first[1] = 0;
     w.hard_hint = 1 << 20;  // anything but Q_HARD (workspace exhausted in the first pass): assume long
-    if (EASY) { w.svc.reqs = nullptr; w.stage = nullptr; }
+    if (EASY) w.stage = nullptr;
     if (!ws_init(w, arena, L.arena_bytes, &L.ref, &L.ix, &L.dup, L.prm, q, !EASY)) w.status = Q_NEED_MORE;
     else align_query<EASY>(w, L.out, rec);
     __syncwarp();
@@ -266,7 +173,6 @@ __global__ void __launch_bounds__(EASY ? XM_BLOCK : XM_FULL_BLOCK, EASY ? XM_MIN
     }
   }
   if (lane == 0) for (int i = 0; i < 14; i++) if (st[i]) atomicAdd(&L.out.stats[i], st[i]);
-  if (!EASY && n_srv > 0 && lane == 0) { __threadfence(); atomicSub(L.svc.active_clients, 1); }
 }
 
 
@@ -827,7 +733,6 @@ static NcclApi& nccl_api() {
 struct xm_handle {
   HostModel m;
   int device = 0, sm_count = 148, blocks_per_sm = 4;
-  int full_warps = XM_FULL_BLOCK / 32, full_blocks_per_sm = XM_FULL_MIN_BLOCKS;  // full kernel: warps per block, blocks per SM
   std::string err;
   cudaStream_t stream = nullptr;
   cudaEvent_t ev2 = nullptr, ev3 = nullptr, ev4 = nullptr, ev5 = nullptr;
@@ -857,11 +762,8 @@ struct xm_handle {
   DevBuf d_csr_cnt, d_csr_base, d_csr_tmp, d_keys_a, d_keys_b, d_sort_tmp, d_big, d_big_busy;
   DevBuf d_sam_len, d_sam_text, d_sam_names, d_sam_name_off, d_sam_cnames, d_sam_cname_off;
   std::shared_ptr<PinnedPool> pinned = std::make_shared<PinnedPool>();
-  bool probe_cycles = false, sort_hard = true;
-  bool use_tma = true;    // XM_TMA=0: reference windows are unpacked from global memory (the round-1 path)
-  int path_servers = 0;   // XM_PATH_SERVERS: SMs of the full kernel's launch that run only the PathAligner search service (0 = every warp searches for itself)
-  DevBuf d_svc;
-  int big_pool = 64;  // XM_BIG_POOL: next-tier arenas available inside a full-kernel launch (0 = off)
+  bool probe_cycles = false;
+  bool use_tma = true;    // false when the full kernel cannot get its dynamic shared memory: reference windows are then unpacked from global memory
   long long cap_choices = 0, cap_sas = 0, cap_blocks = 0;
   size_t ws_budget = (size_t)128 << 30;  // clamped to 60 % of the free device memory in xm_create
   // counts
@@ -1316,19 +1218,12 @@ int xm_create(const xm_params* p, int device, xm_handle** out) {
   cudaGetDeviceProperties(&prop, device);
   h->sm_count = prop.multiProcessorCount;
   { int nb = 0; if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, xm_align_kernel<true>, XM_BLOCK, 0) == cudaSuccess && nb > 0) h->blocks_per_sm = nb; }
-  if (const char* e = getenv("XM_BLOCKS_PER_SM")) { int v = atoi(e); if (v > 0) h->blocks_per_sm = v; }
-  if (const char* e = getenv("XM_SORT_HARD")) h->sort_hard = atoi(e) != 0;
-  if (const char* e = getenv("XM_TMA")) h->use_tma = atoi(e) != 0;
-  if (const char* e = getenv("XM_PATH_SERVERS")) { int v = atoi(e); if (v >= 0 && v < h->sm_count) h->path_servers = v; }
-  if (const char* e = getenv("XM_BIG_POOL")) { int v = atoi(e); if (v >= 0 && v <= 1024) h->big_pool = v; }
-  if (const char* e = getenv("XM_FULL_BLOCKS_PER_SM")) { int v = atoi(e); if (v >= 1 && v <= 8) h->full_blocks_per_sm = v; }
-  if (const char* e = getenv("XM_FULL_WARPS")) { int v = atoi(e); if (v >= 1 && v <= XM_FULL_BLOCK / 32) h->full_warps = v; }
   if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess ||
       cudaEventCreate(&h->ev2) != cudaSuccess || cudaEventCreate(&h->ev3) != cudaSuccess || cudaEventCreate(&h->ev4) != cudaSuccess || cudaEventCreate(&h->ev5) != cudaSuccess) {
     fprintf(stderr, "xmapper_b200: stream/event creation failed: %s\n", cudaGetErrorString(cudaGetLastError()));
     xm_destroy(h); return XM_ERR_CUDA;
   }
-  if (cudaFuncSetAttribute(xm_align_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((XM_FULL_BLOCK / 32) * XM_SVC_BYTES_PER_WARP)) != cudaSuccess) { cudaGetLastError(); h->path_servers = 0; h->use_tma = false; }
+  if (cudaFuncSetAttribute(xm_align_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (XM_FULL_BLOCK / 32) * XM_STAGE_BYTES) != cudaSuccess) { cudaGetLastError(); h->use_tma = false; }
   for (auto& sl : h->slots) {
     if (cudaStreamCreateWithFlags(&sl.copy, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreateWithFlags(&sl.h2d_done, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&sl.kernels_done, cudaEventDisableTiming) != cudaSuccess || cudaEventCreate(&sl.ev0) != cudaSuccess || cudaEventCreate(&sl.ev1) != cudaSuccess) {
@@ -1372,7 +1267,7 @@ void xm_destroy(xm_handle* h) {
     for (cudaEvent_t e : {sl.h2d_done, sl.kernels_done, sl.ev0, sl.ev1}) if (e) cudaEventDestroy(e);
   }
   DevBuf* bufs[] = {&h->d_words, &h->d_word_off, &h->d_len, &h->d_gstart, &h->d_tables, &h->d_dup_off, &h->d_dup_starts, &h->d_chunk, &h->d_q, &h->d_choices, &h->d_sas, &h->d_blocks,
-                    &h->d_misc, &h->d_ids_a, &h->d_ids_b, &h->d_ids_full, &h->d_ws, &h->d_qcycles, &h->d_csr_cnt, &h->d_csr_base, &h->d_csr_tmp, &h->d_keys_a, &h->d_keys_b, &h->d_sort_tmp, &h->d_big, &h->d_big_busy, &h->d_sam_len, &h->d_sam_text, &h->d_sam_names, &h->d_sam_name_off, &h->d_sam_cnames, &h->d_sam_cname_off, &h->d_svc, &h->d_planes, &h->d_contig_off, &h->d_var, &h->d_var_n, &h->d_order, &h->d_var_sizes,
+                    &h->d_misc, &h->d_ids_a, &h->d_ids_b, &h->d_ids_full, &h->d_ws, &h->d_qcycles, &h->d_csr_cnt, &h->d_csr_base, &h->d_csr_tmp, &h->d_keys_a, &h->d_keys_b, &h->d_sort_tmp, &h->d_big, &h->d_big_busy, &h->d_sam_len, &h->d_sam_text, &h->d_sam_names, &h->d_sam_name_off, &h->d_sam_cnames, &h->d_sam_cname_off, &h->d_planes, &h->d_contig_off, &h->d_var, &h->d_var_n, &h->d_order, &h->d_var_sizes,
                     &h->var_scratch.keys_a, &h->var_scratch.keys_b, &h->var_scratch.idx_a, &h->var_scratch.idx_b, &h->var_scratch.gathered, &h->var_scratch.out_keys, &h->var_scratch.n_out, &h->var_scratch.tmp,
                     &h->d_ex_words, &h->d_ex_word_off, &h->d_ex_len, &h->d_ex_gids, &h->d_ex_slot, &h->d_ex_bad,
                     &h->d_fmt_dec, &h->d_fmt_state, &h->d_fmt_len, &h->d_fmt_range, &h->d_fmt_name, &h->d_fmt_text, &h->d_fmt_tmp, &h->d_fmt_ids};
@@ -2062,8 +1957,8 @@ static int align_batch_impl(xm_handle* h, SlotLease& lease, bool wait_h2d, int32
       if (blocks < 1) blocks = 1;
       if ((long long)blocks * warps_per_block * arena > (long long)h->ws_budget && blocks > 1) blocks = (int)(h->ws_budget / (size_t)(arena * warps_per_block));
     } else {
-      cpb = h->full_warps;
-      const int slots = h->sm_count * h->full_blocks_per_sm;   // resident blocks of the full kernel
+      cpb = XM_FULL_BLOCK / 32;
+      const int slots = h->sm_count * XM_FULL_MIN_BLOCKS;   // resident blocks of the full kernel
       long long resident = (long long)slots * cpb;
       arena = tier_arena_bytes(tier, max_seq_len, 2, (long long)h->ws_budget, resident);
       long long clients = resident, max_warps = (long long)(h->ws_budget / (size_t)arena);
@@ -2076,24 +1971,7 @@ static int align_batch_impl(xm_handle* h, SlotLease& lease, bool wait_h2d, int32
       if (blocks > slots) blocks = slots;
     }
     if (blocks < 1) { h->err = "workspace budget too small for one block"; return XM_ERR_CUDA; }
-    // search service: the first n_srv blocks of a full-size launch run only pa_search (they own no arena); small launches keep every block a client
-    int n_srv = 0;
-    L.svc.reqs = nullptr; L.n_server_sms = 0; L.use_tma = (tier >= 0 && h->use_tma) ? 1 : 0;
-    if (tier >= 0 && h->path_servers > 0 && blocks == h->sm_count * h->full_blocks_per_sm && cpb == h->full_warps && h->sm_count > 2 * h->path_servers) {
-      n_srv = h->path_servers;
-      const int client_warps = blocks * cpb;   // upper bound: the ring and the request slots are sized for every warp of the launch
-      unsigned int ring = 1; while ((int)ring < client_warps) ring <<= 1;
-      const size_t req_bytes = ((size_t)client_warps * sizeof(PaReq) + 255) & ~(size_t)255;
-      const size_t total = req_bytes + (size_t)ring * 4 + 256 + 1024 * 4;
-      if (!h->d_svc.ensure(total)) { h->err = "out of device memory (search service)"; return XM_ERR_CUDA; }
-      CK(cudaMemsetAsync(h->d_svc.p, 0, total, st));
-      char* base = (char*)h->d_svc.p;
-      L.svc.reqs = (PaReq*)base; L.svc.ring = (int*)(base + req_bytes); L.svc.ring_mask = ring - 1;
-      unsigned int* ctr = (unsigned int*)(base + req_bytes + (size_t)ring * 4);
-      L.svc.head = ctr; L.svc.tail = ctr + 1; L.svc.active_clients = (int*)(ctr + 2); L.svc.n_claimed = (int*)(ctr + 3);
-      L.svc.client_slots = (int*)(ctr + 4); L.svc.started_blocks = (int*)(ctr + 5); L.svc.sm_role = (int*)(ctr + 64);
-      L.n_server_sms = n_srv;
-    }
+    L.use_tma = (tier >= 0 && h->use_tma) ? 1 : 0;
     if (!h->d_ws.ensure((size_t)blocks * cpb * (size_t)arena)) { h->err = "out of device memory (workspace)"; return XM_ERR_CUDA; }
     CK(cudaMemsetAsync(ticket, 0, 4, st));
     CK(cudaMemsetAsync(n_need_more, 0, 4, st));
@@ -2103,10 +1981,10 @@ static int align_batch_impl(xm_handle* h, SlotLease& lease, bool wait_h2d, int32
     L.ids = ids; L.n_ids = n_ids; L.n_ids_ptr = n_ids_dev; L.need_more = need_more_out; L.arenas = (char*)h->d_ws.p; L.arena_bytes = arena; L.last_tier = (tier == XM_NUM_TIERS - 1);
     L.need_more_key = nullptr;
     L.big_arenas = nullptr; L.big_arena_bytes = 0; L.n_big = 0; L.big_busy = nullptr;
-    if (tier >= 0 && tier + 1 < XM_NUM_TIERS && h->big_pool > 0) {
+    if (tier >= 0 && tier + 1 < XM_NUM_TIERS) {
       // a small pool of next-tier arenas inside this launch: the rare queries that outgrow their arena do not wait for a launch of their own
-      const long long big = tier_arena_bytes(tier + 1, max_seq_len, 2, (long long)h->ws_budget, (long long)h->sm_count * h->full_blocks_per_sm * h->full_warps);
-      int n_big = h->big_pool;
+      const long long big = tier_arena_bytes(tier + 1, max_seq_len, 2, (long long)h->ws_budget, (long long)h->sm_count * XM_FULL_MIN_BLOCKS * (XM_FULL_BLOCK / 32));
+      int n_big = 64;
       while (n_big > 0 && (long long)n_big * big > (long long)h->ws_budget / 4) n_big /= 2;
       if (n_big > 0 && big > arena && h->d_big.ensure((size_t)n_big * (size_t)big) && h->d_big_busy.ensure((size_t)n_big * 4)) {
         CK(cudaMemsetAsync(h->d_big_busy.p, 0, (size_t)n_big * 4, st));
@@ -2114,16 +1992,13 @@ static int align_batch_impl(xm_handle* h, SlotLease& lease, bool wait_h2d, int32
         L.big_arenas = (char*)h->d_big.p; L.big_arena_bytes = big; L.n_big = n_big; L.big_busy = (int*)h->d_big_busy.p;
       }
     }
-    if (tier < 0 && h->sort_hard) {
+    if (tier < 0) {
       if (!h->d_keys_a.ensure((size_t)n_ids * 4) || !h->d_keys_b.ensure((size_t)n_ids * 4)) { h->err = "out of device memory"; return XM_ERR_CUDA; }
       CK(cudaMemsetAsync(h->d_keys_a.p, 0x80, (size_t)n_ids * 4, st));   // slots the kernel leaves unused sort last (key 0x80808080 < 0)
       L.need_more_key = (int32_t*)h->d_keys_a.p;
     }
-    L.exp_dup = 0;
-    L.exp_groups = 1;
-    if (tier >= 0) { if (const char* e = getenv("XM_EXP_DUP")) L.exp_dup = atoi(e); if (const char* e = getenv("XM_EXP_GROUPS")) L.exp_groups = atoi(e) > 0 ? atoi(e) : 1; }
     CK(cudaEventRecord(e0, st));
-    L.dyn_stride = n_srv > 0 ? (int)XM_SVC_BYTES_PER_WARP : (L.use_tma ? XM_STAGE_BYTES : 0);
+    L.dyn_stride = L.use_tma ? XM_STAGE_BYTES : 0;
     if (tier < 0) xm_align_kernel<true><<<blocks, block, 0, st>>>(L);
     else xm_align_kernel<false><<<blocks, 32 * cpb, (size_t)cpb * (size_t)L.dyn_stride, st>>>(L);
     CK(cudaEventRecord(e1, st));
@@ -2155,7 +2030,7 @@ static int align_batch_impl(xm_handle* h, SlotLease& lease, bool wait_h2d, int32
   R->r.stats[XM_STAT_EASY_QUERIES] += nq;
   CK(cudaMemcpyAsync(d_easy_stats, d_stats, 7 * 8, cudaMemcpyDeviceToDevice, st));
   const int32_t* hard_ids = ids_a;
-  if (h->sort_hard && nq > 1) {
+  if (nq > 1) {
     // longest first: the persistent full kernel ends when its slowest query does, so the queries the first pass scored worst (most
     // likely gapped) start first and the cheap ones fill the tail; co-resident warps also run the same kind of query, which the
     // instruction caches reward.  All nq slots are sorted (the unused ones carry the smallest key), so no count is needed here.

@@ -204,9 +204,6 @@ struct MatePath {
 };
 
 struct DAlnStore;  // xm_align.h
-struct PaReq; struct PaOverflow; struct PathState;
-struct PaServiceRef { PaReq* reqs; int* ring; unsigned int ring_mask; unsigned int* head; unsigned int* tail; int* active_clients;
-                      int* sm_role; int* n_claimed; int* client_slots; int* started_blocks; };
 
 #if defined(__CUDA_ARCH__)
 #define XM_CLK() ((unsigned long long)clock64())
@@ -245,7 +242,6 @@ struct WS {
   // delivers it, and the window unpacked to one code per byte (what every stage of the cascade reads).  nullptr: windows are unpacked
   // from global memory into the arena.
   unsigned char* stage; unsigned int stage_phase;
-  PaServiceRef svc; int svc_slot;   // PathAligner search service (xm_align.h): reqs == nullptr = searches run on this warp
   uint32_t* cell_hdr; uint32_t* cellmap; long long cell_words;  // PathAligner lattice map region of the arena (xm_align.h: PathState::cell)
   uint8_t* qbytes[2][2];  // [mate][reverse-complemented]: one code per byte
   int hard_hint;  // first pass: cost estimate of a query handed to the full kernel (its ungapped penalty), used to start long queries first
