@@ -308,17 +308,46 @@ XM_INLINE uint32_t pa_pack_xy(int x, int y) { return ((uint32_t)(uint16_t)(int16
 // priority (binary search to find, lane-parallel shift to insert, the front is the minimum): long reads with large
 // budgets keep hundreds of distinct priorities alive.
 struct PaOverflow { double key; int head, tail; };
+// The warp-uniform state of one search: its constants and the queue's scalars.  On the device it lives in shared memory, one frame
+// per warp (pa_frame), and is read where it is used: at 32 registers the search cannot hold all of it, and a value that ptxas
+// spills goes to local memory, where every lane keeps (and writes through to L2/HBM) its own copy of the same bytes, while a
+// shared-memory read is one broadcast load.  Writes follow the warp-uniform rule (§3 of DESIGN.md): all lanes store the same
+// value while the warp is converged.
+struct PaFrame {
+  const double* pen_tab; const uint8_t* cls_tab; PNode* nodes; const uint8_t* qa; const uint8_t* rb;
+  double ins_start, ins_ext, del_start, del_ext, unaligned, max_ins, max_del, budget, min_indel;
+  unsigned long long steps;
+  // PaQueue: popped entries are chained for reuse once the fresh ones run out; cur_* is the bucket being drained
+  // (cur_key == activePenalty); the live spill buckets are ovf[ovf_lo, ovf_hi), ascending keys
+  PEnt* ent; PaOverflow* ovf;
+  double cur_key;
+  int n_ent, cap, free_head, cur_head, cur_tail, ovf_lo, ovf_hi, cap_ovf;
+  int A, B, H, step, goal_x, goal_y, diagonal;
+  uint32_t gen, clock;   // clock: the write counter (PNode::stamp)
+  int16_t tx, ty, x, y;  // the node being expanded and the neighbour being evaluated (a lattice side is at most 32000)
+  uint8_t may_extend, confident;
+};
+static_assert(sizeof(PaFrame) == 224, "32 frames keep the full kernel's static shared memory within 48 KB");
+// A frame value read where it is used.  On the device this is a volatile shared-memory load: the compiler neither merges it with an
+// earlier load nor keeps the value in a register across the loop body, where it would be spilled.
+template <class T> XM_INLINE T pa_ld(const T& v) {
+#if defined(__CUDA_ARCH__)
+  return *(const volatile T*)&v;
+#else
+  return v;
+#endif
+}
+#if defined(__CUDA_ARCH__)
+__shared__ PaFrame pa_frame[32];   // one per warp of the block; only the full kernel's image contains the search
+#endif
 struct PaQueue {
-  PEnt* ent; int n_ent, cap, free_head;   // popped entries are chained for reuse once the fresh ones run out
-  double cur_key; int cur_head, cur_tail;  // the bucket being drained; cur_key == activePenalty
-  PaOverflow* ovf; int ovf_lo, ovf_hi, cap_ovf;  // live spill buckets are ovf[ovf_lo, ovf_hi), ascending keys
 #if defined(__CUDA_ARCH__)
   double bkey; int bhead, btail;           // this lane's bucket (bhead < 0: free)
 #else
   double bkey[32]; int bhead[32], btail[32];
 #endif
-  XM_INLINE void init(PEnt* e, int capacity, PaOverflow* o, int cap_o) {
-    ent = e; n_ent = 0; cap = capacity; free_head = -1; cur_key = 0; cur_head = -1; cur_tail = -1; ovf = o; ovf_lo = 0; ovf_hi = 0; cap_ovf = cap_o;
+  XM_INLINE void init(PaFrame& f, PEnt* e, int capacity, PaOverflow* o, int cap_o) {
+    f.ent = e; f.n_ent = 0; f.cap = capacity; f.free_head = -1; f.cur_key = 0; f.cur_head = -1; f.cur_tail = -1; f.ovf = o; f.ovf_lo = 0; f.ovf_hi = 0; f.cap_ovf = cap_o;
 #if defined(__CUDA_ARCH__)
     bkey = 0; bhead = -1; btail = -1;
 #else
@@ -326,15 +355,17 @@ struct PaQueue {
 #endif
   }
   // 0 ok, 1 out of entry space, 2 out of overflow space.  pri >= cur_key always (estimates are clamped to activePenalty).
-  XM_INLINE int push(double pri, int x, int y) {
+  XM_INLINE int push(PaFrame& f, double pri, int x, int y) {
+    PEnt* const ent = f.ent;
     int id;
-    if (n_ent < cap) id = n_ent++;
-    else { if (free_head < 0) return 1; id = free_head; free_head = ent[id].next; }
+    if (f.n_ent < f.cap) { id = f.n_ent; f.n_ent = id + 1; }
+    else { id = f.free_head; if (id < 0) return 1; f.free_head = ent[id].next; }
     PEnt e; e.xy = pa_pack_xy(x, y); e.next = -1;
     ent[id] = e;
-    if (pri == cur_key) {
-      if (cur_tail >= 0) ent[cur_tail].next = id; else cur_head = id;
-      cur_tail = id;
+    if (pri == f.cur_key) {
+      const int t = f.cur_tail;
+      if (t >= 0) ent[t].next = id; else f.cur_head = id;
+      f.cur_tail = id;
       return 0;
     }
 #if defined(__CUDA_ARCH__)
@@ -352,7 +383,8 @@ struct PaQueue {
 #endif
     // spill array: first position with key >= pri.  On the device the lanes probe 32 pivots per round (a 32-ary search: two
     // dependent loads for up to 1024 buckets, where a binary search chases ten)
-    int lo = ovf_lo, hi = ovf_hi;
+    PaOverflow* const ovf = f.ovf;
+    int lo = f.ovf_lo, hi = f.ovf_hi;
 #if defined(__CUDA_ARCH__)
     XM_NOUNROLL
     while (hi - lo > 0) {
@@ -370,34 +402,36 @@ struct PaQueue {
     XM_NOUNROLL
     while (lo < hi) { const int mid = (lo + hi) >> 1; if (ovf[mid].key < pri) lo = mid + 1; else hi = mid; }
 #endif
-    if (lo < ovf_hi && ovf[lo].key == pri) { ent[ovf[lo].tail].next = id; ovf[lo].tail = id; return 0; }
+    if (lo < f.ovf_hi && ovf[lo].key == pri) { ent[ovf[lo].tail].next = id; ovf[lo].tail = id; return 0; }
 #if defined(__CUDA_ARCH__)
     const unsigned fre = __ballot_sync(0xffffffffu, bhead < 0);
     if (fre != 0) { const int b = __ffs(fre) - 1; if (lane == b) { bkey = pri; bhead = id; btail = id; } return 0; }
 #else
     for (int b = 0; b < 32; b++) if (bhead[b] < 0) { bkey[b] = pri; bhead[b] = id; btail[b] = id; return 0; }
 #endif
-    if (ovf_hi >= cap_ovf) {
-      if (ovf_lo == 0) return 2;
-      const int n = ovf_hi - ovf_lo;  // slide the live range back to the start of the array
+    if (f.ovf_hi >= f.cap_ovf) {
+      const int olo = f.ovf_lo;
+      if (olo == 0) return 2;
+      const int n = f.ovf_hi - olo;  // slide the live range back to the start of the array
 #if defined(__CUDA_ARCH__)
       XM_NOUNROLL
       for (int base = 0; base < n; base += 32) {
         const int i = base + lane;
-        PaOverflow t; if (i < n) t = ovf[ovf_lo + i];
+        PaOverflow t; if (i < n) t = ovf[olo + i];
         __syncwarp();
         if (i < n) ovf[i] = t;
         __syncwarp();
       }
 #else
-      for (int i = 0; i < n; i++) ovf[i] = ovf[ovf_lo + i];
+      for (int i = 0; i < n; i++) ovf[i] = ovf[olo + i];
 #endif
-      lo -= ovf_lo; ovf_lo = 0; ovf_hi = n;
+      lo -= olo; f.ovf_lo = 0; f.ovf_hi = n;
     }
     {  // insert at lo: shift [lo, ovf_hi) up by one, highest elements first
+      const int ohi = f.ovf_hi;
 #if defined(__CUDA_ARCH__)
       XM_NOUNROLL
-      for (int top = ovf_hi; top > lo; top -= 32) {
+      for (int top = ohi; top > lo; top -= 32) {
         const int i = top - 1 - lane;
         PaOverflow t; if (i >= lo) t = ovf[i];
         __syncwarp();
@@ -405,17 +439,19 @@ struct PaQueue {
         __syncwarp();
       }
 #else
-      for (int i = ovf_hi - 1; i >= lo; i--) ovf[i + 1] = ovf[i];
+      for (int i = ohi - 1; i >= lo; i--) ovf[i + 1] = ovf[i];
 #endif
       PaOverflow t; t.key = pri; t.head = id; t.tail = id;
       ovf[lo] = t;
-      ovf_hi++;
+      f.ovf_hi = ohi + 1;
     }
     return 0;
   }
-  // false: queue empty.  Otherwise (x, y) of the next node in the reference's order; cur_key is its priority.
-  XM_INLINE bool pop(int& x, int& y) {
-    if (cur_head < 0) {  // next bucket = the smallest remaining priority (all are > cur_key)
+  // false: queue empty.  Otherwise (x, y) of the next node in the reference's order; f.cur_key is its priority.
+  XM_INLINE bool pop(PaFrame& f, int& x, int& y) {
+    PEnt* const ent = f.ent;
+    int head = f.cur_head;
+    if (head < 0) {  // next bucket = the smallest remaining priority (all are > cur_key)
       bool have = false; double best = 0; int where = -1;  // where: 0..31 lane bucket, 32+i overflow entry i
 #if defined(__CUDA_ARCH__)
       const int lane = (int)(threadIdx.x & 31);
@@ -435,23 +471,27 @@ struct PaQueue {
 #else
       for (int b = 0; b < 32; b++) if (bhead[b] >= 0 && (!have || bkey[b] < best)) { have = true; best = bkey[b]; where = b; }
 #endif
-      if (ovf_lo < ovf_hi && (!have || ovf[ovf_lo].key < best)) { have = true; best = ovf[ovf_lo].key; where = 32; }
+      const int olo = f.ovf_lo;
+      if (olo < f.ovf_hi && (!have || f.ovf[olo].key < best)) { have = true; best = f.ovf[olo].key; where = 32; }
       if (!have) return false;
-      cur_key = best;
-      if (where >= 32) { cur_head = ovf[ovf_lo].head; cur_tail = ovf[ovf_lo].tail; ovf_lo++; if (ovf_lo == ovf_hi) { ovf_lo = 0; ovf_hi = 0; } }
-      else {
+      f.cur_key = best;
+      if (where >= 32) {
+        const PaOverflow o = f.ovf[olo];
+        head = o.head; f.cur_tail = o.tail;
+        if (olo + 1 == f.ovf_hi) { f.ovf_lo = 0; f.ovf_hi = 0; } else f.ovf_lo = olo + 1;
+      } else {
 #if defined(__CUDA_ARCH__)
-        cur_head = __shfl_sync(0xffffffffu, bhead, where); cur_tail = __shfl_sync(0xffffffffu, btail, where);
+        head = __shfl_sync(0xffffffffu, bhead, where); f.cur_tail = __shfl_sync(0xffffffffu, btail, where);
         if (lane == where) bhead = -1;
 #else
-        cur_head = bhead[where]; cur_tail = btail[where]; bhead[where] = -1;
+        head = bhead[where]; f.cur_tail = btail[where]; bhead[where] = -1;
 #endif
       }
     }
-    const PEnt e = ent[cur_head];
-    ent[cur_head].next = free_head; free_head = cur_head;
-    cur_head = e.next;
-    if (cur_head < 0) cur_tail = -1;
+    const PEnt e = ent[head];
+    ent[head].next = f.free_head; f.free_head = head;
+    f.cur_head = e.next;
+    if (e.next < 0) f.cur_tail = -1;
     x = (int)(int16_t)(e.xy >> 16); y = (int)(int16_t)(e.xy & 0xffffu);
     return true;
   }
@@ -499,32 +539,35 @@ XM_HD inline double pa_estimate(const PathState& s, int x, int y, const PNode& n
 }
 // PathAligner.align :120-192: seeds the queue (:120-150) and runs the best-first search (:153-192) with explore
 // :722-729, update :555-571, computeUpdated :573-719, putNode :446-473 and estimateOverallPenalty :475-521 folded
-// into ONE compact loop: every per-search constant lives in a register, the three neighbours share one copy of the
-// update code, and base pairs are classified through the 256-entry tables.  This loop is where gapped reads spend
-// their time.  Returns 0 goal reached (last_x/last_y), 1 over budget (null), 2 failed (w.status set).
+// into ONE compact loop: every per-search constant is read from the warp's PaFrame where it is used, the three neighbours
+// share one copy of the update code, and base pairs are classified through the 256-entry tables.  This loop is where gapped
+// reads spend their time.  Returns 0 goal reached (last_x/last_y), 1 over budget (null), 2 failed (w.status set).
 XM_FN int pa_search(WS& w, PathState& S, PaOverflow* ovf, int cap_ovf, int& last_x, int& last_y) {
   XM_CHECK_MASK(w);
-  const int A = S.A, B = S.B, H = S.H, step = S.step, goal_x = S.goal_x, goal_y = S.goal_y, diag = S.diagonal;
-  const bool may_extend = S.may_extend != 0, confident = S.an_confident != 0;
-  const double ins_start = S.prm.ins_start, ins_ext = S.prm.ins_ext, del_start = S.prm.del_start, del_ext = S.prm.del_ext, unaligned = S.prm.unaligned;
-  const double max_ins = S.an_max_ins, max_del = S.an_max_del, budget = S.max_interesting + 0.000001;
-  const double min_indel = dmin(ins_start + ins_ext, del_start + del_ext);
-  const double* pen_tab = S.prm.pen_tab; const uint8_t* cls_tab = S.prm.cls_tab;
-  PNode* nodes = S.nodes; const uint8_t* qa = S.qa; const uint8_t* rb = S.rb;
-  const uint32_t gen = S.gen; const int W = S.W;
-  uint32_t clock = S.clock;
+#if defined(__CUDA_ARCH__)
+  PaFrame& F = pa_frame[threadIdx.x >> 5];
+#else
+  PaFrame frame; PaFrame& F = frame;
+#endif
+  F.A = S.A; F.B = S.B; F.H = S.H; F.step = S.step; F.goal_x = S.goal_x; F.goal_y = S.goal_y; F.diagonal = S.diagonal;
+  F.may_extend = S.may_extend != 0; F.confident = S.an_confident != 0;
+  F.ins_start = S.prm.ins_start; F.ins_ext = S.prm.ins_ext; F.del_start = S.prm.del_start; F.del_ext = S.prm.del_ext; F.unaligned = S.prm.unaligned;
+  F.max_ins = S.an_max_ins; F.max_del = S.an_max_del; F.budget = S.max_interesting + 0.000001;
+  F.min_indel = dmin(S.prm.ins_start + S.prm.ins_ext, S.prm.del_start + S.prm.del_ext);
+  F.pen_tab = S.prm.pen_tab; F.cls_tab = S.prm.cls_tab; F.nodes = S.nodes; F.qa = S.qa; F.rb = S.rb;
+  F.gen = S.gen; F.clock = S.clock; F.steps = 0;
   PaQueue Q;
-  Q.init(S.ent, S.ent_cap, ovf, cap_ovf);
+  Q.init(F, S.ent, S.ent_cap, ovf, cap_ovf);
   int qrc = 0;
   // seeding :120-150.  activePenalty is 0 here, estimates are never negative: no clamping needed.  One loop (one copy of
   // the queue code) walks the free-start nodes :120-139 and then the query-overhang nodes :140-150.
   {
-    const int start_x = S.start_x, start_y = S.start_y;
-    const bool along_y = B >= A;
+    const int A = S.A, B = S.B, step = S.step, start_x = S.start_x, start_y = S.start_y;
+    const bool along_y = B >= A, may_extend = S.may_extend != 0;
     double sisp = XM_DISALLOWED;
     if (along_y && may_extend) sisp = S.prm.starting_ins_start();
     const int cnt1 = (along_y ? imax(0, B - A) : imax(0, A - B)) + 1;
-    const int cnt2 = may_extend ? imax(0, j2i(S.an_max_ins / del_ext) - 1) : 0;
+    const int cnt2 = may_extend ? imax(0, j2i(S.an_max_ins / S.prm.del_ext) - 1) : 0;
     XM_NOUNROLL
     for (int i = 0; i < cnt1 + cnt2 && qrc == 0; i++) {
       PNode n; int x, y;
@@ -534,98 +577,128 @@ XM_FN int pa_search(WS& w, PathState& S, PaOverflow* ovf, int cap_ovf, int& last
       } else {
         const int k = i - cnt1 + 1;
         x = start_x + k * step; y = start_y;
-        n.pen = k * unaligned; n.ins_x = XM_DISALLOWED; n.ins_y = XM_DISALLOWED;
+        n.pen = k * S.prm.unaligned; n.ins_x = XM_DISALLOWED; n.ins_y = XM_DISALLOWED;
         // outside the lattice the reference still queues the node (saveNode ignores x < 0; x > width is stored but
         // never read), and popping it can end the search when its priority exceeds the budget
         if (x < -32000 || x > 32000) { qrc = 1; break; }
       }
-      n.stamp = ++clock; n.meta = gen << 8;
-      qrc = Q.push(pa_estimate(S, x, y, n, 0), x, y);
-      if (x >= 0 && x < W) nodes[x * H + y] = n;
+      const uint32_t clock = F.clock + 1;
+      F.clock = clock;
+      n.stamp = clock; n.meta = S.gen << 8;
+      qrc = Q.push(F, pa_estimate(S, x, y, n, 0), x, y);
+      if (x >= 0 && x < S.W) S.nodes[x * S.H + y] = n;
     }
   }
-  unsigned long long steps = 0;
   int rc = 2;
   XM_NOUNROLL
   while (qrc == 0) {
-    int tx, ty;
-    if (!Q.pop(tx, ty)) { w.fail(Q_INTERNAL); break; }  // priorities.poll() == null -> NullPointerException
-    const double active = Q.cur_key;
-    steps++;
-    if (active > budget) { rc = 1; break; }
-    if (tx == goal_x) { last_x = tx; last_y = ty; rc = 0; break; }
+    {
+      int tx, ty;
+      if (!Q.pop(F, tx, ty)) { w.fail(Q_INTERNAL); break; }  // priorities.poll() == null -> NullPointerException
+      F.tx = (int16_t)tx; F.ty = (int16_t)ty;
+      F.steps = F.steps + 1;
+      if (F.cur_key > F.budget) { rc = 1; break; }
+      if (tx == F.goal_x) { last_x = tx; last_y = ty; rc = 0; break; }
+    }
     XM_NOUNROLL
     for (int nb = 0; nb < 3; nb++) {  // (x+step, y), (x, y+step), (x+step, y+step)
-      const int x = tx + (nb != 1 ? step : 0), y = ty + (nb != 0 ? step : 0);
-      if (x <= 0 || x > A || y <= 0 || y > B) continue;
-      const int ie = x * H + y, il = ie - step * H, iu = ie - step, id = il - step;
-      // stamp (low word) and meta (high word) of the node and of its three predecessors: four independent 8-byte loads
-      const PMeta me = *(const PMeta*)&nodes[ie].stamp, ml = *(const PMeta*)&nodes[il].stamp, mu = *(const PMeta*)&nodes[iu].stamp, md = *(const PMeta*)&nodes[id].stamp;
-      const bool he = (me.meta >> 8) == gen, hl = (ml.meta >> 8) == gen, hu = (mu.meta >> 8) == gen, hd = (md.meta >> 8) == gen;
-      if (he) {
-        // every predecessor was last written before this node was: recomputing it would reproduce the values it holds (no improvement)
-        uint32_t newest = 0;
-        if (hl && ml.stamp > newest) newest = ml.stamp;
-        if (hu && mu.stamp > newest) newest = mu.stamp;
-        if (hd && md.stamp > newest) newest = md.stamp;
-        if (me.stamp > newest) continue;
+      {
+        const int step = pa_ld(F.step);
+        const int x = pa_ld(F.tx) + (nb != 1 ? step : 0), y = pa_ld(F.ty) + (nb != 0 ? step : 0);
+        if (x <= 0 || x > pa_ld(F.A) || y <= 0 || y > pa_ld(F.B)) continue;
+        F.x = (int16_t)x; F.y = (int16_t)y;
       }
-      const uint32_t fl_ = hl ? (1u | (ml.meta & 6u)) : 0u, fu = hu ? (1u | (mu.meta & 6u)) : 0u, fd = hd ? (1u | (md.meta & 6u)) : 0u;
+      // below, the neighbour's coordinates and index and the search's constants are read from the frame where they are used
+      uint32_t fpk;   // 3 flag bits (1 present | 6 reached) per predecessor: overlay, insertion, deletion
+      bool he;
+      {
+        PNode* const nodes = pa_ld(F.nodes);
+        const int step = pa_ld(F.step), ie = pa_ld(F.x) * pa_ld(F.H) + pa_ld(F.y), il = ie - step * pa_ld(F.H), iu = ie - step, id = il - step;
+        // stamp (low word) and meta (high word) of the node and of its three predecessors: four independent 8-byte loads
+        const PMeta me = *(const PMeta*)&nodes[ie].stamp, ml = *(const PMeta*)&nodes[il].stamp, mu = *(const PMeta*)&nodes[iu].stamp, md = *(const PMeta*)&nodes[id].stamp;
+        const uint32_t gen = pa_ld(F.gen);
+        he = (me.meta >> 8) == gen;
+        const bool hl = (ml.meta >> 8) == gen, hu = (mu.meta >> 8) == gen, hd = (md.meta >> 8) == gen;
+        if (he) {
+          // every predecessor was last written before this node was: recomputing it would reproduce the values it holds (no improvement)
+          uint32_t newest = 0;
+          if (hl && ml.stamp > newest) newest = ml.stamp;
+          if (hu && mu.stamp > newest) newest = mu.stamp;
+          if (hd && md.stamp > newest) newest = md.stamp;
+          if (me.stamp > newest) continue;
+        }
+        fpk = (hd ? (1u | (md.meta & 6u)) : 0u) | (hl ? (1u | (ml.meta & 6u)) << 3 : 0u) | (hu ? (1u | (mu.meta & 6u)) << 6 : 0u);
+      }
       double ins_x = XM_DISALLOWED, ins_y = XM_DISALLOWED, overlay = XM_DISALLOWED;
-      if (hd) overlay = nodes[id].pen + pen_tab[((int)qa[x - 1] << 4) | (int)rb[y - 1]];
-      if (hl) {
-        const double lp = nodes[il].pen;
-        if (y == goal_y && may_extend) ins_x = lp + unaligned;
-        else {
-          // qa / rb are padded with the sentinel code on both sides: an index off the section leaves the move allowed, as in the reference
-          bool allowed = (cls_tab[((int)qa[x - 1 - step] << 5) | (int)rb[y - 1]] & 1) != 0;
-          if (allowed) allowed = (cls_tab[((int)qa[x - 1] << 5) | (int)rb[y - 1 + step]] & 6) == 0;
-          const double nw = allowed ? lp + ins_start + ins_ext : XM_DISALLOWED;
-          ins_x = dmin(nodes[il].ins_x + ins_ext, nw);
+      {
+        PNode* const nodes = pa_ld(F.nodes);
+        const uint8_t* const qa = pa_ld(F.qa); const uint8_t* const rb = pa_ld(F.rb); const uint8_t* const cls_tab = pa_ld(F.cls_tab);
+        const int x = pa_ld(F.x), y = pa_ld(F.y), step = pa_ld(F.step), ie = x * pa_ld(F.H) + y;
+        if (fpk & 1u) overlay = nodes[ie - step * pa_ld(F.H) - step].pen + pa_ld(F.pen_tab)[((int)qa[x - 1] << 4) | (int)rb[y - 1]];
+        if (fpk & 8u) {
+          const int il = ie - step * pa_ld(F.H);
+          const double lp = nodes[il].pen;
+          if (y == pa_ld(F.goal_y) && pa_ld(F.may_extend)) ins_x = lp + pa_ld(F.unaligned);
+          else {
+            // qa / rb are padded with the sentinel code on both sides: an index off the section leaves the move allowed, as in the reference
+            bool allowed = (cls_tab[((int)qa[x - 1 - step] << 5) | (int)rb[y - 1]] & 1) != 0;
+            if (allowed) allowed = (cls_tab[((int)qa[x - 1] << 5) | (int)rb[y - 1 + step]] & 6) == 0;
+            const double nw = allowed ? lp + pa_ld(F.ins_start) + pa_ld(F.ins_ext) : XM_DISALLOWED;
+            ins_x = dmin(nodes[il].ins_x + pa_ld(F.ins_ext), nw);
+          }
+        }
+        if (fpk & 64u) {
+          const int iu = ie - step;
+          bool allowed = (cls_tab[((int)qa[x - 1] << 5) | (int)rb[y - 1 - step]] & 1) != 0;
+          if (allowed) allowed = (cls_tab[((int)qa[x - 1 + step] << 5) | (int)rb[y - 1]] & 6) == 0;
+          const double nw = allowed ? nodes[iu].pen + pa_ld(F.del_start) + pa_ld(F.del_ext) : XM_DISALLOWED;
+          ins_y = dmin(nodes[iu].ins_y + pa_ld(F.del_ext), nw);
         }
       }
-      if (hu) {
-        bool allowed = (cls_tab[((int)qa[x - 1] << 5) | (int)rb[y - 1 - step]] & 1) != 0;
-        if (allowed) allowed = (cls_tab[((int)qa[x - 1 + step] << 5) | (int)rb[y - 1]] & 6) == 0;
-        const double nw = allowed ? nodes[iu].pen + del_start + del_ext : XM_DISALLOWED;
-        ins_y = dmin(nodes[iu].ins_y + del_ext, nw);
-      }
       const double best = dmin(dmin(overlay, ins_x), ins_y);
-      if (he && !(best < nodes[ie].pen || ins_x < nodes[ie].ins_x || ins_y < nodes[ie].ins_y)) continue;
-      const int sd = x - y - diag;
+      if (he) {
+        const PNode* const o = pa_ld(F.nodes) + (pa_ld(F.x) * pa_ld(F.H) + pa_ld(F.y));
+        if (!(best < o->pen || ins_x < o->ins_x || ins_y < o->ins_y)) continue;
+      }
+      const int sd = pa_ld(F.x) - pa_ld(F.y) - pa_ld(F.diagonal);
       int fl = 0;
       if (best != XM_DISALLOWED) {
-        const int src = (best == overlay) ? fd : (best == ins_x) ? fl_ : fu;
-        fl = (src & 6) | (sd == 0 ? 2 : 4);
+        const uint32_t src = (best == overlay) ? fpk : (best == ins_x) ? fpk >> 3 : fpk >> 6;
+        fl = (int)(src & 6u) | (sd == 0 ? 2 : 4);
       }
       // estimateOverallPenalty :475-521
       double est = best;
-      if (confident) {
-        const int sds = sd * step;
+      if (pa_ld(F.confident)) {
+        const int sds = sd * pa_ld(F.step);
         if (fl & 2) {
-          const bool over = (sds > 0) ? (fabs(sd * ins_ext) > max_ins) : (fabs(sd * del_ext) > max_del);
+          const bool over = (sds > 0) ? (fabs(sd * pa_ld(F.ins_ext)) > pa_ld(F.max_ins)) : (fabs(sd * pa_ld(F.del_ext)) > pa_ld(F.max_del));
           if (over) est = XM_DISALLOWED;
-          else if (!(fl & 4)) est = best + min_indel;
+          else if (!(fl & 4)) est = best + pa_ld(F.min_indel);
         } else if (sds < 0) {
-          const double ie_ = fabs(sd * ins_ext);
-          if (ie_ > max_ins) est = XM_DISALLOWED;
-          else est = best + dmin(ins_start, ins_x - best) + ie_;
+          const double ie_ = fabs(sd * pa_ld(F.ins_ext));
+          if (ie_ > pa_ld(F.max_ins)) est = XM_DISALLOWED;
+          else est = best + dmin(pa_ld(F.ins_start), ins_x - best) + ie_;
         } else {
-          const double de = fabs(sd * del_ext);
-          if (de > max_del) est = XM_DISALLOWED;
-          else est = best + dmin(del_start, ins_y - best) + de;
+          const double de = fabs(sd * pa_ld(F.del_ext));
+          if (de > pa_ld(F.max_del)) est = XM_DISALLOWED;
+          else est = best + dmin(pa_ld(F.del_start), ins_y - best) + de;
         }
       }
+      // the node is stored before it is queued, so that none of its values has to outlive the queue code; a push that fails
+      // ends the search with Q_NEED_MORE, and no later search reads a node of this generation
+      const uint32_t clock = pa_ld(F.clock) + 1;
+      F.clock = clock;
+      PNode n; n.pen = best; n.ins_x = ins_x; n.ins_y = ins_y; n.stamp = clock; n.meta = (pa_ld(F.gen) << 8) | (uint32_t)fl;
+      pa_ld(F.nodes)[(pa_ld(F.x) * pa_ld(F.H) + pa_ld(F.y))] = n;
+      const double active = pa_ld(F.cur_key);
       if (est < active) est = active;
-      qrc = Q.push(est, x, y);
+      qrc = Q.push(F, est, pa_ld(F.x), pa_ld(F.y));
       if (qrc != 0) break;
-      PNode n; n.pen = best; n.ins_x = ins_x; n.ins_y = ins_y; n.stamp = ++clock; n.meta = (gen << 8) | (uint32_t)fl;
-      nodes[ie] = n;
     }
   }
-  S.clock = clock;
+  S.clock = F.clock;
   if (qrc != 0) { w.fail(Q_NEED_MORE); rc = 2; }
-  w.st_path_steps += steps;
+  w.st_path_steps += F.steps;
   return rc;
 }
 
