@@ -45,24 +45,19 @@ XM_INLINE DAln aln_null() { DAln a; a.valid = 0; a.n = 0; a.b = nullptr; a.penal
 XM_FN double block_penalty(const Params& p, const ACtx& c, const Blk& k) {  // AlignmentParameters.getPenalty(AlignedBlock) :106-126
   double pen = 0;
   if (k.a_len == k.b_len) {
-#if defined(__CUDA_ARCH__)
     // lanes classify 32 base pairs at a time; the non-zero penalties are then added in base order (x + 0.0 == x, so
     // skipping the zero terms keeps the reference's left-to-right double sum bit for bit)
-    const int lane = (int)(threadIdx.x & 31);
+    const int lane = lane_id();
     XM_NOUNROLL
-    for (int base = 0; base < k.a_len; base += 32) {
+    for (int base = 0; base < k.a_len; base += XM_LANES) {
       const int i = base + lane;
       double v = 0;
       if (i < k.a_len) v = p.base_penalty(c.a.at(k.a_start + i), c.b.at(k.b_start + i));
-      unsigned m = __ballot_sync(0xffffffffu, v != 0);
+      unsigned m = warp_ballot(v != 0);
       XM_NOUNROLL
-      while (m) { const int src = __ffs(m) - 1; m &= m - 1; pen += __shfl_sync(0xffffffffu, v, src); }
+      while (m) { const int src = first_bit(m) - 1; m &= m - 1; pen += warp_shfl(v, src); }
     }
-    __syncwarp();
-#else
-    XM_NOUNROLL
-    for (int i = 0; i < k.a_len; i++) pen += p.base_penalty(c.a.at(k.a_start + i), c.b.at(k.b_start + i));
-#endif
+    warp_sync();
   } else if (k.a_len > 0) { pen += p.ins_start; pen += p.ins_ext * k.a_len; }
   else { pen += p.del_start; pen += p.del_ext * k.b_len; }
   return pen;
@@ -70,22 +65,17 @@ XM_FN double block_penalty(const Params& p, const ACtx& c, const Blk& k) {  // A
 XM_FN double block_penalty_range(const Params& p, const SeqView& a, const SeqView& b, const Blk& k, int start_b, int end_b) {  // :128-154
   double pen = 0;
   if (k.a_len == k.b_len) {
-#if defined(__CUDA_ARCH__)
-    const int lane = (int)(threadIdx.x & 31);
+    const int lane = lane_id();
     XM_NOUNROLL
-    for (int base = 0; base < k.a_len; base += 32) {
+    for (int base = 0; base < k.a_len; base += XM_LANES) {
       const int i = base + lane, bi = k.b_start + i;
       double v = 0;
       if (i < k.a_len && bi >= start_b && bi < end_b) v = p.base_penalty(a.at(k.a_start + i), b.at(bi));
-      unsigned m = __ballot_sync(0xffffffffu, v != 0);
+      unsigned m = warp_ballot(v != 0);
       XM_NOUNROLL
-      while (m) { const int src = __ffs(m) - 1; m &= m - 1; pen += __shfl_sync(0xffffffffu, v, src); }
+      while (m) { const int src = first_bit(m) - 1; m &= m - 1; pen += warp_shfl(v, src); }
     }
-    __syncwarp();
-#else
-    XM_NOUNROLL
-    for (int i = 0; i < k.a_len; i++) { int bi = k.b_start + i; if (bi >= start_b && bi < end_b) pen += p.base_penalty(a.at(k.a_start + i), b.at(bi)); }
-#endif
+    warp_sync();
   } else if (k.b_start < end_b && k.b_start + k.b_len > start_b) {
     if (k.a_len > 0) { pen += p.ins_start; pen += p.ins_ext * k.a_len; } else { pen += p.del_start; pen += p.del_ext * k.b_len; }
   }
@@ -196,19 +186,14 @@ XM_FN int matcher_section_value(WS& w, MatcherD& m, const SeqView& ref, int sect
       slot = m.slots_used++;
       m.slot_section[slot] = section_index;
       int16_t* t = m.tables + (long long)slot * m.table_entries;
-#if defined(__CUDA_ARCH__)
-      {  // lanes clear the table together (16 bytes per lane per round)
+      {  // lanes clear the table to T_NO together (16 bytes per lane per round; table_entries is a multiple of 8)
         uint4 fill = make_uint4(0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu);
         uint4* t4 = (uint4*)t;
         int n16 = m.table_entries / 8;
         XM_NOUNROLL
-        for (int i = (int)(threadIdx.x & 31); i < n16; i += 32) t4[i] = fill;
-        __syncwarp();
+        for (int i = lane_id(); i < n16; i += XM_LANES) t4[i] = fill;
+        warp_sync();
       }
-#else
-      XM_NOUNROLL
-      for (int i = 0; i < m.table_entries; i++) t[i] = T_NO;
-#endif
       matcher_scan_encodings(m, ref, section_index, [&](int rel, int enc) { t[enc] = (t[enc] == T_NO) ? (int16_t)rel : T_MULTI; });
     }
     if (slot >= 0) {
@@ -720,14 +705,9 @@ XM_FN DAln path_align(WS& w, const ACtx& c, const Sec& q, const Sec& r, const Pa
     qa += 2; rb += 2;   // two sentinel codes (16) on either side: the search reads one position past both ends (xm_types.h: Params::cls_tab)
     XM_NOUNROLL
     for (int k = 0; k < 2; k++) { qa[-1 - k] = 16; qa[s.A + k] = 16; rb[-1 - k] = 16; rb[s.B + k] = 16; }
-#if defined(__CUDA_ARCH__)
-    for (int k = (int)(threadIdx.x & 31); k < s.A; k += 32) qa[k] = c.a.at(s.start_a + k);
-    for (int k = (int)(threadIdx.x & 31); k < s.B; k += 32) rb[k] = c.b.at(s.start_b + k);
-    __syncwarp();
-#else
-    for (int k = 0; k < s.A; k++) qa[k] = c.a.at(s.start_a + k);
-    for (int k = 0; k < s.B; k++) rb[k] = c.b.at(s.start_b + k);
-#endif
+    for (int k = lane_id(); k < s.A; k += XM_LANES) qa[k] = c.a.at(s.start_a + k);
+    for (int k = lane_id(); k < s.B; k += XM_LANES) rb[k] = c.b.at(s.start_b + k);
+    warp_sync();
     s.qa = qa; s.rb = rb;
   }
   w.st_path_calls++; w.st_path_cells += (unsigned long long)s.A * (unsigned long long)s.B;
@@ -735,26 +715,16 @@ XM_FN DAln path_align(WS& w, const ACtx& c, const Sec& q, const Sec& r, const Pa
     int sum_mis = 0, num_mis = 0, sum_mat = 0, num_mat = 0;
     int si = imax(s.start_a, s.start_b - an.predicted), ei = imin(s.end_a, s.end_b - an.predicted);
     int length = ei - si;
-#if defined(__CUDA_ARCH__)
     XM_NOUNROLL
-    for (int i = (int)(threadIdx.x & 31); i < length; i += 32) {  // integer sums: any order
+    for (int i = lane_id(); i < length; i += XM_LANES) {  // integer sums: any order
       int j = i - s.diagonal;
       if (j >= 0 && j < s.B) {
         if (!bp_can_match(pa_qa(s, i), pa_rb(s, j))) { sum_mis += i; num_mis++; } else { sum_mat += i; num_mat++; }
       }
     }
-    __syncwarp();   // different trip counts above: converge before the warp-shared search state is written
-    sum_mis = __reduce_add_sync(0xffffffffu, sum_mis); num_mis = __reduce_add_sync(0xffffffffu, num_mis);
-    sum_mat = __reduce_add_sync(0xffffffffu, sum_mat); num_mat = __reduce_add_sync(0xffffffffu, num_mat);
-#else
-    XM_NOUNROLL
-    for (int i = 0; i < length; i++) {
-      int j = i - s.diagonal;
-      if (j >= 0 && j < s.B) {
-        if (!bp_can_match(pa_qa(s, i), pa_rb(s, j))) { sum_mis += i; num_mis++; } else { sum_mat += i; num_mat++; }
-      }
-    }
-#endif
+    warp_sync();   // different trip counts above: converge before the warp-shared search state is written
+    sum_mis = warp_sum(sum_mis); num_mis = warp_sum(num_mis);
+    sum_mat = warp_sum(sum_mat); num_mat = warp_sum(num_mat);
     s.reverse = (num_mis > 1 && num_mat > 1) ? ((sum_mis / num_mis) > (sum_mat / num_mat) ? 1 : 0) : 1;
   }
   if (s.reverse) { s.step = -1; s.may_extend = (s.start_b == 0); } else { s.step = 1; s.may_extend = (s.end_b == c.b.len); }
@@ -768,24 +738,16 @@ XM_FN DAln path_align(WS& w, const ACtx& c, const Sec& q, const Sec& r, const Pa
   {
     uint32_t gen = w.cell_hdr[0];
     if (gen == 0 || gen >= 0xFFFFFF) {   // first search in this arena since the launch began, or the 24-bit generation wrapped: clear the region
-      const long long n16 = (w.cell_words + 3) >> 2;
-#if defined(__CUDA_ARCH__)
+      const long long n16 = (w.cell_words + 3) >> 2;   // cell_words is a multiple of 4 (ws_init)
       uint4* c4 = (uint4*)w.cellmap;
       XM_NOUNROLL
-      for (long long i = (long long)(threadIdx.x & 31); i < n16; i += 32) c4[i] = make_uint4(0u, 0u, 0u, 0u);
-      __syncwarp();
-#else
-      for (long long i = 0; i < w.cell_words; i++) w.cellmap[i] = 0;
-#endif
+      for (long long i = (long long)lane_id(); i < n16; i += XM_LANES) c4[i] = make_uint4(0u, 0u, 0u, 0u);
+      warp_sync();
       gen = 0;
     }
     gen++;
-#if defined(__CUDA_ARCH__)
-    if ((threadIdx.x & 31) == 0) w.cell_hdr[0] = gen;
-    __syncwarp();
-#else
-    w.cell_hdr[0] = gen;
-#endif
+    if (lane_id() == 0) w.cell_hdr[0] = gen;
+    warp_sync();
     s.nodes = (PNode*)w.cellmap; s.gen = gen; s.clock = 0;
   }
   long long remaining = w.scratch_size - w.scratch_top;
@@ -1060,43 +1022,26 @@ XM_FN PenaltyAnalysisD hba_analyze(WS& w, const ACtx& c, const Sec& q, const Sec
       int other = position;
       int reverse_count = imin(bs - max_nonmatch_end, other);
       bool found = false;
-#if defined(__CUDA_ARCH__)
-      const int lane = (int)(threadIdx.x & 31);
+      const int lane = lane_id();
       XM_NOUNROLL
-      for (int base = 1; base <= reverse_count && !found; base += 32) {  // any mismatch among the bases left of the block
+      for (int base = 1; base <= reverse_count && !found; base += XM_LANES) {  // any mismatch among the bases left of the block
         const int i = base + lane;
         const bool bad = (i <= reverse_count) && !bp_can_match(c.a.at(bs - i), c.b.at(other - i));
-        if (__ballot_sync(0xffffffffu, bad) != 0) found = true;
+        if (warp_ballot(bad) != 0) found = true;
       }
-      __syncwarp();
+      warp_sync();
       if (found) { num_mis++; max_nonmatch_end = bs + bl; }
-#else
-      XM_NOUNROLL
-      for (int i = 1; i <= reverse_count; i++) {
-        if (!bp_can_match(c.a.at(bs - i), c.b.at(other - i))) { num_mis++; found = true; max_nonmatch_end = bs + bl; break; }
-      }
-#endif
       if (!found) {
         int fwd = q.end - bs;
-#if defined(__CUDA_ARCH__)
         XM_NOUNROLL
-        for (int base = bl; base < fwd && !found; base += 32) {  // first mismatch right of the block
+        for (int base = bl; base < fwd && !found; base += XM_LANES) {  // first mismatch right of the block
           const int i = base + lane, ia = bs + i, ib = other + i;
           bool bad = false;
           if (i < fwd) { uint8_t ca = c.a.at(ia); uint8_t cb = (ib < r.end) ? c.b.at(ib) : (uint8_t)0; bad = !bp_can_match(ca, cb); }
-          const unsigned m = __ballot_sync(0xffffffffu, bad);
-          if (m != 0) { num_mis++; found = true; max_nonmatch_end = bs + base + (__ffs(m) - 1) + 1; }
+          const unsigned m = warp_ballot(bad);
+          if (m != 0) { num_mis++; found = true; max_nonmatch_end = bs + base + (first_bit(m) - 1) + 1; }
         }
-        __syncwarp();
-#else
-        XM_NOUNROLL
-        for (int i = bl; i < fwd; i++) {
-          int ia = bs + i, ib = other + i;
-          uint8_t ca = c.a.at(ia);
-          uint8_t cb = (ib < r.end) ? c.b.at(ib) : (uint8_t)0;
-          if (!bp_can_match(ca, cb)) { num_mis++; found = true; max_nonmatch_end = ia + 1; break; }
-        }
-#endif
+        warp_sync();
         if (!found) max_nonmatch_end = q.end;
         int num_other = 0;
         int fwd2 = max_nonmatch_end - bs - bl;
@@ -1276,17 +1221,12 @@ XM_HD inline DAln cascade_t(WS& w, const ACtx& c, const Sec& q, const Sec& r, co
   if constexpr (STAGE == ST_STRAIGHT1 || STAGE == ST_STRAIGHT2 || STAGE == ST_STRAIGHT3) return straight_align_t<false, STAGE>(w, c, q, r, p, an);
   else if constexpr (STAGE == ST_SKIP) {  // SkipHighAmbiguity_Aligner.align :13-28
     int amb = 0;
-#if defined(__CUDA_ARCH__)
     XM_NOUNROLL
-    for (int base = r.start; base < r.end; base += 32) {
-      const int i = base + (int)(threadIdx.x & 31);
-      amb += __popc(__ballot_sync(0xffffffffu, i < r.end && bp_is_ambiguous(c.b.at(i))));
+    for (int base = r.start; base < r.end; base += XM_LANES) {
+      const int i = base + lane_id();
+      amb += bit_count(warp_ballot(i < r.end && bp_is_ambiguous(c.b.at(i))));
     }
-    __syncwarp();
-#else
-    XM_NOUNROLL
-    for (int i = r.start; i < r.end; i++) if (bp_is_ambiguous(c.b.at(i))) amb++;
-#endif
+    warp_sync();
     if (amb >= r.length() / 4) return aln_null();
     return cascade_t<STAGE + 1>(w, c, q, r, p, an);
   }
@@ -1389,27 +1329,27 @@ XM_FN DAln qma_align_match(WS& w, const ACtx& c, const SM& sm, const Params& p, 
   an.max_ins = max_interesting - p.ins_start; an.max_del = max_interesting - p.del_start;
   an.predicted = best_offset; an.confident = sm.from_hash ? 1 : 0;
   if (EASY) return straight_align_t<true, ST_STRAIGHT1>(w, c, q, r, p, an);
-#if defined(__CUDA_ARCH__)
   {  // every stage of the cascade reads the reference through this window: fetch it once - by TMA into shared memory when it fits the
      // warp's staging area, else unpacked from global memory into the arena (lanes split the bases)
     const int wn = r.end - r.start;
+#if defined(__CUDA_ARCH__)
     const uint8_t* sw = stage_window(w, c.b, r.start, r.end);
     if (sw != nullptr) {
       ACtx cw = c;
       cw.b.bytes = sw; cw.b.b0 = r.start; cw.b.bn = wn;
       return cascade_t<ST_STRAIGHT1>(w, cw, q, r, p, an);
     }
+#endif
     if (wn > 0 && w.scratch_top + wn + 64 <= w.scratch_size) {
       uint8_t* wb = (uint8_t*)w.salloc(wn);
       XM_NOUNROLL
-      for (int k = (int)(threadIdx.x & 31); k < wn; k += 32) wb[k] = c.b.at(r.start + k);
-      __syncwarp();
+      for (int k = lane_id(); k < wn; k += XM_LANES) wb[k] = c.b.at(r.start + k);
+      warp_sync();
       ACtx cw = c;
       cw.b.bytes = wb; cw.b.b0 = r.start; cw.b.bn = wn;
       return cascade_t<ST_STRAIGHT1>(w, cw, q, r, p, an);
     }
   }
-#endif
   return cascade_t<ST_STRAIGHT1>(w, c, q, r, p, an);
 }
 XM_HD inline bool sa_store_from(WS& w, SAStore& out, const DAln& a, int contig, int a_mate, int a_rev) {
@@ -2023,12 +1963,8 @@ XM_HD inline bool ws_init(WS& w, char* arena, long long arena_bytes, const RefD*
       int len = q.seq[i].len;
       uint8_t* f = (uint8_t*)take(len + 1); uint8_t* r = (uint8_t*)take(len + 1);
       SeqView pv = q.seq[i]; pv.rc = 0; pv.bytes = nullptr;
-#if defined(__CUDA_ARCH__)
-      for (int k = (int)(threadIdx.x & 31); k < len; k += 32) { uint8_t c = pv.at(k); f[k] = c; r[len - 1 - k] = bp_complement(c); }
-      __syncwarp();
-#else
-      for (int k = 0; k < len; k++) { uint8_t c = pv.at(k); f[k] = c; r[len - 1 - k] = bp_complement(c); }
-#endif
+      for (int k = lane_id(); k < len; k += XM_LANES) { uint8_t c = pv.at(k); f[k] = c; r[len - 1 - k] = bp_complement(c); }
+      warp_sync();
       w.qbytes[i][0] = f; w.qbytes[i][1] = r;
       w.query.seq[i].bytes = nullptr;
     }

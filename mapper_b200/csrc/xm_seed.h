@@ -79,19 +79,20 @@ XM_FN HB merge_blocks(const HB& L, const HB& R, int level) {  // HashBlock(seq,s
 }
 
 XM_INLINE int ext_char_to_int(uint8_t c) { return c == 1 ? 1 : c == 2 ? 2 : c == 4 ? 3 : c == 8 ? 4 : 0; }
+XM_HD constexpr uint32_t upow(uint32_t b, int e) { uint32_t r = 1u; while (e-- > 0) r *= b; return r; }
 
 // HashBlock.withGapAndExtension :67-150. false = null
 // h = fold(h * 7654337 + value(base)) over n bases starting at `from`, stepping `dir` (HashBlock.java:107-135).
 // Integer wrap-around arithmetic is a ring, so on the device 32 lanes each take one base of a 32-base chunk,
 // weight it with the matching power of the multiplier and add the chunk up with shuffles: same 32-bit result.
+// With one lane (the host emulation) a chunk is one base and each round is h = h * M1 + value: the fold itself.
 XM_HD inline int32_t ext_hash(const SeqView& seq, int from, int n, int dir, bool complement) {
   int32_t h = 0;
-#if defined(__CUDA_ARCH__)
-  constexpr uint32_t M1 = 7654337u, M2 = M1 * M1, M4 = M2 * M2, M8 = M4 * M4, M16 = M8 * M8, M32 = M16 * M16;
-  const int lane = (int)(threadIdx.x & 31);
+  constexpr uint32_t M1 = 7654337u, M2 = M1 * M1, M4 = M2 * M2, M8 = M4 * M4, M16 = M8 * M8, MW = upow(M1, XM_LANES);
+  const int lane = lane_id();
   XM_NOUNROLL
-  for (int base = 0; base < n; base += 32) {
-    const int cnt = imin(32, n - base);
+  for (int base = 0; base < n; base += XM_LANES) {
+    const int cnt = imin(XM_LANES, n - base);
     uint32_t term = 0;
     if (lane < cnt) {
       uint8_t c = seq.at(from + dir * (base + lane));
@@ -105,23 +106,12 @@ XM_HD inline int32_t ext_hash(const SeqView& seq, int from, int n, int dir, bool
       if (e & 16) pw *= M16;
       term = (uint32_t)ext_char_to_int(c) * pw;
     }
-    __syncwarp();
-    term += __shfl_xor_sync(0xffffffffu, term, 16);
-    term += __shfl_xor_sync(0xffffffffu, term, 8);
-    term += __shfl_xor_sync(0xffffffffu, term, 4);
-    term += __shfl_xor_sync(0xffffffffu, term, 2);
-    term += __shfl_xor_sync(0xffffffffu, term, 1);
-    uint32_t pc = (cnt == 32) ? M32 : 1u;
-    if (cnt != 32) { if (cnt & 1) pc *= M1; if (cnt & 2) pc *= M2; if (cnt & 4) pc *= M4; if (cnt & 8) pc *= M8; if (cnt & 16) pc *= M16; }
+    warp_sync();
+    term = warp_xor_sum(term);
+    uint32_t pc = (cnt == XM_LANES) ? MW : 1u;
+    if (cnt != XM_LANES) { if (cnt & 1) pc *= M1; if (cnt & 2) pc *= M2; if (cnt & 4) pc *= M4; if (cnt & 8) pc *= M8; if (cnt & 16) pc *= M16; }
     h = (int32_t)((uint32_t)h * pc + term);
   }
-#else
-  for (int k = 0; k < n; k++) {
-    uint8_t c = seq.at(from + dir * k);
-    if (complement) c = bp_complement(c);
-    h = wadd(wmul(h, 7654337), ext_char_to_int(c));
-  }
-#endif
   return h;
 }
 XM_FN bool with_gap_and_extension(const HB& b, const SeqView& seq, HB& out) {
@@ -482,30 +472,21 @@ XM_FN bool pyr_build(WS& w, MatePath& m) {
   const int len = m.q.len;
   XM_CHECK_MASK(w);
   if (len > P.cap_blocks || P.cap_levels < 2 || len > 32000) { w.fail(Q_NEED_MORE); return false; }
-#if defined(__CUDA_ARCH__)
-  const int lane = (int)(threadIdx.x & 31);
+  const int lane = lane_id();
   const unsigned lt_mask = (1u << lane) - 1u;
   bool amb = false;
   XM_NOUNROLL
-  for (int k = lane; k < len; k += 32) {
+  for (int k = lane; k < len; k += XM_LANES) {
     uint8_t code = m.q.at(k);
     amb |= bp_is_ambiguous(code);
     P.blk[k] = base_block16(code, k); P.child[k] = -1; P.up[k] = -1;
   }
   // The lanes leave the loop after different trip counts.  A vote synchronises them for the vote only; what follows (the scalar
   // MultiHashBlock build in particular) is executed by every lane on the same warp-shared state and needs the warp CONVERGED.
-  __syncwarp();
+  warp_sync();
   XM_CHECK_MASK(w);
-  amb = __any_sync(0xffffffffu, amb);
+  amb = warp_any(amb);
   XM_CHECK_MASK(w);
-#else
-  bool amb = false;
-  for (int k = 0; k < len; k++) {
-    uint8_t code = m.q.at(k);
-    amb |= bp_is_ambiguous(code);
-    P.blk[k] = base_block16(code, k); P.child[k] = -1; P.up[k] = -1;
-  }
-#endif
   P.level_off[0] = 0; P.level_off[1] = len; P.n_levels = 1;
   P.opt = nullptr; P.n_opt = 0; P.cap_opt = 0;
   if (amb) return pyr_build_ambiguous(w, m);  // IUPAC-ambiguous query bases: MultiHashBlocks, scalar build
@@ -515,10 +496,9 @@ XM_FN bool pyr_build(WS& w, MatePath& m) {
     if (level >= P.cap_levels) { w.fail(Q_NEED_MORE); return false; }
     const int cur_off = prev_off + n_prev;
     int n_new = 0;
-#if defined(__CUDA_ARCH__)
-    __syncwarp();
+    warp_sync();
     XM_NOUNROLL
-    for (int base = 0; base < n_prev - 1; base += 32) {
+    for (int base = 0; base < n_prev - 1; base += XM_LANES) {
       const int i = base + lane;
       const bool valid = i < n_prev - 1;
       bool keep = false;
@@ -527,27 +507,15 @@ XM_FN bool pyr_build(WS& w, MatePath& m) {
         L = P.blk[prev_off + i]; R = P.blk[prev_off + i + 1];
         keep = ((int)L.start + (int)L.len >= (int)R.start) && ((L.flags & 2) || (R.flags & 1));  // shouldMergeBlocks :200-208
       }
-      const unsigned mask = __ballot_sync(0xffffffffu, keep);
-      const int total = __popc(mask);
+      const unsigned mask = warp_ballot(keep);
+      const int total = bit_count(mask);
       if (cur_off + n_new + total > P.cap_blocks) { w.fail(Q_NEED_MORE); return false; }
-      const int pos = n_new + __popc(mask & lt_mask);
+      const int pos = n_new + bit_count(mask & lt_mask);
       if (keep) { P.blk[cur_off + pos] = merge_blocks16(L, R); P.child[cur_off + pos] = (int16_t)i; P.up[cur_off + pos] = -1; }
       if (valid) P.up[prev_off + i] = keep ? (int16_t)pos : (int16_t)-1;
       n_new += total;
     }
-    __syncwarp();
-#else
-    for (int i = 0; i < n_prev - 1; i++) {
-      const HB16 L = P.blk[prev_off + i], R = P.blk[prev_off + i + 1];
-      bool keep = ((int)L.start + (int)L.len >= (int)R.start) && ((L.flags & 2) || (R.flags & 1));
-      if (keep) {
-        if (cur_off + n_new + 1 > P.cap_blocks) { w.fail(Q_NEED_MORE); return false; }
-        P.blk[cur_off + n_new] = merge_blocks16(L, R); P.child[cur_off + n_new] = (int16_t)i; P.up[cur_off + n_new] = -1;
-        P.up[prev_off + i] = (int16_t)n_new;
-        n_new++;
-      } else P.up[prev_off + i] = -1;
-    }
-#endif
+    warp_sync();
     if (n_new == 0) break;
     P.level_off[level + 1] = cur_off + n_new; P.n_levels = level + 1;
     prev_off = cur_off; n_prev = n_new; level++;
@@ -854,33 +822,24 @@ XM_FN bool counting_step(WS& w, MatePath& m) {  // step :40-179
   const int64_t pos0 = (int64_t)(word >> 24);   // first position of the bucket
   // Each hit is verified independently (flank comparison, :98-153); the bins are then updated in bucket order.
   // On the device 32 lanes verify 32 hits at a time and lane results are replayed in order by the whole warp.
-#if defined(__CUDA_ARCH__)
-  const int lane = (int)(threadIdx.x & 31);
+  const int lane = lane_id();
   XM_NOUNROLL
-  for (int base = 0; base < count; base += 32) {
-    const int n = imin(32, count - base);
+  for (int base = 0; base < count; base += XM_LANES) {
+    const int n = imin(XM_LANES, count - base);
     SM mine; mine.mate = -1; mine.rev = 0; mine.contig = 0; mine.offset = 0; mine.from_hash = 1;
     if (lane < n) mine = verify_hit(w, m, qb, t->position(pos0 + base + lane), invert);
-    __syncwarp();   // back from the divergent call: the replay below updates warp-shared state with every lane
+    warp_sync();   // back from the divergent call: the replay below updates warp-shared state with every lane
     XM_NOUNROLL
     for (int j = 0; j < n; j++) {
       SM full;
-      full.mate = __shfl_sync(0xffffffffu, mine.mate, j);
+      full.mate = warp_shfl(mine.mate, j);
       if (full.mate < 0) continue;
-      full.rev = __shfl_sync(0xffffffffu, mine.rev, j); full.contig = __shfl_sync(0xffffffffu, mine.contig, j);
-      full.offset = __shfl_sync(0xffffffffu, mine.offset, j); full.from_hash = 1;
+      full.rev = warp_shfl(mine.rev, j); full.contig = warp_shfl(mine.contig, j);
+      full.offset = warp_shfl(mine.offset, j); full.from_hash = 1;
       counting_update_matches(w, m, full, qb, count);
       if (w.status != 0) return false;
     }
   }
-#else
-  for (int k = 0; k < count; k++) {
-    SM full = verify_hit(w, m, qb, t->position(pos0 + k), invert);
-    if (full.mate < 0) continue;
-    counting_update_matches(w, m, full, qb, count);
-    if (w.status != 0) return false;
-  }
-#endif
   if (qb.start >= m.max_nonoverlap_visited) { m.max_nonoverlap_visited = qb.end(); m.n_nonoverlap_visited++; }
   m.n_blocks_anywhere++;
   m.min_num_distinct = -1;

@@ -2,6 +2,7 @@
 // This header is compiled by nvcc for sm_100a (the product) and by g++ for the test-only host emulation
 // harness (tests/emu/), which exists so the device logic can be checked against the oracle on a box without a
 // GPU.  The shipped library never runs this code on the CPU.
+// One source serves both builds, lane-split loops included: see "the warp" below.
 #pragma once
 #include <stdint.h>
 #include <math.h>
@@ -18,6 +19,9 @@
 #define XM_INLINE inline
 #define XM_FN inline
 #define XM_NOUNROLL
+// CUDA's 16-byte vector for the lane-strided clears; may_alias: it writes over int16_t / uint32_t arrays
+struct __attribute__((may_alias)) uint4 { uint32_t x, y, z, w; };
+inline uint4 make_uint4(uint32_t x, uint32_t y, uint32_t z, uint32_t w) { uint4 v; v.x = x; v.y = y; v.z = z; v.w = w; return v; }
 #endif
 
 #if defined(XM_TRACE) && !defined(__CUDA_ARCH__)
@@ -176,9 +180,45 @@ struct OutArena {
   unsigned long long* stats;   // [0] probes [1] seeds [2] hits [3] straight [4] path calls [5] path steps [6] path cells
 };
 
+// ---- the warp ----
 // On the device one WARP owns a query and all 32 lanes execute the per-query code in lock step on identical
 // values (warp-uniform control flow; data-parallel inner loops are split across lanes where marked).  Side effects
 // that must happen once per query are issued by lane 0 and their result is broadcast.
+// Lane-split loops are written once, through the helpers below (on the device: the intrinsic with the full mask).  The host
+// emulation is a warp of one lane - a ballot is the predicate, a shuffle or a sum returns its argument, warp_sync() does
+// nothing - so such a loop runs serially in base order; compaction across lanes, the replay of lanes j > 0 and the xor tree
+// run only on the GPU.  nvcc's host pass sees XM_LANES == 1 too: no type or host-side size may depend on it.
+#if defined(__CUDA_ARCH__)
+static constexpr int XM_LANES = 32;
+__device__ __forceinline__ int lane_id() { return (int)(threadIdx.x & 31); }
+__device__ __forceinline__ unsigned warp_ballot(bool p) { return __ballot_sync(0xffffffffu, p); }
+__device__ __forceinline__ bool warp_any(bool p) { return __any_sync(0xffffffffu, p); }
+template <class T> __device__ __forceinline__ T warp_shfl(T v, int src) { return __shfl_sync(0xffffffffu, v, src); }
+__device__ __forceinline__ int warp_sum(int v) { return __reduce_add_sync(0xffffffffu, v); }
+__device__ __forceinline__ uint32_t warp_xor_sum(uint32_t v) {  // every lane gets the (wrapping) sum of all 32
+  v += __shfl_xor_sync(0xffffffffu, v, 16);
+  v += __shfl_xor_sync(0xffffffffu, v, 8);
+  v += __shfl_xor_sync(0xffffffffu, v, 4);
+  v += __shfl_xor_sync(0xffffffffu, v, 2);
+  v += __shfl_xor_sync(0xffffffffu, v, 1);
+  return v;
+}
+__device__ __forceinline__ void warp_sync() { __syncwarp(); }
+__device__ __forceinline__ int first_bit(unsigned m) { return __ffs(m); }   // 1 + index of the lowest set bit, 0 for none
+__device__ __forceinline__ int bit_count(unsigned m) { return __popc(m); }
+#else
+static constexpr int XM_LANES = 1;
+inline int lane_id() { return 0; }
+inline unsigned warp_ballot(bool p) { return p ? 1u : 0u; }
+inline bool warp_any(bool p) { return p; }
+template <class T> inline T warp_shfl(T v, int) { return v; }
+inline int warp_sum(int v) { return v; }
+inline uint32_t warp_xor_sum(uint32_t v) { return v; }
+inline void warp_sync() {}
+inline int first_bit(unsigned m) { return __builtin_ffs((int)m); }
+inline int bit_count(unsigned m) { return __builtin_popcount(m); }
+#endif
+
 XM_INLINE unsigned long long xm_atomic_add(unsigned long long* p, unsigned long long v) {
 #if defined(__CUDA_ARCH__)
   unsigned long long o = 0;

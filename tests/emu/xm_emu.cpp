@@ -2,6 +2,10 @@
 // It lets the kernel logic be compared with the oracle on a box without a GPU, one query per loop iteration,
 // with the same workspace tiers the CUDA launcher uses.  It is NOT part of the product: libxmapper_b200.so never
 // contains this file and has no CPU path.
+// The emulation runs the device source itself: the per-query code's lane-split loops are written through the warp helpers of
+// xm_types.h, which g++ compiles as a warp of one lane (XM_LANES = 1), so each loop runs serially in base order.  What one lane
+// cannot exercise - compaction across lanes, the replay of lanes j > 0, the xor tree across lanes - and the device-only parts
+// (the lattice search's 32-bucket queue and shared-memory frame, TMA staging) are covered by the GPU tests only.
 #include <cstring>
 #include "../../mapper_b200/csrc/xm_align.h"
 #include "../../mapper_b200/csrc/xm_host_model.h"
