@@ -645,18 +645,34 @@ __global__ void xm_sam_kernel(SamD S, BatchD batch, int nq) {
 }
 
 // ---------------------------------------------------------------- handle
+// The one owner of device memory in this file: every cudaMalloc / cudaFree is here, and a buffer is freed when its owner goes away.
 struct DevBuf {
   void* p = nullptr; size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  DevBuf(DevBuf&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+  DevBuf& operator=(DevBuf&& o) noexcept { if (this != &o) { release(); p = o.p; cap = o.cap; o.p = nullptr; o.cap = 0; } return *this; }
+  ~DevBuf() { release(); }
   bool ensure(size_t bytes) {
     if (bytes <= cap) return true;
-    if (p) cudaFree(p);
-    p = nullptr; cap = 0;
+    release();
     size_t want = bytes + bytes / 8 + 256;
     if (cudaMalloc(&p, want) != cudaSuccess) { cudaGetLastError(); if (cudaMalloc(&p, bytes) != cudaSuccess) { p = nullptr; return false; } want = bytes; }
     cap = want;
     return true;
   }
   void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+  // ensure (at least 16 bytes) + a synchronous host->device copy
+  bool upload(const void* src, size_t bytes) { return ensure(bytes ? bytes : 16) && (!bytes || cudaMemcpy(p, src, bytes, cudaMemcpyHostToDevice) == cudaSuccess); }
+  // exactly `bytes`, keeping the first keep_bytes (copied on st, which is synchronised); on failure the old buffer stays as it was
+  bool grow(size_t bytes, size_t keep_bytes, cudaStream_t st) {
+    void* np = nullptr;
+    if (cudaMalloc(&np, bytes) != cudaSuccess) { cudaGetLastError(); return false; }
+    if ((keep_bytes && cudaMemcpyAsync(np, p, keep_bytes, cudaMemcpyDeviceToDevice, st) != cudaSuccess) || cudaStreamSynchronize(st) != cudaSuccess) { cudaFree(np); return false; }
+    release(); p = np; cap = bytes;
+    return true;
+  }
 };
 
 #include "xm_counts.cuh"
@@ -786,6 +802,7 @@ struct xm_handle {
 };
 
 static double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+static double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
 #define CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { h->err = std::string(#call) + ": " + cudaGetErrorString(e_); return XM_ERR_CUDA; } } while (0)
 // RAII lease of a batch slot: the least recently used free one, so that the device copies of recent results live as long as possible
@@ -804,23 +821,26 @@ struct SlotLease {
   xm_handle::BatchSlot& slot() { return h->slots[i]; }
 };
 
+// the reference codes and their layout, and the device view of them (h->ref)
+static int upload_reference(xm_handle* h) {
+  const HostModel& M = h->m;
+  if (!h->d_words.upload(M.words.data(), M.words.size() * 2) || !h->d_word_off.upload(M.word_off.data(), M.word_off.size() * 8) ||
+      !h->d_len.upload(M.len.data(), M.len.size() * 4) || !h->d_gstart.upload(M.gstart.data(), M.gstart.size() * 8)) { h->err = "device upload failed (reference)"; return XM_ERR_CUDA; }
+  h->ref.n_contigs = M.n_contigs; h->ref.words = (const uint16_t*)h->d_words.p; h->ref.word_off = (const int64_t*)h->d_word_off.p;
+  h->ref.len = (const int32_t*)h->d_len.p; h->ref.gstart = (const int64_t*)h->d_gstart.p; h->ref.total_fr = M.total_fr;
+  return XM_OK;
+}
+
 static int mirror_model(xm_handle* h) {
   HostModel& M = h->m;
   if (h->mirrored_generation == M.generation && h->mirrored_dup_generation == M.dup_generation) return XM_OK;
   if (M.n_contigs < 1) { h->err = "reference not set"; return XM_ERR_STATE; }
   if (!M.index_finished) { h->err = "index not set (xm_set_index_length + xm_finish_index, or xm_build_index)"; return XM_ERR_STATE; }
-  auto up = [&](DevBuf& b, const void* src, size_t bytes) -> bool {
-    if (!b.ensure(bytes ? bytes : 16)) return false;
-    if (bytes && cudaMemcpy(b.p, src, bytes, cudaMemcpyHostToDevice) != cudaSuccess) return false;
-    return true;
-  };
   bool ok = true;
   if (h->mirrored_generation != M.generation) {   // reference + index tables
-    ok = up(h->d_words, M.words.data(), M.words.size() * 2) && up(h->d_word_off, M.word_off.data(), M.word_off.size() * 8) &&
-         up(h->d_len, M.len.data(), M.len.size() * 4) && up(h->d_gstart, M.gstart.data(), M.gstart.size() * 8);
+    if (int rc = upload_reference(h)) return rc;
     size_t nt = (size_t)M.max_built + 1;
     if (M.tables.size() < nt) M.tables.resize(nt);
-    for (auto& b : h->d_ix_chunks) b.release();
     h->d_ix_chunks.clear();
     h->d_buckets.resize(nt); h->d_positions.resize(nt); h->d_positions_hi.resize(nt);
     std::vector<TableD> tabs(nt);
@@ -828,23 +848,20 @@ static int mirror_model(xm_handle* h) {
       const HostTable& T = M.tables[i];
       tabs[i].capacity = T.capacity; tabs[i].max_count = T.max_count; tabs[i].buckets = nullptr; tabs[i].positions = nullptr; tabs[i].positions_hi = nullptr;
       if (!T.buckets.empty()) {
-        ok = up(h->d_buckets[i], T.buckets.data(), T.buckets.size() * 8) && up(h->d_positions[i], T.positions.data(), T.positions.size() * 4);
+        ok = h->d_buckets[i].upload(T.buckets.data(), T.buckets.size() * 8) && h->d_positions[i].upload(T.positions.data(), T.positions.size() * 4);
         tabs[i].buckets = (const uint64_t*)h->d_buckets[i].p; tabs[i].positions = (const uint32_t*)h->d_positions[i].p;
-        if (ok && !T.positions_hi.empty()) { ok = up(h->d_positions_hi[i], T.positions_hi.data(), T.positions_hi.size()); tabs[i].positions_hi = (const uint8_t*)h->d_positions_hi[i].p; }
+        if (ok && !T.positions_hi.empty()) { ok = h->d_positions_hi[i].upload(T.positions_hi.data(), T.positions_hi.size()); tabs[i].positions_hi = (const uint8_t*)h->d_positions_hi[i].p; }
       }
     }
-    ok = ok && up(h->d_tables, tabs.data(), nt * sizeof(TableD));
+    ok = ok && h->d_tables.upload(tabs.data(), nt * sizeof(TableD));
     h->tables_host = tabs;
   }
   if (ok) {   // the duplication table (small; re-uploaded on its own when only it changed)
-    std::vector<int64_t> doff((size_t)M.n_contigs + 1, 0); std::vector<int32_t> dst;
-    for (int c = 0; c < M.n_contigs; c++) { if ((size_t)c < M.dup_starts.size()) dst.insert(dst.end(), M.dup_starts[(size_t)c].begin(), M.dup_starts[(size_t)c].end()); doff[(size_t)c + 1] = (int64_t)dst.size(); }
-    dst.push_back(0);
-    ok = up(h->d_dup_off, doff.data(), doff.size() * 8) && up(h->d_dup_starts, dst.data(), dst.size() * 4);
+    std::vector<int64_t> doff; std::vector<int32_t> dst;
+    M.dup_csr(doff, dst);
+    ok = h->d_dup_off.upload(doff.data(), doff.size() * 8) && h->d_dup_starts.upload(dst.data(), dst.size() * 4);
   }
   if (!ok) { h->err = std::string("device upload failed: ") + cudaGetErrorString(cudaGetLastError()); return XM_ERR_CUDA; }
-  h->ref.n_contigs = M.n_contigs; h->ref.words = (const uint16_t*)h->d_words.p; h->ref.word_off = (const int64_t*)h->d_word_off.p;
-  h->ref.len = (const int32_t*)h->d_len.p; h->ref.gstart = (const int64_t*)h->d_gstart.p; h->ref.total_fr = M.total_fr;
   h->ix.min_interesting = M.min_interesting; h->ix.max_built = M.max_built; h->ix.gapmers = M.gapmers; h->ix.tables = (const TableD*)h->d_tables.p;
   h->dup.window = M.dup_window; h->dup.granularity = M.dup_granularity; h->dup.off = (const int64_t*)h->d_dup_off.p; h->dup.starts = (const int32_t*)h->d_dup_starts.p;
   h->mirrored_generation = M.generation; h->mirrored_dup_generation = M.dup_generation;
@@ -955,6 +972,44 @@ __global__ void __launch_bounds__(128) xm_dup_scan_kernel(DupScanD D) {
     }
   }
 }
+// xm_dup_scan_kernel<GROUPS> over the tables of lengths min_len..max_len.  The records come back in `recs` and stay in `d_recs`:
+// the ancestry code goes on reading them on the device.
+template <class Rec> struct DupScan { std::vector<Rec> recs; DevBuf d_recs; int n_groups = 0; };
+template <bool GROUPS, class Rec>
+static int dup_scan(xm_handle* h, int min_len, int max_len, int min_copies, DupScan<Rec>& out) {
+  const char* what = GROUPS ? "ancestry group" : "duplication";
+  cudaStream_t st = h->stream;
+  const int blocks = h->sm_count * 8, warps = blocks * 4;
+  int max_items = 2;
+  for (int bl = std::max(1, min_len); bl <= max_len; bl++) max_items = std::max(max_items, 2 * h->tables_host[(size_t)bl].max_count);
+  DevBuf d_scratch, d_n;
+  DupScanD D; D.ref = h->ref; D.min_copies = min_copies; D.max_items = max_items; D.recs = nullptr; D.grecs = nullptr;
+  D.scratch_stride = (((long long)max_items * (long long)(sizeof(DupItem) + (GROUPS ? 12 : 0))) + 255) & ~255LL;
+  if (!d_scratch.ensure((size_t)warps * (size_t)D.scratch_stride) || !d_n.ensure(16)) { h->err = std::string("out of device memory (") + what + " scan)"; return XM_ERR_CUDA; }
+  D.scratch = (char*)d_scratch.p; D.n_recs = (unsigned long long*)d_n.p; D.n_groups = (int*)((char*)d_n.p + 8);
+  unsigned long long cap = 1ull << 20, found = 0;
+  for (int attempt = 0; attempt < 2; attempt++) {   // second attempt: the buffer sized by the first one's count
+    if (!out.d_recs.ensure((size_t)cap * sizeof(Rec))) { h->err = std::string("out of device memory (") + what + " records)"; return XM_ERR_CUDA; }
+    if constexpr (GROUPS) D.grecs = (Rec*)out.d_recs.p; else D.recs = (Rec*)out.d_recs.p;
+    D.cap = cap;
+    CK(cudaMemsetAsync(d_n.p, 0, 16, st));
+    for (int bl = std::max(1, min_len); bl <= max_len; bl++) {
+      const TableD& T = h->tables_host[(size_t)bl];
+      if (T.buckets == nullptr) continue;
+      D.t = T; D.bl = bl; D.prefix = (bl + 3) / 4;
+      xm_dup_scan_kernel<GROUPS><<<blocks, 128, 0, st>>>(D);
+    }
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(&found, d_n.p, 8, cudaMemcpyDeviceToHost, st));
+    if (GROUPS) CK(cudaMemcpyAsync(&out.n_groups, (char*)d_n.p + 8, 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (found <= cap) break;
+    cap = found;
+  }
+  out.recs.resize((size_t)found);
+  if (found) CK(cudaMemcpy(out.recs.data(), out.d_recs.p, (size_t)found * sizeof(Rec), cudaMemcpyDeviceToHost));
+  return XM_OK;
+}
 static int build_duplications_device(xm_handle* h, int min_len, int max_len, int min_copies, int window) {
   HostModel& M = h->m;
   if (min_len < 0) min_len = M.choose_min_dup_len();
@@ -963,44 +1018,15 @@ static int build_duplications_device(xm_handle* h, int min_len, int max_len, int
   if (max_len > 64) { h->err = "xm_build_duplications: block lengths above 64 are not supported by the device scan (128-bit text keys); xm_build_duplications_host takes any length"; return XM_ERR_ARG; }
   if (min_copies < 1) min_copies = 1;
   const bool trace = getenv("XM_TRACE_SETUP") != nullptr;
-  auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-  const double t_begin = now();
+  const double t_begin = now_s();
   if (int rc = mirror_model(h)) return rc;
-  const double t_mirror = now();
-  cudaStream_t st = h->stream;
-  const int blocks = h->sm_count * 8, warps = blocks * 4;
-  int max_items = 2;
-  for (int bl = std::max(1, min_len); bl <= max_len; bl++) max_items = std::max(max_items, 2 * h->tables_host[(size_t)bl].max_count);
-  DevBuf d_scratch, d_recs, d_n;
-  struct Free { std::vector<DevBuf*> v; ~Free() { for (DevBuf* b : v) b->release(); } } fr;
-  fr.v = {&d_scratch, &d_recs, &d_n};
-  DupScanD D; D.ref = h->ref; D.min_copies = min_copies;
-  D.scratch_stride = (((long long)max_items * (long long)sizeof(DupItem)) + 255) & ~255LL;
-  if (!d_scratch.ensure((size_t)warps * (size_t)D.scratch_stride) || !d_n.ensure(16)) { h->err = "out of device memory (duplication scan)"; return XM_ERR_CUDA; }
-  D.scratch = (char*)d_scratch.p; D.n_recs = (unsigned long long*)d_n.p;
-  unsigned long long cap = 1ull << 20, found = 0;
-  std::vector<HostModel::DupRecH> recs;
-  for (int attempt = 0; attempt < 2; attempt++) {   // second attempt: the buffer sized by the first one's count
-    if (!d_recs.ensure((size_t)cap * sizeof(HostModel::DupRecH))) { h->err = "out of device memory (duplication records)"; return XM_ERR_CUDA; }
-    D.recs = (HostModel::DupRecH*)d_recs.p; D.cap = cap;
-    CK(cudaMemsetAsync(d_n.p, 0, 16, st));
-    for (int bl = std::max(1, min_len); bl <= max_len; bl++) {
-      const TableD& T = h->tables_host[(size_t)bl];
-      if (T.buckets == nullptr) continue;
-      D.t = T; D.bl = bl; D.prefix = (bl + 3) / 4;
-      xm_dup_scan_kernel<false><<<blocks, 128, 0, st>>>(D);
-    }
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(&found, d_n.p, 8, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    if (found <= cap) break;
-    cap = found;
-  }
-  const double t_scan = now();
-  recs.resize((size_t)found);
-  if (found) CK(cudaMemcpy(recs.data(), d_recs.p, (size_t)found * sizeof(HostModel::DupRecH), cudaMemcpyDeviceToHost));
-  M.merge_duplications(recs, min_len, window);
-  if (trace) fprintf(stderr, "[xm] duplications: mirror %.3f s, device scan of lengths %d..%d %.3f s (%llu blocks found), merge %.3f s\n", t_mirror - t_begin, min_len, max_len, t_scan - t_mirror, found, now() - t_scan);
+  const double t_mirror = now_s();
+  DupScan<HostModel::DupRecH> S;
+  if (int rc = dup_scan<false>(h, min_len, max_len, min_copies, S)) return rc;
+  const double t_scan = now_s();
+  const size_t found = S.recs.size();
+  M.merge_duplications(S.recs, min_len, window);
+  if (trace) fprintf(stderr, "[xm] duplications: mirror %.3f s, device scan of lengths %d..%d %.3f s (%zu blocks found), merge %.3f s\n", t_mirror - t_begin, min_len, max_len, t_scan - t_mirror, found, now_s() - t_scan);
   return XM_OK;
 }
 
@@ -1262,21 +1288,10 @@ void xm_destroy(xm_handle* h) {
   cudaSetDevice(h->device);
   if (h->comm && nccl_api().ok) { nccl_api().CommDestroy(h->comm); h->comm = nullptr; }
   for (auto& sl : h->slots) {
-    for (DevBuf* b : {&sl.d_packed, &sl.d_seq_word_off, &sl.d_seq_len, &sl.d_n_seqs, &sl.d_expected, &sl.d_per, &sl.d_first_seq, &sl.d_csr_slab}) b->release();
     if (sl.copy) cudaStreamDestroy(sl.copy);
     for (cudaEvent_t e : {sl.h2d_done, sl.kernels_done, sl.ev0, sl.ev1}) if (e) cudaEventDestroy(e);
   }
-  DevBuf* bufs[] = {&h->d_words, &h->d_word_off, &h->d_len, &h->d_gstart, &h->d_tables, &h->d_dup_off, &h->d_dup_starts, &h->d_chunk, &h->d_q, &h->d_choices, &h->d_sas, &h->d_blocks,
-                    &h->d_misc, &h->d_ids_a, &h->d_ids_b, &h->d_ids_full, &h->d_ws, &h->d_qcycles, &h->d_csr_cnt, &h->d_csr_base, &h->d_csr_tmp, &h->d_keys_a, &h->d_keys_b, &h->d_sort_tmp, &h->d_big, &h->d_big_busy, &h->d_sam_len, &h->d_sam_text, &h->d_sam_names, &h->d_sam_name_off, &h->d_sam_cnames, &h->d_sam_cname_off, &h->d_planes, &h->d_contig_off, &h->d_var, &h->d_var_n, &h->d_order, &h->d_var_sizes,
-                    &h->var_scratch.keys_a, &h->var_scratch.keys_b, &h->var_scratch.idx_a, &h->var_scratch.idx_b, &h->var_scratch.gathered, &h->var_scratch.out_keys, &h->var_scratch.n_out, &h->var_scratch.tmp,
-                    &h->d_ex_words, &h->d_ex_word_off, &h->d_ex_len, &h->d_ex_gids, &h->d_ex_slot, &h->d_ex_bad,
-                    &h->d_fmt_dec, &h->d_fmt_state, &h->d_fmt_len, &h->d_fmt_range, &h->d_fmt_name, &h->d_fmt_text, &h->d_fmt_tmp, &h->d_fmt_ids};
-  for (DevBuf* b : bufs) b->release();
   if (h->fmt_text) h->pinned->give(h->fmt_text, h->fmt_cap);
-  for (auto& b : h->d_buckets) b.release();
-  for (auto& b : h->d_positions) b.release();
-  for (auto& b : h->d_positions_hi) b.release();
-  for (auto& b : h->d_ix_chunks) b.release();
   if (h->stream) cudaStreamDestroy(h->stream);
   for (cudaEvent_t e : {h->ev2, h->ev3, h->ev4, h->ev5}) if (e) cudaEventDestroy(e);
   delete h;
@@ -1341,12 +1356,9 @@ static int build_index_device(xm_handle* h, int max_used, int min_interesting = 
   if (hi > 16000) { h->err = "xm_build_index: lengths above 16000 are not supported by the device builder (16-bit block coordinates within a slice)"; return XM_ERR_ARG; }
   int key_bits = 33; while ((1 << (key_bits - 32)) <= hi) key_bits++;   // sort key = used << 32 | bucket
   cudaStream_t st = h->stream;
-  auto up = [&](DevBuf& b, const void* src, size_t bytes) -> bool { return b.ensure(bytes ? bytes : 16) && (!bytes || cudaMemcpy(b.p, src, bytes, cudaMemcpyHostToDevice) == cudaSuccess); };
-  if (!up(h->d_words, M.words.data(), M.words.size() * 2) || !up(h->d_word_off, M.word_off.data(), M.word_off.size() * 8) ||
-      !up(h->d_len, M.len.data(), M.len.size() * 4) || !up(h->d_gstart, M.gstart.data(), M.gstart.size() * 8)) { h->err = "device upload failed (reference)"; return XM_ERR_CUDA; }
+  if (int rc = upload_reference(h)) return rc;
   IndexBuildD B;
-  B.ref.n_contigs = M.n_contigs; B.ref.words = (const uint16_t*)h->d_words.p; B.ref.word_off = (const int64_t*)h->d_word_off.p;
-  B.ref.len = (const int32_t*)h->d_len.p; B.ref.gstart = (const int64_t*)h->d_gstart.p; B.ref.total_fr = M.total_fr;
+  B.ref = h->ref;
   const int slice_len = 8192;
   std::vector<int> sc, ss, amb_sc, amb_ss;   // plain slices; slices whose window holds an IUPAC-ambiguous base (the host builder's test)
   for (int c = 0; c < M.n_contigs; c++) for (int s0 = 0; s0 < M.len[(size_t)c]; s0 += slice_len) {
@@ -1362,9 +1374,7 @@ static int build_index_device(xm_handle* h, int max_used, int min_interesting = 
   if (n_amb && slice_len + 4 * hi + 256 > 32000) { h->err = "xm_build_index: hash lengths this long are not supported on IUPAC-ambiguous references (16-bit window coordinates)"; return XM_ERR_ARG; }
   DevBuf d_amb_sc, d_amb_ss, d_amb_arena, d_keep, d_pos_hi;
   DevBuf d_sc, d_ss, d_cap, d_cnt, d_keys_a, d_keys_b, d_vals_a, d_vals_b, d_tmp, d_run_key, d_run_cnt, d_nruns, d_cnt64, d_kept, d_first, d_bbase, d_buckets, d_pos;
-  struct Free { std::vector<DevBuf*> v; ~Free() { for (DevBuf* b : v) b->release(); } } fr;
-  fr.v = {&d_amb_sc, &d_amb_ss, &d_amb_arena, &d_keep, &d_pos_hi, &d_sc, &d_ss, &d_cap, &d_cnt, &d_keys_a, &d_keys_b, &d_vals_a, &d_vals_b, &d_tmp, &d_run_key, &d_run_cnt, &d_nruns, &d_cnt64, &d_kept, &d_first, &d_bbase, &d_buckets, &d_pos};
-  if (!up(d_sc, sc.data(), sc.size() * 4) || !up(d_ss, ss.data(), ss.size() * 4) || !up(d_cap, cap.data(), cap.size() * 4) || !d_cnt.ensure(64)) { h->err = "out of device memory (index build)"; return XM_ERR_CUDA; }
+  if (!d_sc.upload(sc.data(), sc.size() * 4) || !d_ss.upload(ss.data(), ss.size() * 4) || !d_cap.upload(cap.data(), cap.size() * 4) || !d_cnt.ensure(64)) { h->err = "out of device memory (index build)"; return XM_ERR_CUDA; }
   B.slice_contig = (const int*)d_sc.p; B.slice_start = (const int*)d_ss.p; B.n_slices = (int)sc.size(); B.slice_len = slice_len;
   B.hi = hi; B.min_interesting = M.min_interesting; B.gapmers = M.gapmers; B.cap = (const int*)d_cap.p;
   const int blocks = h->sm_count * 8, warps = blocks * 4;
@@ -1376,7 +1386,7 @@ static int build_index_device(xm_handle* h, int max_used, int min_interesting = 
   IndexBuildD A = B;
   int amb_blocks = 0;
   if (n_amb) {
-    if (!up(d_amb_sc, amb_sc.data(), amb_sc.size() * 4) || !up(d_amb_ss, amb_ss.data(), amb_ss.size() * 4)) { h->err = "out of device memory (index build)"; return XM_ERR_CUDA; }
+    if (!d_amb_sc.upload(amb_sc.data(), amb_sc.size() * 4) || !d_amb_ss.upload(amb_ss.data(), amb_ss.size() * 4)) { h->err = "out of device memory (index build)"; return XM_ERR_CUDA; }
     const long long wlen = slice_len + 4LL * hi + 256;
     long long amb_mb = 64; if (const char* e = getenv("XM_INDEX_AMB_ARENA_MB")) amb_mb = std::max(8, atoi(e));
     A.arena_bytes = ((((wlen + 3) * 4 + 15) & ~15LL) + (10 * wlen + 256) * 20 + 64 + (amb_mb << 20) + 255) & ~255LL;
@@ -1386,7 +1396,7 @@ static int build_index_device(xm_handle* h, int max_used, int min_interesting = 
     A.arenas = (char*)d_amb_arena.p;
     A.slice_contig = (const int*)d_amb_sc.p; A.slice_start = (const int*)d_amb_ss.p; A.n_slices = n_amb;
   }
-  DevBuf d_hist; fr.v.push_back(&d_hist);
+  DevBuf d_hist;
   if (!d_hist.ensure(((size_t)hi + 2) * 8)) { h->err = "out of device memory (index build)"; return XM_ERR_CUDA; }
   int used_lo = 0, used_hi = 0x7fffffff;   // the block lengths of the current chunk
   auto emit = [&](unsigned long long* keys, void* vals, unsigned long long cap_entries) -> int {
@@ -1438,11 +1448,7 @@ static int build_index_device(xm_handle* h, int max_used, int min_interesting = 
     chunks.push_back({lo, hi});
   }
   if (getenv("XM_TRACE_SETUP")) fprintf(stderr, "[xm] index build: %llu entries for block lengths <= %d, at most %llu per sort: %zu chunk(s) of lengths\n", E, hi, max_entries, chunks.size());
-  for (auto& b : h->d_buckets) b.release();
-  for (auto& b : h->d_positions) b.release();
-  for (auto& b : h->d_positions_hi) b.release();
-  for (auto& b : h->d_ix_chunks) b.release();
-  h->d_ix_chunks.clear();
+  h->d_buckets.clear(); h->d_positions.clear(); h->d_positions_hi.clear(); h->d_ix_chunks.clear();   // the old tables go before the new ones are allocated
   std::vector<TableD> tabs((size_t)hi + 1);
   for (int k = 0; k <= hi; k++) { tabs[(size_t)k].capacity = 1; tabs[(size_t)k].max_count = 1; tabs[(size_t)k].buckets = nullptr; tabs[(size_t)k].positions = nullptr; tabs[(size_t)k].positions_hi = nullptr; }
   auto sort_fill = [&](auto pos_tag) -> int {
@@ -1504,7 +1510,7 @@ static int build_index_device(xm_handle* h, int max_used, int min_interesting = 
     for (int k = 0; k <= hi; k++) { bbase[(size_t)k] = words; if (first[(size_t)k + 1] > first[(size_t)k]) words += cap[(size_t)k]; }
     const long long n_pos = koff[(size_t)hi + 1];
     tab_bbase = bbase; tab_koff = koff;
-    if (!up(d_bbase, bbase.data(), bbase.size() * 8) || !d_buckets.ensure((size_t)words * 8 + 16) || !d_pos.ensure((size_t)n_pos * 4 + 16) || (wide && !d_pos_hi.ensure((size_t)n_pos + 16))) { h->err = "out of device memory (index tables)"; return XM_ERR_CUDA; }
+    if (!d_bbase.upload(bbase.data(), bbase.size() * 8) || !d_buckets.ensure((size_t)words * 8 + 16) || !d_pos.ensure((size_t)n_pos * 4 + 16) || (wide && !d_pos_hi.ensure((size_t)n_pos + 16))) { h->err = "out of device memory (index tables)"; return XM_ERR_CUDA; }
     IndexFillD<PosT> F;
     F.run_key = (const unsigned long long*)d_run_key.p; F.run_cnt = (const int*)d_run_cnt.p; F.run_start = run_start; F.kept_off = kept_off; F.n_runs = n_runs;
     F.first_run = (const int*)d_first.p; F.cap = (const int*)d_cap.p; F.bucket_base = (const long long*)d_bbase.p;
@@ -1544,7 +1550,7 @@ static int build_index_device(xm_handle* h, int max_used, int min_interesting = 
   }
   M.max_built = hi; M.index_finished = true; M.generation++;
   // the tables stay where the fill kernels wrote them: the device view is current, nothing is uploaded again
-  if (!up(h->d_tables, tabs.data(), tabs.size() * sizeof(TableD))) { h->err = "device upload failed (index tables)"; return XM_ERR_CUDA; }
+  if (!h->d_tables.upload(tabs.data(), tabs.size() * sizeof(TableD))) { h->err = "device upload failed (index tables)"; return XM_ERR_CUDA; }
   h->tables_host = tabs;
   h->mirrored_generation = M.generation; h->mirrored_dup_generation = ~0ull;   // mirror_model still uploads the duplication table and sets the views
   return XM_OK;
@@ -1553,56 +1559,25 @@ static int build_index_device(xm_handle* h, int max_used, int min_interesting = 
 static int infer_ancestors_device(xm_handle* h, double threshold, int min_interesting, int max_short, bool verify, int64_t* n_changed) {
   HostModel& M = h->m;
   const bool trace = getenv("XM_TRACE_SETUP") != nullptr;
-  auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-  const double t_begin = now();
+  const double t_begin = now_s();
   *n_changed = 0;
   // a) the temporary index: lengths up to 2 * minDuplicationLength (M/DuplicationDetector.java:17-31)
   const int min_len = M.choose_min_dup_len(), max_len = 2 * min_len;
   if (max_len > 64) { h->err = "xm_infer_ancestors: duplication lengths above 64 (a reference over 2^32 bases) are not supported by the device scan"; return XM_ERR_ARG; }
   if (int rc = build_index_device(h, max_len, min_interesting, max_short)) return rc;
   if (int rc = mirror_model(h)) return rc;
-  const double t_index = now();
+  const double t_index = now_s();
   // b) the group scan: DuplicationDetector(3 copies, window 1) :129-214, every member of every group
   cudaStream_t st = h->stream;
   const int blocks = h->sm_count * 8, warps = blocks * 4;
-  int max_items = 2;
-  for (int bl = min_len; bl <= max_len; bl++) max_items = std::max(max_items, 2 * h->tables_host[(size_t)bl].max_count);
-  DevBuf d_scratch, d_recs, d_n, d_keys, d_vals, d_keys2, d_vals2, d_tmp, d_goff, d_moff, d_mst, d_mlen, d_mgid, d_groups, d_state, d_pop, d_bits, d_plane, d_fwd_off,
-         d_ovf, d_retry, d_retry_off;
-  struct Free { std::vector<DevBuf*> v; ~Free() { for (DevBuf* b : v) b->release(); } } fr;
-  fr.v = {&d_scratch, &d_recs, &d_n, &d_keys, &d_vals, &d_keys2, &d_vals2, &d_tmp, &d_goff, &d_moff, &d_mst, &d_mlen, &d_mgid, &d_groups, &d_state, &d_pop, &d_bits, &d_plane,
-          &d_fwd_off, &d_ovf, &d_retry, &d_retry_off};
-  DupScanD D; D.ref = h->ref; D.min_copies = 3; D.max_items = max_items; D.recs = nullptr;
-  D.scratch_stride = (((long long)max_items * (long long)(sizeof(DupItem) + 12)) + 255) & ~255LL;
-  if (!d_scratch.ensure((size_t)warps * (size_t)D.scratch_stride) || !d_n.ensure(64)) { h->err = "out of device memory (ancestry group scan)"; return XM_ERR_CUDA; }
-  D.scratch = (char*)d_scratch.p; D.n_recs = (unsigned long long*)d_n.p; D.n_groups = (int*)((char*)d_n.p + 8);
-  unsigned long long cap = 1ull << 20, found = 0;
-  int n_groups = 0;
-  for (int attempt = 0; attempt < 2; attempt++) {   // second attempt: the buffer sized by the first one's count
-    if (!d_recs.ensure((size_t)cap * sizeof(HostModel::DupGrpRec))) { h->err = "out of device memory (ancestry group records)"; return XM_ERR_CUDA; }
-    D.grecs = (HostModel::DupGrpRec*)d_recs.p; D.cap = cap;
-    CK(cudaMemsetAsync(d_n.p, 0, 64, st));
-    for (int bl = min_len; bl <= max_len; bl++) {
-      const TableD& T = h->tables_host[(size_t)bl];
-      if (T.buckets == nullptr) continue;
-      D.t = T; D.bl = bl; D.prefix = (bl + 3) / 4;
-      xm_dup_scan_kernel<true><<<blocks, 128, 0, st>>>(D);
-    }
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(&found, d_n.p, 8, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(&n_groups, (char*)d_n.p + 8, 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    if (found <= cap) break;
-    cap = found;
-  }
-  if (found >= (1ull << 31)) { h->err = "xm_infer_ancestors: more than 2^31 duplication group members"; return XM_ERR_ARG; }
-  const int n_rec = (int)found;
-  std::vector<HostModel::DupGrpRec> recs((size_t)n_rec);
-  if (n_rec) CK(cudaMemcpy(recs.data(), d_recs.p, (size_t)n_rec * sizeof(HostModel::DupGrpRec), cudaMemcpyDeviceToHost));
-  const double t_scan = now();
+  DupScan<HostModel::DupGrpRec> S;
+  if (int rc = dup_scan<true>(h, min_len, max_len, 3, S)) return rc;
+  if (S.recs.size() >= (1ull << 31)) { h->err = "xm_infer_ancestors: more than 2^31 duplication group members"; return XM_ERR_ARG; }
+  const int n_rec = (int)S.recs.size(), n_groups = S.n_groups;
+  const double t_scan = now_s();
   // c) saveDuplications with the groups kept, every sequence; the groups some merged entry still references (DuplicationDetector.getAll)
   std::vector<std::vector<std::pair<int32_t, HostModel::Dup>>> by_seq;
-  M.merge_duplication_groups(recs, 1, by_seq);
+  M.merge_duplication_groups(S.recs, 1, by_seq);
   const size_t n_seqs = 2 * (size_t)M.n_contigs;
   std::vector<int64_t> moff(n_seqs + 1, 0);
   std::vector<int32_t> mst, mlen, mgid;
@@ -1613,18 +1588,18 @@ static int infer_ancestors_device(xm_handle* h, double threshold, int min_intere
   }
   std::vector<int32_t> groups;
   for (int g = 0; g < n_groups; g++) if (referenced[(size_t)g]) groups.push_back(g);
-  const double t_merge = now();
+  const double t_merge = now_s();
   double t_analysis = t_merge;
   int n_retried = 0;
+  DevBuf d_ctr, d_keys, d_vals, d_keys2, d_vals2, d_tmp, d_goff, d_moff, d_mst, d_mlen, d_mgid, d_groups, d_state, d_pop, d_bits, d_plane, d_fwd_off, d_ovf, d_retry, d_retry_off;
   if (!groups.empty()) {
-    auto up = [&](DevBuf& b, const void* src, size_t bytes) -> bool { return b.ensure(bytes ? bytes : 16) && (!bytes || cudaMemcpy(b.p, src, bytes, cudaMemcpyHostToDevice) == cudaSuccess); };
-    if (!up(d_moff, moff.data(), moff.size() * 8) || !up(d_mst, mst.data(), mst.size() * 4) || !up(d_mlen, mlen.data(), mlen.size() * 4) ||
-        !up(d_mgid, mgid.data(), mgid.size() * 4) || !up(d_groups, groups.data(), groups.size() * 4)) { h->err = "device upload failed (merged duplications)"; return XM_ERR_CUDA; }
+    if (!d_moff.upload(moff.data(), moff.size() * 8) || !d_mst.upload(mst.data(), mst.size() * 4) || !d_mlen.upload(mlen.data(), mlen.size() * 4) ||
+        !d_mgid.upload(mgid.data(), mgid.size() * 4) || !d_groups.upload(groups.data(), groups.size() * 4)) { h->err = "device upload failed (merged duplications)"; return XM_ERR_CUDA; }
     // the member CSR: records sorted by group id
     int key_bits = 1; while (key_bits < 32 && (1ll << key_bits) < (long long)n_groups) key_bits++;
     if (!d_keys.ensure((size_t)n_rec * 4) || !d_vals.ensure((size_t)n_rec * 4) || !d_keys2.ensure((size_t)n_rec * 4) || !d_vals2.ensure((size_t)n_rec * 4) ||
         !d_goff.ensure(((size_t)n_groups + 1) * 4)) { h->err = "out of device memory (ancestry groups)"; return XM_ERR_CUDA; }
-    xm_anc_keys_kernel<<<(n_rec + 255) / 256, 256, 0, st>>>((const HostModel::DupGrpRec*)d_recs.p, n_rec, (uint32_t*)d_keys.p, (uint32_t*)d_vals.p);
+    xm_anc_keys_kernel<<<(n_rec + 255) / 256, 256, 0, st>>>((const HostModel::DupGrpRec*)S.d_recs.p, n_rec, (uint32_t*)d_keys.p, (uint32_t*)d_vals.p);
     size_t tb = 0;
     cub::DeviceRadixSort::SortPairs(nullptr, tb, (const uint32_t*)d_keys.p, (uint32_t*)d_keys2.p, (const uint32_t*)d_vals.p, (uint32_t*)d_vals2.p, n_rec, 0, key_bits, st);
     if (!d_tmp.ensure(tb + 16)) { h->err = "out of device memory (ancestry group sort)"; return XM_ERR_CUDA; }
@@ -1638,19 +1613,19 @@ static int infer_ancestors_device(xm_handle* h, double threshold, int min_intere
     const int n_work = 2 * (int)groups.size();
     const size_t bit_words = (size_t)((M.total_fr + 31) / 32);
     if (!d_state.ensure(2 * (size_t)n_rec * sizeof(AncMember)) || !d_pop.ensure((size_t)warps * (size_t)pop_cap) || !d_bits.ensure(bit_words * 4) ||
-        !d_plane.ensure((size_t)M.total_forward) || !up(d_fwd_off, fwd_off.data(), fwd_off.size() * 8) || !d_ovf.ensure((size_t)n_work * 16 + 64)) {
+        !d_plane.ensure((size_t)M.total_forward) || !d_fwd_off.upload(fwd_off.data(), fwd_off.size() * 8) || !d_ovf.ensure((size_t)n_work * 16 + 64) || !d_ctr.ensure(64)) {
       h->err = "out of device memory (ancestry analyses)"; return XM_ERR_CUDA;
     }
     CK(cudaMemsetAsync(d_bits.p, 0, bit_words * 4, st));
     CK(cudaMemsetAsync(d_plane.p, 0xFF, (size_t)M.total_forward, st));
     AncD A;
-    A.ref = h->ref; A.recs = (const HostModel::DupGrpRec*)d_recs.p; A.member = (const uint32_t*)d_vals2.p; A.goff = (const int*)d_goff.p;
+    A.ref = h->ref; A.recs = (const HostModel::DupGrpRec*)S.d_recs.p; A.member = (const uint32_t*)d_vals2.p; A.goff = (const int*)d_goff.p;
     A.moff = (const int64_t*)d_moff.p; A.mst = (const int32_t*)d_mst.p; A.mlen = (const int32_t*)d_mlen.p; A.mgid = (const int32_t*)d_mgid.p;
     A.groups = (const int32_t*)d_groups.p; A.n_work = n_work;
     A.retry_item = nullptr; A.retry_resume = nullptr; A.retry_off = nullptr;
     A.state = (AncMember*)d_state.p; A.n_members = n_rec;
     A.popular = (uint8_t*)d_pop.p; A.pop_cap = pop_cap;
-    int* counters = (int*)d_n.p;   // [0] ticket, [1] overflow count, [2..4] error record
+    int* counters = (int*)d_ctr.p;   // [0] ticket, [1] overflow count, [2..4] error record
     A.ticket = counters; A.ovf_n = counters + 1; A.err = counters + 2;
     A.written = (unsigned int*)d_bits.p; A.plane = (uint8_t*)d_plane.p; A.fwd_off = (const int64_t*)d_fwd_off.p;
     A.ovf_need = (long long*)d_ovf.p; A.ovf_item = (int32_t*)((char*)d_ovf.p + (size_t)n_work * 8); A.ovf_resume = A.ovf_item + n_work;
@@ -1659,11 +1634,11 @@ static int infer_ancestors_device(xm_handle* h, double threshold, int min_intere
     A.mismatch1 = -1 + threshold * 1;           // mismatchScore(1)
     A.leave_bonus = (-3 + threshold * 3) * -1;  // mismatchScore(3) * -1
     A.verify = verify ? 1 : 0;
-    CK(cudaMemsetAsync(d_n.p, 0, 64, st));
+    CK(cudaMemsetAsync(d_ctr.p, 0, 64, st));
     xm_ancestry_kernel<<<blocks, 128, 0, st>>>(A);
     CK(cudaGetLastError());
     int ctr[8] = {0};
-    CK(cudaMemcpyAsync(ctr, d_n.p, 32, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(ctr, d_ctr.p, 32, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     if (ctr[1] > 0) {   // second attempt: the analyses that ran out of scratch, each with the scratch its bounds can need
       const int n_ovf = ctr[1];
@@ -1684,21 +1659,21 @@ static int infer_ancestors_device(xm_handle* h, double threshold, int min_intere
         const int nb = i1 - i0;
         retry.insert(retry.end(), ovf_item.begin() + i0, ovf_item.begin() + i1);
         retry.insert(retry.end(), ovf_resume.begin() + i0, ovf_resume.begin() + i1);
-        if (!up(d_retry, retry.data(), retry.size() * 4) || !up(d_retry_off, off.data(), off.size() * 8) || !d_pop.ensure((size_t)off.back() + 16)) {
+        if (!d_retry.upload(retry.data(), retry.size() * 4) || !d_retry_off.upload(off.data(), off.size() * 8) || !d_pop.ensure((size_t)off.back() + 16)) {
           h->err = "out of device memory (ancestry analyses, second attempt)"; return XM_ERR_CUDA;
         }
         A.retry_item = (const int32_t*)d_retry.p; A.retry_resume = A.retry_item + nb; A.retry_off = (const long long*)d_retry_off.p;
         A.popular = (uint8_t*)d_pop.p; A.n_work = nb;
-        CK(cudaMemsetAsync(d_n.p, 0, 8, st));   // ticket and overflow count; the error record stays
+        CK(cudaMemsetAsync(d_ctr.p, 0, 8, st));   // ticket and overflow count; the error record stays
         xm_ancestry_kernel<<<blocks, 128, 0, st>>>(A);
         CK(cudaGetLastError());
-        CK(cudaMemcpyAsync(ctr, d_n.p, 32, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(ctr, d_ctr.p, 32, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
         if (ctr[1] != 0) { h->err = "xm_infer_ancestors: an analysis outran the scratch its bounds allow (internal error)"; return XM_ERR_STATE; }
         i0 = i1;
       }
     }
-    t_analysis = now();
+    t_analysis = now_s();
     if (ctr[2]) {   // OverriddenSequence.putEncoded :19-27
       const int sid = ctr[3];
       h->err = "Cannot override contig " + std::to_string(sid >> 1) + ((sid & 1) ? "-rev" : "") + "[" + std::to_string(ctr[4]) + "]: already overridden";
@@ -1707,10 +1682,10 @@ static int infer_ancestors_device(xm_handle* h, double threshold, int min_intere
     // e) the forward plane into the packed reference, and back into the handle's reference
     const long long n_words = (long long)M.words.size();
     xm_anc_apply_kernel<<<(unsigned)((n_words + 255) / 256), 256, 0, st>>>((uint16_t*)h->d_words.p, n_words, (const int64_t*)h->d_word_off.p, (const int32_t*)h->d_len.p, M.n_contigs,
-                                                                          (const int64_t*)d_fwd_off.p, (const uint8_t*)d_plane.p, (unsigned long long*)((char*)d_n.p + 32));
+                                                                          (const int64_t*)d_fwd_off.p, (const uint8_t*)d_plane.p, (unsigned long long*)((char*)d_ctr.p + 32));
     CK(cudaGetLastError());
     unsigned long long changed = 0;
-    CK(cudaMemcpyAsync(&changed, (char*)d_n.p + 32, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&changed, (char*)d_ctr.p + 32, 8, cudaMemcpyDeviceToHost, st));
     std::vector<uint16_t> words((size_t)n_words);
     CK(cudaMemcpyAsync(words.data(), h->d_words.p, (size_t)n_words * 2, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
@@ -1718,7 +1693,7 @@ static int infer_ancestors_device(xm_handle* h, double threshold, int min_intere
     *n_changed = (int64_t)changed;
   }
   if (trace) fprintf(stderr, "[xm] infer ancestors: index %.3f s, scan %.3f s (%d members of %d groups), merge %.3f s (%zu groups analysed), analysis %.3f s (%d analyses re-run), apply %.3f s (%lld positions changed)\n",
-                     t_index - t_begin, t_scan - t_index, n_rec, n_groups, t_merge - t_scan, groups.size(), t_analysis - t_merge, n_retried, now() - t_analysis, (long long)*n_changed);
+                     t_index - t_begin, t_scan - t_index, n_rec, n_groups, t_merge - t_scan, groups.size(), t_analysis - t_merge, n_retried, now_s() - t_analysis, (long long)*n_changed);
   return XM_OK;
 }
 
@@ -1781,11 +1756,7 @@ int xm_infer_ancestors(xm_handle* h, double dissimilarity_threshold, int32_t min
   // xm_set_reference; the codes changed only on success (infer_ancestors_device touches HostModel::words last).
   if (rc != XM_OK) *n_changed = 0;
   h->m.reference_codes_changed();
-  for (auto& b : h->d_ix_chunks) b.release();
-  h->d_ix_chunks.clear();
-  for (auto& b : h->d_buckets) b.release();
-  for (auto& b : h->d_positions) b.release();
-  for (auto& b : h->d_positions_hi) b.release();
+  h->d_ix_chunks.clear(); h->d_buckets.clear(); h->d_positions.clear(); h->d_positions_hi.clear();
   return rc;
 }
 int xm_get_reference(xm_handle* h, int32_t contig, uint16_t* packed4) {
@@ -1815,13 +1786,9 @@ static int var_reduce_now(xm_handle* h) {
 }
 static int var_reserve(xm_handle* h, unsigned long long want) {   // keeps recs[0, var_n)
   if (want <= h->var_cap) return XM_OK;
-  unsigned long long ncap = want + want / 2 + 65536;
-  void* np = nullptr;
-  if (cudaMalloc(&np, (size_t)ncap * sizeof(VarRec)) != cudaSuccess) { cudaGetLastError(); h->err = "out of device memory (variant table)"; return XM_ERR_CUDA; }
-  if (h->var_n) cudaMemcpyAsync(np, h->d_var.p, (size_t)h->var_n * sizeof(VarRec), cudaMemcpyDeviceToDevice, h->stream);
-  cudaStreamSynchronize(h->stream);
-  if (h->d_var.p) cudaFree(h->d_var.p);
-  h->d_var.p = np; h->d_var.cap = (size_t)ncap * sizeof(VarRec); h->var_cap = ncap;
+  const unsigned long long ncap = want + want / 2 + 65536;
+  if (!h->d_var.grow((size_t)ncap * sizeof(VarRec), (size_t)h->var_n * sizeof(VarRec), h->stream)) { h->err = "out of device memory (variant table)"; return XM_ERR_CUDA; }
+  h->var_cap = ncap;
   return XM_OK;
 }
 // enqueue: one launch of xm_counts_kernel behind the align kernels; the number of records it wanted to write comes back in *n_after
@@ -2063,12 +2030,10 @@ static int align_batch_impl(xm_handle* h, SlotLease& lease, bool wait_h2d, int32
     unsigned long long used[3];
     CK(cudaMemcpy(used, d_used, 24, cudaMemcpyDeviceToHost));
     auto grow = [&](DevBuf& b, long long& cap, unsigned long long& u, size_t elem) -> bool {
-      unsigned long long keep = u < (unsigned long long)cap ? u : (unsigned long long)cap;
-      long long ncap = (long long)(2 * (u > (unsigned long long)cap ? u : (unsigned long long)cap)) + 4096;
-      void* np = nullptr;
-      if (cudaMalloc(&np, (size_t)ncap * elem) != cudaSuccess) return false;
-      cudaMemcpy(np, b.p, (size_t)keep * elem, cudaMemcpyDeviceToDevice);
-      cudaFree(b.p); b.p = np; b.cap = (size_t)ncap * elem; cap = ncap; u = keep;
+      const unsigned long long keep = std::min(u, (unsigned long long)cap);
+      const long long ncap = (long long)(2 * std::max(u, (unsigned long long)cap)) + 4096;
+      if (!b.grow((size_t)ncap * elem, (size_t)keep * elem, st)) return false;
+      cap = ncap; u = keep;
       return true;
     };
     if (!grow(h->d_choices, h->cap_choices, used[0], sizeof(OutChoice)) || !grow(h->d_sas, h->cap_sas, used[1], sizeof(OutSA)) || !grow(h->d_blocks, h->cap_blocks, used[2], 16)) {

@@ -507,6 +507,13 @@ struct HostModel {
     dup_starts[(size_t)contig].assign(starts, starts + n);
     dup_set = true; dup_generation++;
   }
+  // the duplication table as DupD reads it: the starts of contig c are starts[off[c], off[c + 1]); one trailing 0 keeps `starts`
+  // non-empty when no contig has a duplication
+  void dup_csr(std::vector<int64_t>& off, std::vector<int32_t>& starts) const {
+    off.assign((size_t)n_contigs + 1, 0); starts.clear();
+    for (int c = 0; c < n_contigs; c++) { if ((size_t)c < dup_starts.size()) starts.insert(starts.end(), dup_starts[(size_t)c].begin(), dup_starts[(size_t)c].end()); off[(size_t)c + 1] = (int64_t)starts.size(); }
+    starts.push_back(0);
+  }
 };
 
 // Workspace tiers: bytes of per-query arena. Queries that exhaust a tier are re-run from scratch in the next one

@@ -77,9 +77,8 @@ void* xe_align_batch(void* h, int nq, const uint16_t* packed, const int64_t* seq
   std::vector<TableD> tabs(M.tables.size());
   for (size_t i = 0; i < M.tables.size(); i++) { tabs[i].capacity = M.tables[i].capacity; tabs[i].max_count = M.tables[i].max_count; tabs[i].buckets = M.tables[i].buckets.empty() ? nullptr : M.tables[i].buckets.data(); tabs[i].positions = M.tables[i].positions.data(); tabs[i].positions_hi = M.tables[i].positions_hi.empty() ? nullptr : M.tables[i].positions_hi.data(); }
   IndexD ix; ix.min_interesting = M.min_interesting; ix.max_built = M.max_built; ix.gapmers = M.gapmers; ix.tables = tabs.data();
-  std::vector<int64_t> doff((size_t)M.n_contigs + 1, 0); std::vector<int32_t> dst;
-  for (int c = 0; c < M.n_contigs; c++) { if ((size_t)c < M.dup_starts.size()) dst.insert(dst.end(), M.dup_starts[(size_t)c].begin(), M.dup_starts[(size_t)c].end()); doff[(size_t)c + 1] = (int64_t)dst.size(); }
-  dst.push_back(0);
+  std::vector<int64_t> doff; std::vector<int32_t> dst;
+  M.dup_csr(doff, dst);
   DupD dup; dup.window = M.dup_window; dup.granularity = M.dup_granularity; dup.off = doff.data(); dup.starts = dst.data();
 
   std::vector<int64_t> first((size_t)nq + 1, 0);
