@@ -3,8 +3,8 @@
  * Drop-in boundary: replaces the body of mapper.AlignerWorker.process()/align() in mathjeff/Mapper @ ae7f346a
  * (src/main/java/mapper/AlignerWorker.java:157-261; constructor state :22-33) — a batch of queries in, the
  * List<QueryAlignments> the AlignmentListeners receive (:652-656) out.  Everything left of the boundary
- * (FASTA/FASTQ parsing, options, SAM/VCF/mutations writers) stays the reference's Java host; the binding a
- * maintainer adds (Panama FFM / JNI) is shown in INTEGRATION.md.
+ * (options, file writers) stays the host's: the reference's Java host, whose binding a maintainer adds (Panama FFM / JNI), is shown
+ * in INTEGRATION.md; `python -m mapper_b200` is this project's own host.
  *
  * All pointers are HOST memory unless stated.  Every call returns 0 on success and a negative xm_status on
  * failure; xm_last_error(handle) returns the message (the host throws RuntimeException, matching
@@ -261,6 +261,43 @@ int xm_format_vcf(xm_handle* h, int32_t contig, const char* contig_name, int64_t
  * length); needs no examples. */
 int xm_format_mutations(xm_handle* h, int32_t contig, const char* contig_name, int64_t start, int64_t end, const xm_variant_filter* f,
                         const char** text, int64_t* n_bytes);
+
+/* Read ingestion (the FASTA/FASTQ readers and M/SequenceSplitter.java:9-38 in front of Mapper.compare): text in, the arrays
+ * xm_align_batch takes out.  Parses the complete records at the start of text[0, n_bytes).
+ *   - Records.  FASTA: a '>' header line followed by any number of sequence lines up to the next '>' (any line width; blank lines are
+ *     skipped).  FASTQ: exactly four lines, "@name", the sequence, '+' with anything after it, and a quality line as long as the
+ *     sequence (multi-line FASTQ is not supported).  "\r\n" line ends are accepted.
+ *   - Bases.  The 15 IUPAC letters of QV/Basepairs, in either case, become their 4-bit codes.  Any other byte in a sequence line, a
+ *     quality line of the wrong length, a missing '+' line, a FASTQ record not starting with '@', text before the first FASTA header or
+ *     a FASTQ input ending inside a record returns XM_ERR_ARG; xm_last_error names the record (index within this call) and the byte offset.
+ *   - Names.  The header line after its marker, to the end of the line, without a trailing '\r' (the reference's FastaParser was not
+ *     available to check this choice against).
+ *   - Chunking.  A record is complete when its last line ends in '\n', or when at_eof != 0; a FASTA record only once the next header
+ *     is seen (or at_eof).  *n_consumed = the bytes of the complete records parsed (all n_bytes when at_eof and every record was taken);
+ *     the caller passes the rest again, followed by the next chunk.  At most max_records records are parsed (< 0: no limit): a
+ *     paired-end caller takes the same number of records from both files.
+ *   - Splitting.  split_size > 0: a record longer than split_size becomes n = (len - 1) / split_size + 1 sequences, piece k covering
+ *     [len*k/n, len*(k+1)/n) and named "name[start:end]" (SURVEY.md §5; unchecked against the reference's splitter).  XM_R_RECORD maps
+ *     every sequence back to its record.
+ * The text goes to the device through a pinned staging buffer; line ends (one ballot per warp over the bytes, then a scan), record
+ * bounds, lengths, the split, word offsets, packing, names and the checks run there (kernels xm_parse_*, on a stream of their own, so a
+ * call overlaps an xm_align_batch on the same handle); the arrays come back in one copy into a pinned slab owned by the xm_reads.
+ * n_bytes < 2^31 per call. */
+enum xm_text_format { XM_FASTA = 0, XM_FASTQ = 1 };
+typedef struct xm_reads xm_reads;
+int xm_parse_reads(xm_handle* h, int32_t format, const char* text, int64_t n_bytes, int32_t at_eof,
+                   int64_t max_records, int32_t split_size, xm_reads** out, int64_t* n_consumed);
+enum xm_reads_array {
+  XM_R_PACKED = 0,        /* uint16: packed4, the layout xm_align_batch takes */
+  XM_R_SEQ_WORD_OFF = 1,  /* int64, n + 1 */
+  XM_R_SEQ_LEN = 2,       /* int32 */
+  XM_R_NAME_OFF = 3,      /* int64, n + 1, into XM_R_NAMES */
+  XM_R_NAMES = 4,         /* char */
+  XM_R_RECORD = 5         /* int64: index within this call of the record a sequence came from */
+};
+/* Element count of array `which` of r (n = number of sequences), *ptr = its first element; valid until xm_release_reads(r). */
+int64_t xm_reads_array(const xm_reads* r, int which, const void** ptr);
+void xm_release_reads(xm_reads* r);
 
 /* Measurement aid (bench.py's roofline): sustained issue rates of this GPU, in warp-instructions per second over the whole chip,
  * from three micro-benchmark kernels timed with CUDA events - out[0] INT32 (IMAD chains), out[1] FP64 (DADD chains), out[2] FP32

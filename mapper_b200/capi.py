@@ -17,11 +17,15 @@ EXPORTS = ["xm_create", "xm_destroy", "xm_last_error", "xm_set_reference", "xm_s
            "xm_get_duplications", "xm_infer_ancestors", "xm_get_reference", "xm_align_batch", "xm_align_batch_device", "xm_results_array", "xm_release_results",
            "xm_counts_enable", "xm_counts_device_ptr", "xm_counts_fetch", "xm_format_sam",
            "xm_comm_unique_id", "xm_comm_init", "xm_counts_reduce", "xm_counts_batch_info", "xm_variants_fetch", "xm_measure_peaks", "xm_counts_reduce_times",
-           "xm_variants_examples", "xm_variants_set_examples", "xm_format_vcf", "xm_format_mutations"]
+           "xm_variants_examples", "xm_variants_set_examples", "xm_format_vcf", "xm_format_mutations",
+           "xm_parse_reads", "xm_reads_array", "xm_release_reads"]
 
 RESULT_ARRAYS = [("q_comp_off", np.int64), ("comp_choice_off", np.int64), ("choice_sa_off", np.int64), ("sa_block_off", np.int64),
                  ("choice_f64", np.float64), ("sa_f64", np.float64), ("choice_inner", np.int32), ("sa_contig", np.int32),
                  ("blocks", np.int32), ("q_status", np.int32), ("sa_reversed", np.uint8), ("stats", np.int64), ("q_cycles", np.int64)]
+READS_ARRAYS = [("packed", np.uint16), ("seq_word_off", np.int64), ("seq_len", np.int32), ("name_off", np.int64), ("names", np.uint8),
+                ("record", np.int64)]
+FASTA, FASTQ = 0, 1
 STAT = dict(kernel_ns=0, launches=1, tier0=2, tier1=3, tier2=4, probes=5, seeds=6, hits=7, straight=8, path_calls=9,
             path_steps=10, path_cells=11, h2d_bytes=12, d2h_bytes=13, align_kernel_ns=14, tier0_ns=15, tier1_ns=16, tier2_ns=17,
             cyc_seed=18, cyc_straight=19, cyc_hba=20, cyc_path=21, cyc_tables=22, cyc_spare=23, cyc_total=24, easy=25, easy_ns=26, easy_done=27, easy_probes=28, easy_hits=29, easy_straight=30)
@@ -69,6 +73,7 @@ def load_library():
         L = C.CDLL(LIB_PATH)
         L.xm_last_error.restype = C.c_char_p
         L.xm_results_array.restype = C.c_int64
+        L.xm_reads_array.restype = C.c_int64
         _LIB = L
     return _LIB
 
@@ -95,6 +100,10 @@ class XmError(RuntimeError):
 
 def _ptr(a):
     return a.ctypes.data_as(C.c_void_p)
+
+
+def _bytes(s):
+    return s if isinstance(s, bytes) else s.encode()
 
 
 class _ResultOwner:
@@ -268,7 +277,10 @@ class XMapper:
         return out, sam
 
     def format_sam(self, r, seq_names, contig_names):
+        """seq_names / contig_names: lists of str, or (bytes, int64 offsets) pairs as parse_reads_raw returns them."""
         def blob(names):
+            if isinstance(names, tuple):
+                return bytes(names[0]) + b"\0", np.ascontiguousarray(names[1], dtype=np.int64)
             enc = [n.encode() for n in names]
             off = np.zeros(len(enc) + 1, dtype=np.int64)
             if enc:
@@ -287,6 +299,37 @@ class XMapper:
                                           C.c_void_p(d_n_seqs), C.c_void_p(d_expected), C.c_void_p(d_per), int(max_seq_len), C.byref(r))
         self._ok(rc, allow=() if strict else (-4,))
         return self._take(r, copy)
+
+    # ---- read ingestion ----
+    def parse_reads_raw(self, text, fmt, split_size=0, at_eof=True, max_records=-1):
+        """xm_parse_reads over bytes `text` (fmt: FASTA or FASTQ): (dict of the arrays of enum xm_reads_array, copied; "names" is
+        bytes), n_consumed."""
+        r, n_consumed = C.c_void_p(), C.c_int64()
+        self._ok(self.L.xm_parse_reads(self.h, int(fmt), text, C.c_int64(len(text)), int(bool(at_eof)), C.c_int64(max_records), int(split_size),
+                                       C.byref(r), C.byref(n_consumed)))
+        out = {}
+        try:
+            for i, (name, dt) in enumerate(READS_ARRAYS):
+                ptr = C.c_void_p()
+                n = self.L.xm_reads_array(r, i, C.byref(ptr))
+                nb = n * np.dtype(dt).itemsize
+                out[name] = np.ctypeslib.as_array(C.cast(ptr, C.POINTER(C.c_uint8)), shape=(nb,)).view(dt).copy() if nb else np.zeros(0, dtype=dt)
+        finally:
+            self.L.xm_release_reads(r)
+        out["names"] = out["names"].tobytes()
+        return out, n_consumed.value
+
+    def parse_reads(self, text, fmt, split_size=0, at_eof=True, max_records=-1):
+        """FASTA / FASTQ text parsed on the device.  Returns (batch of single-sequence queries in the shape align_batch takes, names as a
+        list of str, record index per sequence, n_consumed)."""
+        a, n_consumed = self.parse_reads_raw(text, fmt, split_size, at_eof, max_records)
+        n = len(a["seq_len"])
+        packed = a["packed"] if len(a["packed"]) else np.zeros(1, dtype=np.uint16)
+        batch = dict(packed=packed, seq_word_off=a["seq_word_off"], seq_len=a["seq_len"], n_seqs=np.ones(n, dtype=np.uint8),
+                     expected_inner=np.zeros(n, dtype=np.float64), per_penalty=np.ones(n, dtype=np.float64))
+        off, blob = a["name_off"], a["names"]
+        names = [blob[off[i]:off[i + 1]].decode("utf-8", "surrogateescape") for i in range(n)]
+        return batch, names, a["record"], n_consumed
 
     # ---- per-position counts ----
     def counts_enable(self, query_end_fraction=0.1):
@@ -371,14 +414,20 @@ class XMapper:
         off = np.zeros(len(gids) + 1, dtype=np.int64)
         if len(gids):
             off[1:] = np.cumsum([len(p) for p in packed])
-        words = np.concatenate(packed + [np.zeros(1, dtype=np.uint16)])
-        self._ok(self.L.xm_variants_set_examples(self.h, C.c_int64(len(gids)), _ptr(np.ascontiguousarray(gids)), _ptr(words), _ptr(off), _ptr(lens)))
+        self.upload_variant_examples(gids, np.concatenate(packed + [np.zeros(0, dtype=np.uint16)]), off, lens)
+
+    def upload_variant_examples(self, gids, packed, seq_word_off, seq_len):
+        """xm_variants_set_examples with the reads already packed (gids as variants_examples() lists them)."""
+        words = np.concatenate([np.asarray(packed, dtype=np.uint16), np.zeros(1, dtype=np.uint16)])
+        self._ok(self.L.xm_variants_set_examples(self.h, C.c_int64(len(gids)), _ptr(np.ascontiguousarray(gids, dtype=np.int64)), _ptr(words),
+                                                 _ptr(np.ascontiguousarray(seq_word_off, dtype=np.int64)), _ptr(np.ascontiguousarray(seq_len, dtype=np.int32))))
 
     def format_vcf(self, contig, name, start, end, flt=None, include_non_mutations=True, show_support=True):
-        """VCF body lines of positions [start, end) of contig `contig`; flt: dict of MutationDetectionParameters thresholds or None."""
+        """VCF body lines of positions [start, end) of contig `contig` named `name` (str or bytes); flt: dict of MutationDetectionParameters
+        thresholds or None."""
         f = to_xm_filter(flt)
         text, n = C.c_char_p(), C.c_int64()
-        self._ok(self.L.xm_format_vcf(self.h, int(contig), name.encode(), C.c_int64(start), C.c_int64(end), C.byref(f), int(bool(include_non_mutations)),
+        self._ok(self.L.xm_format_vcf(self.h, int(contig), _bytes(name), C.c_int64(start), C.c_int64(end), C.byref(f), int(bool(include_non_mutations)),
                                       int(bool(show_support)), C.byref(text), C.byref(n)))
         return C.string_at(text, n.value).decode()
 
@@ -386,5 +435,5 @@ class XMapper:
         """Mutations body lines of [start, end) of contig `contig` (start and end on the 8192 grid, or end = the contig length)."""
         f = to_xm_filter(flt)
         text, n = C.c_char_p(), C.c_int64()
-        self._ok(self.L.xm_format_mutations(self.h, int(contig), name.encode(), C.c_int64(start), C.c_int64(end), C.byref(f), C.byref(text), C.byref(n)))
+        self._ok(self.L.xm_format_mutations(self.h, int(contig), _bytes(name), C.c_int64(start), C.c_int64(end), C.byref(f), C.byref(text), C.byref(n)))
         return C.string_at(text, n.value).decode()

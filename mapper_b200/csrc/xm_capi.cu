@@ -677,6 +677,7 @@ struct DevBuf {
 
 #include "xm_counts.cuh"
 #include "xm_variants_fmt.cuh"
+#include "xm_parse.cuh"
 
 // pinned host slabs for results, recycled between batches (cudaHostAlloc of 100 MB costs tens of ms)
 struct PinnedPool {
@@ -708,6 +709,12 @@ struct xm_results {
   void* sam = nullptr; size_t sam_cap = 0;   // pinned text of the latest xm_format_sam (from the same pool as the slab)
   std::shared_ptr<PinnedPool> pool; void* slab = nullptr; size_t slab_cap = 0;
   ~xm_results() { if (slab && pool) pool->give(slab, slab_cap); if (sam && pool) pool->give(sam, sam_cap); }
+};
+// the arrays of one xm_parse_reads call (enum xm_reads_array), views into one pinned slab
+struct xm_reads {
+  std::shared_ptr<PinnedPool> pool; void* slab = nullptr; size_t slab_cap = 0;
+  int64_t off[6] = {0, 0, 0, 0, 0, 0}, n[6] = {0, 0, 0, 0, 0, 0};
+  ~xm_reads() { if (slab && pool) pool->give(slab, slab_cap); }
 };
 
 // ---- NCCL, loaded at run time (the host process may already carry its own libnccl; no link-time dependency) ----
@@ -797,6 +804,11 @@ struct xm_handle {
   DevBuf d_ex_words, d_ex_word_off, d_ex_len, d_ex_gids, d_ex_slot, d_ex_bad;
   DevBuf d_fmt_dec, d_fmt_state, d_fmt_len, d_fmt_range, d_fmt_name, d_fmt_text, d_fmt_tmp, d_fmt_ids;
   void* fmt_text = nullptr; size_t fmt_cap = 0;   // pinned text of the latest xm_format_vcf / xm_format_mutations
+  // read parsing (xm_parse.cuh): its own lock, stream and buffers, so that parsing the next chunk overlaps the batch being aligned
+  std::mutex parse_mu; cudaStream_t parse_stream = nullptr;
+  DevBuf d_pz_text, d_pz_tiles, d_pz_line_end, d_pz_flag, d_pz_line_rec, d_pz_rec_line, d_pz_bases, d_pz_lbase, d_pz_pieces, d_pz_piece_off;
+  DevBuf d_pz_start, d_pz_len, d_pz_rec, d_pz_words, d_pz_name_len, d_pz_word_off, d_pz_name_off, d_pz_slab, d_pz_tmp, d_pz_misc;
+  void* pz_stage = nullptr; size_t pz_stage_cap = 0;   // pinned staging of the text
   ncclComm_t comm = nullptr; int comm_ranks = 0, comm_rank = 0;
   double last_planes_ms = 0, last_variants_ms = 0;   // xm_counts_reduce: device time of the plane all-reduce, wall time of the variant-table exchange   // xm_comm_init: the communicator xm_counts_reduce uses
 };
@@ -1228,6 +1240,17 @@ __global__ void xm_anc_goff_kernel(const uint32_t* keys, int n, int n_groups, in
   for (int g = (i == 0 ? 0 : (int)keys[i - 1] + 1); g <= k; g++) goff[g] = i;
   if (i == n - 1) for (int g = k + 1; g <= n_groups; g++) goff[g] = n;
 }
+// xm_parse_reads: scans on the parser's stream, with its own scratch
+template <class In, class Out>
+static cudaError_t pz_scan(xm_handle* h, const In* in, Out* out, int n, bool inclusive) {
+  cudaStream_t st = h->parse_stream;
+  size_t tb = 0;
+  if (inclusive) cub::DeviceScan::InclusiveSum(nullptr, tb, in, out, n, st); else cub::DeviceScan::ExclusiveSum(nullptr, tb, in, out, n, st);
+  if (!h->d_pz_tmp.ensure(tb + 16)) return cudaErrorMemoryAllocation;
+  return inclusive ? cub::DeviceScan::InclusiveSum(h->d_pz_tmp.p, tb, in, out, n, st) : cub::DeviceScan::ExclusiveSum(h->d_pz_tmp.p, tb, in, out, n, st);
+}
+static unsigned pz_blocks(long long n, int threads) { return (unsigned)((n + threads - 1) / threads); }
+
 extern "C" {
 
 int xm_create(const xm_params* p, int device, xm_handle** out) {
@@ -1244,7 +1267,7 @@ int xm_create(const xm_params* p, int device, xm_handle** out) {
   cudaGetDeviceProperties(&prop, device);
   h->sm_count = prop.multiProcessorCount;
   { int nb = 0; if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, xm_align_kernel<true>, XM_BLOCK, 0) == cudaSuccess && nb > 0) h->blocks_per_sm = nb; }
-  if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess ||
+  if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess || cudaStreamCreateWithFlags(&h->parse_stream, cudaStreamNonBlocking) != cudaSuccess ||
       cudaEventCreate(&h->ev2) != cudaSuccess || cudaEventCreate(&h->ev3) != cudaSuccess || cudaEventCreate(&h->ev4) != cudaSuccess || cudaEventCreate(&h->ev5) != cudaSuccess) {
     fprintf(stderr, "xmapper_b200: stream/event creation failed: %s\n", cudaGetErrorString(cudaGetLastError()));
     xm_destroy(h); return XM_ERR_CUDA;
@@ -1292,7 +1315,9 @@ void xm_destroy(xm_handle* h) {
     for (cudaEvent_t e : {sl.h2d_done, sl.kernels_done, sl.ev0, sl.ev1}) if (e) cudaEventDestroy(e);
   }
   if (h->fmt_text) h->pinned->give(h->fmt_text, h->fmt_cap);
+  if (h->pz_stage) h->pinned->give(h->pz_stage, h->pz_stage_cap);
   if (h->stream) cudaStreamDestroy(h->stream);
+  if (h->parse_stream) cudaStreamDestroy(h->parse_stream);
   for (cudaEvent_t e : {h->ev2, h->ev3, h->ev4, h->ev5}) if (e) cudaEventDestroy(e);
   delete h;
 }
@@ -2519,6 +2544,179 @@ int xm_format_mutations(xm_handle* h, int32_t contig, const char* contig_name, i
                         const char** text, int64_t* n_bytes) {
   return format_variants(h, XM_FMT_MUT, contig, contig_name, start, end, f, 0, 0, text, n_bytes);
 }
+
+int xm_parse_reads(xm_handle* h, int32_t format, const char* text, int64_t n_bytes, int32_t at_eof, int64_t max_records, int32_t split_size,
+                   xm_reads** out, int64_t* n_consumed) {
+  if (out) *out = nullptr;
+  if (n_consumed) *n_consumed = 0;
+  if (!h || !out || !n_consumed || (format != XM_FASTA && format != XM_FASTQ) || n_bytes < 0 || (n_bytes > 0 && !text) || split_size < 0) return XM_ERR_ARG;
+  if (n_bytes >= (1ll << 31)) { h->err = "xm_parse_reads: pass fewer than 2^31 bytes per call"; return XM_ERR_ARG; }
+  std::lock_guard<std::mutex> parse(h->parse_mu);
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = h->parse_stream;
+  const bool fastq = format == XM_FASTQ;
+  const long long n = n_bytes;
+  const char* fmt_name = fastq ? "FASTQ" : "FASTA";
+  // the text goes up through the pinned staging buffer
+  if (h->pz_stage && h->pz_stage_cap < (size_t)n + 1) { h->pinned->give(h->pz_stage, h->pz_stage_cap); h->pz_stage = nullptr; }
+  if (!h->pz_stage) h->pz_stage = h->pinned->take((size_t)n + 1, h->pz_stage_cap);
+  if (!h->pz_stage) { h->err = "out of pinned host memory (xm_parse_reads)"; return XM_ERR_CUDA; }
+  if (n) memcpy(h->pz_stage, text, (size_t)n);
+  const int n_tiles = (int)std::max<long long>(1, (n + PZ_TILE - 1) / PZ_TILE);
+  if (!h->d_pz_text.ensure((size_t)n + 16) || !h->d_pz_tiles.ensure(((size_t)n_tiles + 1) * 8) || !h->d_pz_misc.ensure(64)) { h->err = "out of device memory (xm_parse_reads)"; return XM_ERR_CUDA; }
+  const char* d_text = (const char*)h->d_pz_text.p;
+  unsigned int* tile_cnt = (unsigned int*)h->d_pz_tiles.p;
+  unsigned int* tile_off = tile_cnt + n_tiles + 1;
+  PzErr* d_err = (PzErr*)h->d_pz_misc.p;
+  int* d_count = (int*)((char*)h->d_pz_misc.p + 32);
+  if (n) CK(cudaMemcpyAsync(h->d_pz_text.p, h->pz_stage, (size_t)n, cudaMemcpyHostToDevice, st));
+  CK(cudaMemsetAsync(d_err, 0xff, sizeof(PzErr), st));
+  // line ends
+  xm_parse_nl_kernel<false><<<n_tiles, PZ_THREADS, 0, st>>>(d_text, n, tile_cnt, nullptr, nullptr);
+  CK(cudaMemsetAsync(tile_cnt + n_tiles, 0, 4, st));
+  CK(pz_scan(h, tile_cnt, tile_off, n_tiles + 1, false));
+  unsigned int n_nl = 0;
+  CK(cudaMemcpyAsync(&n_nl, tile_off + n_tiles, 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  const bool tail = at_eof && n > 0 && text[n - 1] != '\n';   // the last line of the input needs no '\n'
+  const int n_lines = (int)n_nl + (tail ? 1 : 0);
+  const long long text_end = n;
+  if (!h->d_pz_line_end.ensure(((size_t)n_lines + 1) * 8)) { h->err = "out of device memory (xm_parse_reads)"; return XM_ERR_CUDA; }
+  long long* line_end = (long long*)h->d_pz_line_end.p;
+  xm_parse_nl_kernel<true><<<n_tiles, PZ_THREADS, 0, st>>>(d_text, n, tile_cnt, tile_off, line_end);
+  if (tail) CK(cudaMemcpyAsync(line_end + n_nl, &text_end, 8, cudaMemcpyHostToDevice, st));
+  ParseD P;
+  P.text = d_text; P.n = n; P.fastq = fastq ? 1 : 0; P.split = split_size; P.line_end = line_end; P.n_lines = n_lines;
+  P.rec_line = nullptr; P.line_rec = nullptr; P.lbase = nullptr; P.err = d_err;
+  // records: complete ones only, at most max_records
+  long long n_rec = 0, n_avail = 0;
+  int lines_end = 0;
+  if (fastq) {
+    n_avail = n_lines / 4;
+    n_rec = max_records >= 0 ? std::min<long long>(n_avail, max_records) : n_avail;
+    lines_end = (int)(4 * n_rec);
+  } else {
+    if (!h->d_pz_flag.ensure(((size_t)n_lines + 1) * 4) || !h->d_pz_line_rec.ensure(((size_t)n_lines + 1) * 4) || !h->d_pz_rec_line.ensure(((size_t)n_lines + 2) * 4)) {
+      h->err = "out of device memory (xm_parse_reads)"; return XM_ERR_CUDA;
+    }
+    int* flag = (int*)h->d_pz_flag.p;
+    int* rec_line = (int*)h->d_pz_rec_line.p;
+    int n_hdr = 0;
+    if (n_lines) {
+      xm_parse_class_kernel<<<pz_blocks(n_lines, 256), 256, 0, st>>>(P, flag);
+      CK(pz_scan(h, flag, (int*)h->d_pz_line_rec.p, n_lines, true));
+      size_t tb = 0;
+      cub::DeviceSelect::Flagged(nullptr, tb, cub::CountingInputIterator<int>(0), flag, rec_line, d_count, n_lines, st);
+      if (!h->d_pz_tmp.ensure(tb + 16)) { h->err = "out of device memory (xm_parse_reads)"; return XM_ERR_CUDA; }
+      CK(cub::DeviceSelect::Flagged(h->d_pz_tmp.p, tb, cub::CountingInputIterator<int>(0), flag, rec_line, d_count, n_lines, st));
+      CK(cudaMemcpyAsync(&n_hdr, d_count, 4, cudaMemcpyDeviceToHost, st));
+      CK(cudaStreamSynchronize(st));
+    }
+    n_avail = at_eof ? n_hdr : std::max(n_hdr - 1, 0);   // without the end of the input, a record is complete when the next header is seen
+    n_rec = max_records >= 0 ? std::min<long long>(n_avail, max_records) : n_avail;
+    lines_end = n_lines;
+    if (n_rec < n_hdr) { CK(cudaMemcpyAsync(&lines_end, rec_line + n_rec, 4, cudaMemcpyDeviceToHost, st)); CK(cudaStreamSynchronize(st)); }
+    else CK(cudaMemcpyAsync(rec_line + n_rec, &lines_end, 4, cudaMemcpyHostToDevice, st));
+    P.rec_line = rec_line; P.line_rec = (const int*)h->d_pz_line_rec.p;
+  }
+  P.n_rec = (int)n_rec; P.lines_end = lines_end;
+  // bytes taken: through the end of the last parsed record, or all of it when the input ends after it
+  const bool all = at_eof && (fastq ? n_rec == n_avail : lines_end == n_lines);
+  long long consumed = 0, tail_start = 0;
+  if (lines_end > 0) { CK(cudaMemcpyAsync(&tail_start, line_end + lines_end - 1, 8, cudaMemcpyDeviceToHost, st)); CK(cudaStreamSynchronize(st)); tail_start++; }
+  consumed = all ? n : tail_start;
+  // per line bases and checks, per record pieces
+  if (!h->d_pz_bases.ensure(((size_t)lines_end + 1) * 8) || !h->d_pz_lbase.ensure(((size_t)lines_end + 1) * 8) ||
+      !h->d_pz_pieces.ensure(((size_t)n_rec + 1) * 8) || !h->d_pz_piece_off.ensure(((size_t)n_rec + 1) * 8)) { h->err = "out of device memory (xm_parse_reads)"; return XM_ERR_CUDA; }
+  xm_parse_lines_kernel<<<pz_blocks(lines_end + 1, 256), 256, 0, st>>>(P, (long long*)h->d_pz_bases.p);
+  CK(pz_scan(h, (const long long*)h->d_pz_bases.p, (long long*)h->d_pz_lbase.p, lines_end + 1, false));
+  P.lbase = (const long long*)h->d_pz_lbase.p;
+  xm_parse_rec_kernel<<<pz_blocks(n_rec + 1, 256), 256, 0, st>>>(P, (long long*)h->d_pz_pieces.p);
+  CK(pz_scan(h, (const long long*)h->d_pz_pieces.p, (long long*)h->d_pz_piece_off.p, (int)n_rec + 1, false));
+  long long n_seq = 0;
+  PzErr e;
+  CK(cudaMemcpyAsync(&n_seq, (const long long*)h->d_pz_piece_off.p + n_rec, 8, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(&e, d_err, sizeof(PzErr), cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  CK(cudaGetLastError());
+  auto fail = [&](const PzErr& x) {
+    const long long off = (long long)(x.key >> 3), line = (long long)x.line;
+    const int kind = (int)(x.key & 7);
+    long long rec = line / 4;
+    if (!fastq) { int lr = 0; if (cudaMemcpy(&lr, P.line_rec + line, 4, cudaMemcpyDeviceToHost) != cudaSuccess) cudaGetLastError(); rec = lr - 1; }
+    std::string what;
+    switch (kind) {
+      case PZ_BAD_BASE: { char b[64]; snprintf(b, sizeof b, "byte 0x%02x ('%c') is not an IUPAC base letter", (unsigned char)text[off], text[off] >= 32 && text[off] < 127 ? text[off] : '?'); what = b; break; }
+      case PZ_BAD_MARKER: what = "a FASTQ record must start with a '@' line"; break;
+      case PZ_NO_PLUS: what = "missing '+' line (multi-line FASTQ is not supported)"; break;
+      case PZ_QUAL_LEN: what = "the quality line is not as long as the sequence line"; break;
+      case PZ_BEFORE_HEADER: what = "text before the first '>' header"; break;
+    }
+    h->err = std::string("xm_parse_reads: ") + fmt_name + " record " + std::to_string(rec) + ", byte offset " + std::to_string(off) + ": " + what;
+    return XM_ERR_ARG;
+  };
+  if (e.key != ~0ull) return fail(e);
+  if (fastq && all) {   // only blank lines may follow the last complete record
+    for (long long i = tail_start; i < n; i++) if (text[i] != '\n' && text[i] != '\r') {
+      h->err = "xm_parse_reads: FASTQ record " + std::to_string(n_rec) + ", byte offset " + std::to_string(tail_start) + ": the input ends inside the record (a record is four lines)";
+      return XM_ERR_ARG;
+    }
+  }
+  if (n_seq >= (1ll << 31)) { h->err = "xm_parse_reads: more than 2^31 - 1 sequences in one call"; return XM_ERR_ARG; }
+  // pieces, word and name offsets
+  const size_t ns1 = (size_t)n_seq + 1;
+  if (!h->d_pz_start.ensure(ns1 * 8) || !h->d_pz_len.ensure(ns1 * 4) || !h->d_pz_rec.ensure(ns1 * 8) || !h->d_pz_words.ensure(ns1 * 8) ||
+      !h->d_pz_name_len.ensure(ns1 * 8) || !h->d_pz_word_off.ensure(ns1 * 8) || !h->d_pz_name_off.ensure(ns1 * 8)) { h->err = "out of device memory (xm_parse_reads)"; return XM_ERR_CUDA; }
+  PieceD Q;
+  Q.piece_off = (const long long*)h->d_pz_piece_off.p; Q.start = (long long*)h->d_pz_start.p; Q.len = (int32_t*)h->d_pz_len.p; Q.rec = (int64_t*)h->d_pz_rec.p;
+  Q.words = (long long*)h->d_pz_words.p; Q.name_len = (long long*)h->d_pz_name_len.p;
+  if (n_rec) xm_parse_piece_kernel<<<pz_blocks(n_rec, 128), 128, 0, st>>>(P, Q);
+  CK(cudaMemsetAsync(Q.words + n_seq, 0, 8, st));
+  CK(cudaMemsetAsync(Q.name_len + n_seq, 0, 8, st));
+  CK(pz_scan(h, (const long long*)Q.words, (long long*)h->d_pz_word_off.p, (int)ns1, false));
+  CK(pz_scan(h, (const long long*)Q.name_len, (long long*)h->d_pz_name_off.p, (int)ns1, false));
+  long long tot[2] = {0, 0};
+  CK(cudaMemcpyAsync(&tot[0], (const long long*)h->d_pz_word_off.p + n_seq, 8, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(&tot[1], (const long long*)h->d_pz_name_off.p + n_seq, 8, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  // one device slab in the layout of the host slab: packed, seq_word_off, seq_len, name_off, names, record
+  std::unique_ptr<xm_reads> R(new xm_reads());
+  const int64_t counts[6] = {tot[0], (int64_t)ns1, n_seq, (int64_t)ns1, tot[1], n_seq};
+  const int64_t widths[6] = {2, 8, 4, 8, 1, 8};
+  size_t bytes = 0;
+  for (int k = 0; k < 6; k++) { R->off[k] = (int64_t)bytes; R->n[k] = counts[k]; bytes += ((size_t)(counts[k] * widths[k]) + 15) & ~(size_t)15; }
+  if (!h->d_pz_slab.ensure(bytes + 16)) { h->err = "out of device memory (xm_parse_reads)"; return XM_ERR_CUDA; }
+  char* ds = (char*)h->d_pz_slab.p;
+  CK(cudaMemcpyAsync(ds + R->off[1], h->d_pz_word_off.p, ns1 * 8, cudaMemcpyDeviceToDevice, st));
+  CK(cudaMemcpyAsync(ds + R->off[2], h->d_pz_len.p, (size_t)n_seq * 4, cudaMemcpyDeviceToDevice, st));
+  CK(cudaMemcpyAsync(ds + R->off[3], h->d_pz_name_off.p, ns1 * 8, cudaMemcpyDeviceToDevice, st));
+  CK(cudaMemcpyAsync(ds + R->off[5], h->d_pz_rec.p, (size_t)n_seq * 8, cudaMemcpyDeviceToDevice, st));
+  PackD K;
+  K.start = Q.start; K.len = Q.len; K.rec = Q.rec; K.word_off = (const int64_t*)h->d_pz_word_off.p; K.name_off = (const int64_t*)h->d_pz_name_off.p;
+  K.packed = (uint16_t*)(ds + R->off[0]); K.names = ds + R->off[4]; K.n_seq = n_seq;
+  if (n_seq) {
+    xm_parse_pack_kernel<<<pz_blocks(n_seq * 32, 256), 256, 0, st>>>(P, K);
+    xm_parse_names_kernel<<<pz_blocks(n_seq * 32, 256), 256, 0, st>>>(P, K);
+  }
+  CK(cudaGetLastError());
+  R->pool = h->pinned;
+  R->slab = h->pinned->take(bytes + 16, R->slab_cap);
+  if (!R->slab) { h->err = "out of pinned host memory (xm_parse_reads)"; return XM_ERR_CUDA; }
+  CK(cudaMemcpyAsync(R->slab, ds, bytes, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(&e, d_err, sizeof(PzErr), cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  CK(cudaGetLastError());
+  if (e.key != ~0ull) return fail(e);
+  *n_consumed = consumed;
+  *out = R.release();
+  return XM_OK;
+}
+int64_t xm_reads_array(const xm_reads* r, int which, const void** ptr) {
+  if (!r || !ptr || which < 0 || which > XM_R_RECORD) return -1;
+  *ptr = (const char*)r->slab + r->off[which];
+  return r->n[which];
+}
+void xm_release_reads(xm_reads* r) { delete r; }
 
 // out[0] INT32 IMAD, out[1] FP64 DADD, out[2] FP32 FFMA (full-rate pipe = the dispatch ceiling): sustained warp-instructions per second over the whole chip (the loop
 // bodies are 128 arithmetic instructions per iteration per warp; loop overhead is below 2 %); out[3] = SM count, out[4] = SM clock in Hz
