@@ -299,6 +299,16 @@ enum xm_reads_array {
 int64_t xm_reads_array(const xm_reads* r, int which, const void** ptr);
 void xm_release_reads(xm_reads* r);
 
+/* Ranks n names by unsigned byte order, a proper prefix first (String.compareTo for ASCII names): ranks[i] = the number of distinct
+ * names smaller than name i; equal names get equal ranks.  This is the name order DirectionalAlignments.betterExample breaks example
+ * ties with, the order keys xm_counts_batch_info takes.  names / name_off as xm_parse_reads returns them (name_off: n + 1 entries,
+ * non-decreasing, name_off[0] == 0).  Runs on the device of h, on its stream (kernels xm_rank_*, mapper_b200/csrc/xm_names.cuh): each
+ * round sorts the names still tied by their next 7 bytes and splits the ties, so a call takes one round per 7 bytes of the longest
+ * prefix that two distinct names share (two 64-bit-key radix sorts over the names still tied, each round), plus one.  The device
+ * scratch (about 100 bytes per name plus the names) is freed before the call returns.  n < 2^31; bad offsets or a larger n return
+ * XM_ERR_ARG. */
+int xm_rank_names(xm_handle* h, int64_t n, const char* names, const int64_t* name_off, int64_t* ranks);
+
 /* Measurement aid (bench.py's roofline): sustained issue rates of this GPU, in warp-instructions per second over the whole chip,
  * from three micro-benchmark kernels timed with CUDA events - out[0] INT32 (IMAD chains), out[1] FP64 (DADD chains), out[2] FP32
  * FFMA chains (full-rate pipe: the issue-slot ceiling); out[3] = number of SMs, out[4] = maximum SM clock in Hz.  SURVEY.md §8(d) takes the relevant

@@ -1,27 +1,33 @@
-"""python -m mapper_b200: map FASTA/FASTQ reads against a FASTA reference on one GPU and write SAM, VCF and mutations files.
+"""python -m mapper_b200: map FASTA/FASTQ reads against a FASTA reference on one or more GPUs and write SAM, VCF and mutations files.
 
-The front end of X-Mapper's Mapper.run (SURVEY.md §3.1), driving the C ABI; it holds no algorithm.
-  1. Reference: parsed on the device (xm_parse_reads), contigs sorted as Mapper.sortAndComplementReference sorts them (descending
-     length, ties in input order), xm_set_reference, optionally xm_infer_ancestors (--infer-ancestors, set up as M/Mapper.java:666-692),
-     xm_build_index(longest query or split piece) and xm_build_duplications(-1, -1, 2, 1000).
+The front end of X-Mapper's Mapper.run (SURVEY.md §3.1), driving the C ABI; it holds no algorithm.  --device takes one CUDA ordinal or a
+comma list of them: one handle per device, every handle holding the same reference, index and duplication table.
+  1. Reference: parsed on the first device (xm_parse_reads), contigs sorted as Mapper.sortAndComplementReference sorts them (descending
+     length, ties in input order) and given to every handle (xm_set_reference).  --infer-ancestors (set up as M/Mapper.java:666-692) runs
+     on the first device, whose "-anc" contigs go to the others (xm_get_reference -> xm_set_reference).  xm_build_index(longest query or
+     split piece) and xm_build_duplications(-1, -1, 2, 1000) run on all devices at once.
   2. A pre-pass over the queries: the longest sequence for the index and, when counts are written, the rank of every sequence name in
-     byte order (String.compareTo for ASCII names), the name order DirectionalAlignments.betterExample breaks example ties with.
-  3. Batches: parsed on the device while the previous batch aligns (a second thread), xm_counts_batch_info, xm_align_batch and
-     xm_format_sam right after it in the same thread (the slot rule of INTEGRATION.md §1).  A query the device could not align is an
-     error naming the read, never a silent drop.
-  4. After the last batch: the example reads of the VCF support column are read again from the inputs and uploaded, and the VCF and
-     mutations bodies are formatted on the device per contig, in name order (VcfWriter.java:111-114).
+     byte order (String.compareTo for ASCII names), the name order DirectionalAlignments.betterExample breaks example ties with.  The
+     names are ranked on the first device (xm_rank_names).
+  3. Batches, in file order: parsed on the first device while earlier batches align (a second thread), then batch k goes to device
+     k mod N.  Each device's worker thread runs xm_counts_batch_info, xm_align_batch and xm_format_sam (the slot rule of INTEGRATION.md
+     §1); the SAM text is written in batch order.  A query the device could not align is an error naming the read, never a silent drop.
+  4. After the last batch, with several devices: the count planes and variant tables are reduced over all of them (xm_comm_init,
+     xm_counts_reduce over NCCL), so the first handle holds the whole table.  Then the example reads of the VCF support column are read
+     again from the inputs and uploaded, and the VCF and mutations bodies are formatted on the first device per contig, in name order
+     (VcfWriter.java:111-114).
 
 Headers are this command's own: the reference's header texts are not in this repository and embed the command line (BASELINE.md §5),
 so SAM gets @SQ lines in database order, the VCF a #CHROM column line, and the mutations file none.  Parity with the reference is for the
-bodies.  Files ending in .gz are read through gzip on the host.  Every reference flag this command does not implement exits with
-status 2 and names the flag.
+bodies.  The output does not depend on the number of devices.  Files ending in .gz are read through gzip on the host.  Every reference
+flag this command does not implement exits with status 2 and names the flag.
 """
 import argparse
 import gzip
 import queue
 import sys
 import threading
+import time
 
 import numpy as np
 
@@ -53,7 +59,7 @@ def parse_args(argv):
     p.add_argument("--out-vcf", metavar="F")
     p.add_argument("--out-mutations", metavar="F")
     p.add_argument("--distinguish-query-ends", type=float, default=0.1, metavar="F", help="query_end_fraction of the counts (default 0.1)")
-    p.add_argument("--device", type=int, default=0, metavar="N", help="CUDA device")
+    p.add_argument("--device", type=device_list, default=[0], metavar="N[,M...]", help="CUDA device, or a comma list of distinct devices")
     p.add_argument("--batch-reads", type=int, default=262144, metavar="N", help="queries per alignment batch")
     args, extra = p.parse_known_args(argv)
     for a in extra:
@@ -66,6 +72,17 @@ def parse_args(argv):
     if args.batch_reads < 1 or args.split_queries_past_size < 0:
         p.error("--batch-reads must be positive and --split-queries-past-size non-negative")
     return args
+
+
+def device_list(text):
+    """--device: "N" or "N,M,...", distinct non-negative ordinals."""
+    try:
+        devs = [int(x) for x in text.split(",")]
+    except ValueError:
+        raise argparse.ArgumentTypeError("expected N or a comma list N,M,... of CUDA devices, got %r" % text) from None
+    if any(d < 0 for d in devs) or len(set(devs)) != len(devs):
+        raise argparse.ArgumentTypeError("devices must be distinct and non-negative, got %r" % text)
+    return devs
 
 
 def fmt_of(path):
@@ -161,29 +178,61 @@ def query_batches(g, args, batch_reads):
 
 
 def prefetch(gen):
-    """Runs the generator one item ahead in a second thread: the next chunk is parsed while the current batch aligns."""
+    """Runs the generator one item ahead in a second thread: the next chunk is parsed while the current batches align.  Closing the
+    returned generator early stops that thread and joins it."""
     q = queue.Queue(maxsize=1)
-    end = object()
+    end, stop = object(), threading.Event()
 
     def run():
         try:
             for item in gen:
+                if stop.is_set():
+                    return
                 q.put(item)
             q.put(end)
         except BaseException as e:  # noqa: BLE001 - handed to the consumer
             q.put(e)
-    threading.Thread(target=run, daemon=True).start()
-    while True:
-        item = q.get()
-        if item is end:
-            return
-        if isinstance(item, BaseException):
-            raise item
-        yield item
+    t = threading.Thread(target=run, daemon=True)
+    t.start()
+    try:
+        while True:
+            item = q.get()
+            if item is end:
+                return
+            if isinstance(item, BaseException):
+                raise item
+            yield item
+    finally:
+        stop.set()
+        while t.is_alive():   # a put the producer may be blocked in
+            try:
+                q.get(timeout=0.05)
+            except queue.Empty:
+                pass
+        t.join()
 
 
-def load_reference(g, paths):
-    """Contigs of all reference files, sorted by descending length (stable), uploaded; returns [(name bytes, length)]."""
+def on_all(handles, fn):
+    """fn(rank, handle) for every handle at once, one thread each; all threads are joined, then the first error is raised."""
+    errors = [None] * len(handles)
+
+    def run(d):
+        try:
+            fn(d, handles[d])
+        except BaseException as e:  # noqa: BLE001 - raised below, after the join
+            errors[d] = e
+    threads = [threading.Thread(target=run, args=(d,)) for d in range(len(handles))]
+    for t in threads:
+        t.start()
+    for t in threads:
+        t.join()
+    for e in errors:
+        if e is not None:
+            raise e
+
+
+def read_reference(g, paths):
+    """Contigs of all reference files parsed on g, sorted by descending length (stable): (packed contigs, lengths, names)."""
     parts = []
     for path in paths:
         src = Source(path, 0)
@@ -199,64 +248,169 @@ def load_reference(g, paths):
     lens = a["seq_len"].astype(np.int64)
     order = sorted(range(len(lens)), key=lambda i: -lens[i])
     wo, no = a["seq_word_off"], a["name_off"]
-    g.set_reference([a["packed"][wo[i]:wo[i + 1]] for i in order], [int(lens[i]) for i in order])
-    return [(a["names"][no[i]:no[i + 1]], int(lens[i])) for i in order]
+    return ([a["packed"][wo[i]:wo[i + 1]] for i in order], [int(lens[i]) for i in order], [a["names"][no[i]:no[i + 1]] for i in order])
+
+
+def align_one(g, first, a, per_query, ranks, paired_model, contig_names):
+    """One batch on handle g: returns (SAM text, align kernel ns).  first: global id of the batch's first sequence."""
+    n_seq = len(a["seq_len"])
+    nq = n_seq // per_query
+    batch = dict(packed=a["packed"] if len(a["packed"]) else np.zeros(1, np.uint16), seq_word_off=a["seq_word_off"], seq_len=a["seq_len"],
+                 n_seqs=np.full(nq, per_query, dtype=np.uint8),
+                 expected_inner=np.full(nq, paired_model[0] if per_query == 2 else 0.0), per_penalty=np.full(nq, paired_model[1] if per_query == 2 else 1.0))
+    if ranks is not None:
+        g.counts_batch_info(first, ranks[first:first + n_seq])
+    res, text = g.align_batch_sam(batch, (a["names"], a["name_off"]), contig_names, strict=False)
+    bad = np.nonzero(res["q_status"])[0]
+    if len(bad):
+        s = int(bad[0]) * per_query
+        raise SystemExit("query %r could not be aligned on the device (status %d); %d queries of this batch failed" %
+                         (a["names"][a["name_off"][s]:a["name_off"][s + 1]].decode(errors="replace"), int(res["q_status"][bad[0]]), len(bad)))
+    return text, int(res["stats"][capi.STAT["kernel_ns"]])
+
+
+def map_batches(handles, batches, ranks, paired_model, contig_names, write, reduce=False):
+    """Aligns `batches` ((array dict, sequences per query) in file order): batch k on handles[k % N], in one worker thread per handle,
+    with the global id of its first sequence and, when ranks is given, its sequences' name ranks (xm_counts_batch_info).  write() gets
+    the SAM text of every batch, in batch order.  reduce: after the last batch, once every worker has finished without error, the
+    counts of all handles are reduced (xm_comm_init + xm_counts_reduce, collectives entered by one thread per handle).
+    An error in `batches` or in a worker stops the dispatch; every thread is joined before the error of the earliest batch is raised.
+    Returns (sequences, batches, align kernel ns per handle, reduce wall seconds)."""
+    n_dev = len(handles)
+    inbox = [queue.Queue(maxsize=2) for _ in handles]
+    done = queue.Queue()
+    failed = threading.Event()
+    kernel_ns = [0] * n_dev
+
+    def worker(d):
+        while True:
+            job = inbox[d].get()
+            if job is None:
+                return
+            if failed.is_set():
+                continue   # drained, so that the dispatcher never blocks on a stopped worker
+            k, first, a, per_query = job
+            try:
+                text, ns = align_one(handles[d], first, a, per_query, ranks, paired_model, contig_names)
+                kernel_ns[d] += ns
+                done.put((k, text, None))
+            except BaseException as e:  # noqa: BLE001 - raised by the dispatcher
+                failed.set()
+                done.put((k, None, e))
+
+    threads = [threading.Thread(target=worker, args=(d,)) for d in range(n_dev)]
+    for t in threads:
+        t.start()
+    ready, errors = {}, []
+    n_out = n_batches = first = 0
+
+    def flush():   # results that have arrived, written in batch order up to the first error
+        nonlocal n_out
+        while True:
+            try:
+                k, text, e = done.get_nowait()
+            except queue.Empty:
+                return
+            if e is not None:
+                errors.append((k, e))
+            ready[k] = text
+            while n_out in ready and not errors:
+                write(ready.pop(n_out))
+                n_out += 1
+
+    try:
+        for a, per_query in batches:
+            if failed.is_set():
+                break
+            inbox[n_batches % n_dev].put((n_batches, first, a, per_query))
+            first += len(a["seq_len"])
+            n_batches += 1
+            flush()
+    except BaseException as e:  # noqa: BLE001 - raised below, after every thread has been joined
+        errors.append((n_batches, e))
+    finally:
+        close = getattr(batches, "close", None)
+        if close:
+            close()
+        for q in inbox:
+            q.put(None)
+        for t in threads:
+            t.join()
+    flush()
+    if errors:
+        raise min(errors, key=lambda x: x[0])[1]
+    reduce_s = 0.0
+    if reduce:
+        t0 = time.perf_counter()
+        uid = handles[0].comm_unique_id()
+        on_all(handles, lambda d, g: (g.comm_init(n_dev, d, uid), g.counts_reduce()))
+        reduce_s = time.perf_counter() - t0
+    return first, n_batches, kernel_ns, reduce_s
 
 
 def main(argv=None):
     args = parse_args(sys.argv[1:] if argv is None else argv)
     params = dict(synth.DEFAULT_PARAMS, enable_gapmers=0 if args.no_gapmers else 1)
     paired_model = args.spacing or (0.0, 1.0)   # without --spacing: the library's Query.java defaults
-    g = capi.XMapper(params, device=args.device)
-    contigs = load_reference(g, args.reference)
+    t0 = time.perf_counter()
+    handles = []
+    try:
+        for dev in args.device:
+            handles.append(capi.XMapper(params, device=dev))
+        map_files(args, params, paired_model, handles, t0)
+    finally:
+        for g in handles:
+            g.close()
+
+
+def map_files(args, params, paired_model, handles, t0):
+    g = handles[0]
+    packed, lens, names = read_reference(g, args.reference)
+    on_all(handles, lambda d, h: h.set_reference(packed, lens))
     if args.infer_ancestors:
-        total, min_dup = sum(n for _, n in contigs), 1
+        total, min_dup = sum(lens), 1
         while (1 << min_dup) < total:   # minDuplicationLength = SequenceDatabase.log2RoundUp(totalForwardSize)
             min_dup += 1
         g.infer_ancestors(params["max_error_rate"] / params["mutation"], min_interesting=min_dup, max_short=8)
-        contigs = [(name + b"-anc", n) for name, n in contigs]   # the inferred sequences are named "<name>-anc" (M/Mapper.java:675-681)
+        names = [name + b"-anc" for name in names]   # the inferred sequences are named "<name>-anc" (M/Mapper.java:675-681)
+        if len(handles) > 1:
+            anc = [synth.pack_contig(g.get_reference(c)) for c in range(len(lens))]
+            on_all(handles[1:], lambda d, h: h.set_reference(anc, lens))
+    contigs = list(zip(names, lens))
     counts = bool(args.out_vcf or args.out_mutations)
+    t_setup = time.perf_counter()
     # pre-pass: longest sequence, and the name rank of every sequence
-    max_len, names = 1, []
+    max_len, blobs, offs, n_name_bytes = 1, [], [], 0
     for a, _ in query_batches(g, args, 1 << 22):
         if len(a["seq_len"]):
             max_len = max(max_len, int(a["seq_len"].max()))
         if counts:
-            no, blob = a["name_off"], a["names"]
-            names += [blob[no[i]:no[i + 1]] for i in range(len(no) - 1)]
-    g.build_index(max_len)
-    g.build_duplications(-1, -1, 2, 1000)
-    ranks = None
-    if counts:
-        ranks = np.unique(np.array(names, dtype=object), return_inverse=True)[1].astype(np.int64).reshape(-1)
-        g.counts_enable(args.distinguish_query_ends)
+            blobs.append(a["names"])
+            offs.append(a["name_off"][1:] + n_name_bytes)
+            n_name_bytes += len(a["names"])
+    ranks = g.rank_names(b"".join(blobs), np.concatenate([np.zeros(1, np.int64)] + offs)) if counts else None
+    del blobs, offs
+    t_prepass = time.perf_counter()
+
+    def build(d, h):
+        h.build_index(max_len)
+        h.build_duplications(-1, -1, 2, 1000)
+        if counts:
+            h.counts_enable(args.distinguish_query_ends)
+    on_all(handles, build)
+    t_index = time.perf_counter()
     contig_names = (b"".join(n for n, _ in contigs), np.concatenate([[0], np.cumsum([len(n) for n, _ in contigs])]).astype(np.int64))
     sam = open(args.out_sam, "wb") if args.out_sam else None
-    if sam:
-        sam.write(b"".join(b"@SQ\tSN:%s\tLN:%d\n" % (n, ln) for n, ln in contigs))
-    first, n_batches, kernel_ns = 0, 0, 0
-    for a, per_query in prefetch(query_batches(g, args, args.batch_reads)):
-        n_seq = len(a["seq_len"])
-        nq = n_seq // per_query
-        batch = dict(packed=a["packed"] if len(a["packed"]) else np.zeros(1, np.uint16), seq_word_off=a["seq_word_off"], seq_len=a["seq_len"],
-                     n_seqs=np.full(nq, per_query, dtype=np.uint8),
-                     expected_inner=np.full(nq, paired_model[0] if per_query == 2 else 0.0), per_penalty=np.full(nq, paired_model[1] if per_query == 2 else 1.0))
-        if counts:
-            g.counts_batch_info(first, ranks[first:first + n_seq])
-        res, text = g.align_batch_sam(batch, (a["names"], a["name_off"]), contig_names, strict=False)
-        bad = np.nonzero(res["q_status"])[0]
-        if len(bad):
-            s = int(bad[0]) * per_query
-            raise SystemExit("query %r could not be aligned on the device (status %d); %d queries of this batch failed" %
-                             (a["names"][a["name_off"][s]:a["name_off"][s + 1]].decode(errors="replace"), int(res["q_status"][bad[0]]), len(bad)))
+    try:
         if sam:
-            sam.write(text.encode())
-        first += n_seq
-        n_batches += 1
-        kernel_ns += int(res["stats"][capi.STAT["kernel_ns"]])
-    if sam:
-        sam.close()
-    print("mapper_b200: %d sequences in %d batches, align kernels %.3f s (device time)" % (first, n_batches, kernel_ns / 1e9), file=sys.stderr)
+            sam.write(b"".join(b"@SQ\tSN:%s\tLN:%d\n" % (n, ln) for n, ln in contigs))
+        write = (lambda text: sam.write(text.encode())) if sam else (lambda text: None)
+        n_seq, n_batches, kernel_ns, reduce_s = map_batches(handles, prefetch(query_batches(g, args, args.batch_reads)), ranks, paired_model,
+                                                            contig_names, write, reduce=counts and len(handles) > 1)
+    finally:
+        if sam:
+            sam.close()
+    t_map = time.perf_counter()
     by_name = sorted(range(len(contigs)), key=lambda c: contigs[c][0])   # TreeMap<String> order of the contig names
     if args.out_vcf:
         upload_examples(g, args)
@@ -272,7 +426,12 @@ def main(argv=None):
                 name, ln = contigs[c]
                 for s in range(0, ln, MUTATIONS_RANGE):
                     f.write(g.format_mutations(c, name, s, min(ln, s + MUTATIONS_RANGE), MUTATIONS_FILTER).encode())
-    g.close()
+    t_end = time.perf_counter()
+    print("mapper_b200: %d sequences in %d batches on %d device%s, align kernels %.3f s (device time; per device %s)" %
+          (n_seq, n_batches, len(handles), "s" if len(handles) > 1 else "", sum(kernel_ns) / 1e9, " ".join("%.3f" % (k / 1e9) for k in kernel_ns)),
+          file=sys.stderr)
+    print("mapper_b200: wall s: set-up %.3f, pre-pass %.3f, index %.3f, mapping %.3f, reduce %.3f, formatting %.3f" %
+          (t_setup - t0, t_prepass - t_setup, t_index - t_prepass, t_map - t_index - reduce_s, reduce_s, t_end - t_map), file=sys.stderr)
 
 
 def upload_examples(g, args):

@@ -18,7 +18,7 @@ EXPORTS = ["xm_create", "xm_destroy", "xm_last_error", "xm_set_reference", "xm_s
            "xm_counts_enable", "xm_counts_device_ptr", "xm_counts_fetch", "xm_format_sam",
            "xm_comm_unique_id", "xm_comm_init", "xm_counts_reduce", "xm_counts_batch_info", "xm_variants_fetch", "xm_measure_peaks", "xm_counts_reduce_times",
            "xm_variants_examples", "xm_variants_set_examples", "xm_format_vcf", "xm_format_mutations",
-           "xm_parse_reads", "xm_reads_array", "xm_release_reads"]
+           "xm_parse_reads", "xm_reads_array", "xm_release_reads", "xm_rank_names"]
 
 RESULT_ARRAYS = [("q_comp_off", np.int64), ("comp_choice_off", np.int64), ("choice_sa_off", np.int64), ("sa_block_off", np.int64),
                  ("choice_f64", np.float64), ("sa_f64", np.float64), ("choice_inner", np.int32), ("sa_contig", np.int32),
@@ -330,6 +330,17 @@ class XMapper:
         off, blob = a["name_off"], a["names"]
         names = [blob[off[i]:off[i + 1]].decode("utf-8", "surrogateescape") for i in range(n)]
         return batch, names, a["record"], n_consumed
+
+    def rank_names(self, names, name_off):
+        """xm_rank_names: int64 ranks of the names names[name_off[i]:name_off[i + 1]] (bytes, or a uint8 array) in unsigned byte order,
+        equal names ranked equal: np.unique(names, return_inverse=True)[1], computed on the device."""
+        off = np.ascontiguousarray(name_off, dtype=np.int64)
+        if off.ndim != 1 or len(off) < 1:
+            raise ValueError("name_off needs n + 1 entries")
+        blob = np.frombuffer(names, dtype=np.uint8) if isinstance(names, (bytes, bytearray)) else np.ascontiguousarray(names, dtype=np.uint8)
+        out = np.zeros(len(off) - 1, dtype=np.int64)
+        self._ok(self.L.xm_rank_names(self.h, C.c_int64(len(off) - 1), _ptr(blob), _ptr(off), _ptr(out)))
+        return out
 
     # ---- per-position counts ----
     def counts_enable(self, query_end_fraction=0.1):

@@ -678,6 +678,7 @@ struct DevBuf {
 #include "xm_counts.cuh"
 #include "xm_variants_fmt.cuh"
 #include "xm_parse.cuh"
+#include "xm_names.cuh"
 
 // pinned host slabs for results, recycled between batches (cudaHostAlloc of 100 MB costs tens of ms)
 struct PinnedPool {
@@ -2717,6 +2718,75 @@ int64_t xm_reads_array(const xm_reads* r, int which, const void** ptr) {
   return r->n[which];
 }
 void xm_release_reads(xm_reads* r) { delete r; }
+
+int xm_rank_names(xm_handle* h, int64_t n, const char* names, const int64_t* name_off, int64_t* ranks) {
+  if (!h) return XM_ERR_ARG;
+  if (n < 0 || n >= (1ll << 31) || !name_off || (n > 0 && !ranks)) { h->err = "xm_rank_names: 0 <= n < 2^31 names, name_off[n + 1] and ranks[n] are required"; return XM_ERR_ARG; }
+  if (name_off[0] != 0) { h->err = "xm_rank_names: name_off[0] != 0"; return XM_ERR_ARG; }
+  for (int64_t i = 0; i < n; i++) if (name_off[i + 1] < name_off[i]) { h->err = "xm_rank_names: name_off is not non-decreasing at " + std::to_string(i); return XM_ERR_ARG; }
+  const int64_t n_bytes = name_off[n];
+  if (n_bytes > 0 && !names) { h->err = "xm_rank_names: names is NULL"; return XM_ERR_ARG; }
+  if (n == 0) return XM_OK;
+  std::lock_guard<std::mutex> compute(h->compute_mu);
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = h->stream;
+  const int ni = (int)n;
+  int label_bits = 1;
+  while ((1ll << label_bits) < n) label_bits++;
+  // scratch for this call only: it is freed on return, so ranking a large run leaves no device memory behind for the batches
+  DevBuf d_names, d_off, d_act, d_act2, d_key, d_key2, d_iota, d_p1, d_lab1, d_p2, d_sin, d_sout, d_keep, d_final, d_tmp, d_misc;
+  const size_t N = (size_t)n;
+  if (!d_names.ensure((size_t)n_bytes + 16) || !d_off.ensure((N + 1) * 8) || !d_act.ensure(N * 8) || !d_act2.ensure(N * 8) || !d_key.ensure(N * 8) ||
+      !d_key2.ensure(N * 8) || !d_iota.ensure(N * 4) || !d_p1.ensure(N * 4) || !d_lab1.ensure(N * 4) || !d_p2.ensure(N * 4) ||
+      !d_sin.ensure((N + 1) * 8) || !d_sout.ensure((N + 1) * 8) || !d_keep.ensure(N) || !d_final.ensure(N * 4) || !d_misc.ensure(16)) {
+    h->err = "out of device memory (xm_rank_names)"; return XM_ERR_CUDA;
+  }
+  uint64_t *act = (uint64_t*)d_act.p, *act2 = (uint64_t*)d_act2.p, *key = (uint64_t*)d_key.p, *key2 = (uint64_t*)d_key2.p;
+  uint32_t *iota = (uint32_t*)d_iota.p, *p1 = (uint32_t*)d_p1.p, *lab1 = (uint32_t*)d_lab1.p, *p2 = (uint32_t*)d_p2.p, *fin = (uint32_t*)d_final.p;
+  int2 *sin = (int2*)d_sin.p, *sout = (int2*)d_sout.p;
+  uint8_t* keep = (uint8_t*)d_keep.p;
+  int* d_count = (int*)d_misc.p;
+  size_t t1 = 0, t2 = 0, t3 = 0, t4 = 0, t5 = 0;
+  cub::DeviceRadixSort::SortPairs(nullptr, t1, key, key2, iota, p1, ni, 0, 64, st);
+  cub::DeviceRadixSort::SortPairs(nullptr, t2, lab1, iota, p1, p2, ni, 0, label_bits, st);
+  cub::DeviceScan::InclusiveScan(nullptr, t3, sin, sout, RnMax2(), ni, st);
+  cub::DeviceSelect::Flagged(nullptr, t4, key, keep, act, d_count, ni, st);
+  cub::DeviceScan::ExclusiveSum(nullptr, t5, (const int*)nullptr, (int*)nullptr, ni + 1, st);
+  const size_t tb = std::max(std::max(std::max(t1, t2), std::max(t3, t4)), t5) + 256;
+  if (!d_tmp.ensure(tb)) { h->err = "out of device memory (xm_rank_names)"; return XM_ERR_CUDA; }
+  if (n_bytes) CK(cudaMemcpyAsync(d_names.p, names, (size_t)n_bytes, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(d_off.p, name_off, (N + 1) * 8, cudaMemcpyHostToDevice, st));
+  // every name starts in the one class of label 0, as item (0 << 32 | i)
+  xm_rank_init_kernel<<<pz_blocks(n, RN_THREADS), RN_THREADS, 0, st>>>(ni, act);
+  int m = ni;
+  for (int d = 0; m > 0; d++) {
+    const unsigned blocks = pz_blocks(m, RN_THREADS);
+    size_t q;
+    xm_rank_key_kernel<<<blocks, RN_THREADS, 0, st>>>((const uint8_t*)d_names.p, (const int64_t*)d_off.p, act, m, d, key, iota);
+    q = tb; CK(cub::DeviceRadixSort::SortPairs(d_tmp.p, q, key, key2, iota, p1, m, 0, 64, st));
+    xm_rank_label_kernel<<<blocks, RN_THREADS, 0, st>>>(act, p1, m, lab1);
+    q = tb; CK(cub::DeviceRadixSort::SortPairs(d_tmp.p, q, lab1, iota, p1, p2, m, 0, label_bits, st));
+    xm_rank_gather_kernel<<<blocks, RN_THREADS, 0, st>>>(act, key, p2, m, act2, key2);
+    xm_rank_flags_kernel<<<blocks, RN_THREADS, 0, st>>>(act2, key2, m, sin);
+    q = tb; CK(cub::DeviceScan::InclusiveScan(d_tmp.p, q, sin, sout, RnMax2(), m, st));
+    xm_rank_split_kernel<<<blocks, RN_THREADS, 0, st>>>(act2, key2, sout, m, fin, keep, key);
+    q = tb; CK(cub::DeviceSelect::Flagged(d_tmp.p, q, key, keep, act, d_count, m, st));
+    CK(cudaMemcpyAsync(&m, d_count, 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+  }
+  // dense ranks: the number of labels in use below a name's label
+  int* mark = (int*)d_sin.p;
+  int* below = (int*)d_sout.p;
+  CK(cudaMemsetAsync(mark, 0, (N + 1) * 4, st));
+  xm_rank_mark_kernel<<<pz_blocks(n, RN_THREADS), RN_THREADS, 0, st>>>(fin, ni, mark);
+  size_t q = tb;
+  CK(cub::DeviceScan::ExclusiveSum(d_tmp.p, q, mark, below, ni + 1, st));
+  xm_rank_dense_kernel<<<pz_blocks(n, RN_THREADS), RN_THREADS, 0, st>>>(fin, below, ni, (int64_t*)d_act2.p);
+  CK(cudaMemcpyAsync(ranks, d_act2.p, N * 8, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  CK(cudaGetLastError());
+  return XM_OK;
+}
 
 // out[0] INT32 IMAD, out[1] FP64 DADD, out[2] FP32 FFMA (full-rate pipe = the dispatch ceiling): sustained warp-instructions per second over the whole chip (the loop
 // bodies are 128 arithmetic instructions per iteration per warp; loop overhead is below 2 %); out[3] = SM count, out[4] = SM clock in Hz
